@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, sm_100a)
     python bench.py --impl reference --steps K --warmup W     # reference arm: the unmodified reference (oracle/_ref) on the host cores
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs as DIR/*.npy
 
 A "step" is one training step (zero_grad -> forward -> CE(label_smoothing) -> backward -> clip -> AdamW,
 R/training/train.py:258-271) over one batch of synthetic RadioML-shaped frames (random-init weights).
@@ -293,6 +294,30 @@ def ncu_traffic(table, workload, kernel_class, frames, default_frames):
     return traffic, f"ncu capture at this launch size ({ent.get('report')})"
 
 
+# --dump-outputs: elements kept per array (float32), 64 MB in all
+DUMP_ELEMS = {"logits": 4 << 20, "parameters": 12 << 20}
+
+
+def dump_outputs(out_dir, trainer):
+    """Writes what the last training step handed its caller to out_dir/<name>.npy (float32): `logits`, the [B, classes]
+    output of its forward pass, and `parameters`, the model's parameters after its AdamW update (named_parameters order,
+    flattened and concatenated).  An array with more elements than DUMP_ELEMS allows is replaced by a fixed, seeded
+    sample of them (sorted flat indices, the same for every run with the same arguments), so the outputs of two builds
+    can be compared element for element.  Compare them with a tolerance: the weight-gradient GEMMs add split-K partial
+    sums with atomics, so two runs of one build already differ in the last bits, and training steps amplify that (bf16,
+    default workload, 25 steps: logits 2e-3 and parameters 5e-4 of their largest magnitude, measured on a B200 at 1000 W)."""
+    import numpy as np
+    import torch
+    arrays = {"logits": trainer._logits,
+              "parameters": torch.cat([p.detach().reshape(-1) for p in trainer.model.parameters()])}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.float().cpu().numpy()
+        if a.size > DUMP_ELEMS[name]:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_ELEMS[name], replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -313,7 +338,11 @@ def main():
     ap.add_argument("--graph", action="store_true",
                     help="single GPU: drive the step as one CUDA-graph replay (GraphTrainStep) -- the launch-bound small batches")
     ap.add_argument("--profile-out", default="")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the logits and updated parameters of the last timed training step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     w = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference_arm(args, w, args.workload)
@@ -406,6 +435,8 @@ def main():
     if step_cls is GraphTrainStep:      # kernels of the library launched by the graph replays of the timed region
         launches += (trainer.replays - replays0) * trainer.kernels_per_replay
     loss, acc = trainer.read_stats()
+    if args.dump_outputs and rank == 0:     # before the steps below train the model further
+        dump_outputs(args.dump_outputs, trainer)
 
     # ---- end to end from host buffers (e2e) -----------------------------------------------------------
     pipe = HostPipeline(trainer, tuple(host_x[0].shape))

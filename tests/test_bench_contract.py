@@ -1,9 +1,12 @@
-"""bench.py contract checks that need no GPU: the reference arm prints one well-formed JSON line."""
+"""bench.py contract checks: the reference arm prints one well-formed JSON line; --dump-outputs (the end-to-end run of
+our arm needs a GPU)."""
 import json
 import math
 import os
 import subprocess
 import sys
+
+import pytest
 
 from conftest import ROOT
 
@@ -61,28 +64,86 @@ def test_ncu_launch_list_summary_parses_the_committed_capture(tmp_path):
     assert abs(sum(shares) - 100.0) < 1.0
 
 
-def test_vendored_reference_is_a_byte_copy_and_runs(tmp_path):
-    """oracle/make_ref.py copies the reference's model code unmodified (sha256 manifest) and the copy is importable; the
-    reference arm's train step is the reference's own loop body (R/training/train.py:258-271)."""
-    import pytest
-    if not os.path.isdir("/root/reference/Transformer_Thesis"):
-        pytest.skip("the reference tree exists in the build container only")
-    sys.path.insert(0, ROOT)
+# A stand-in for the reference's model code with its layout (Transformer_Thesis/{transformer_rawIQ,ViT}/models/**.py,
+# sub-packages without __init__.py) and two files make_ref.py must leave behind: a non-Python file and a script outside
+# models/.  The classes take the reference's constructor arguments.
+_STAND_IN_MODELS = {
+    "transformer_rawIQ/models/transformer_rawIQ.py": (
+        "import torch\nfrom .blocks.head import head\n\n\nclass AMCTransformer(torch.nn.Module):\n"
+        "    def __init__(self, in_channels, seq_length, num_classes, device='cpu', **kw):\n"
+        "        super().__init__()\n        self.head = head(in_channels * seq_length, num_classes)\n\n"
+        "    def forward(self, x):\n        return self.head(x.flatten(1))\n"),
+    "transformer_rawIQ/models/blocks/head.py": "import torch\n\n\ndef head(k, n):\n    return torch.nn.Linear(k, n)\n",
+    "ViT/models/amc_transformer.py": (
+        "import torch\n\n\nclass AMCTransformer(torch.nn.Module):\n"
+        "    def __init__(self, in_channels, img_size_h, img_size_w, num_classes, device='cpu', **kw):\n"
+        "        super().__init__()\n        self.head = torch.nn.Linear(in_channels * img_size_h * img_size_w, num_classes)\n\n"
+        "    def forward(self, x):\n        return self.head(x.flatten(1))\n"),
+}
+_STAND_IN_OTHER = {"transformer_rawIQ/models/notes.txt": "not Python\n", "ViT/training/train.py": "raise SystemExit\n"}
+
+
+def _forget_vendored_modules():
     from oracle import make_ref
-    m = make_ref.vendor("/root/reference", str(tmp_path / "_ref"))
-    assert len(m) == 18 and all(k.startswith(("transformer_rawIQ/models/", "ViT/models/")) for k in m)
-    make_ref.vendor("/root/reference", str(tmp_path / "_ref"), check=True)
+    for k in [k for k in sys.modules if k.split(".")[0] in make_ref.PACKAGES]:
+        del sys.modules[k]
+
+
+def _run_reference_steps(bench, torch):
+    for name, x, n_cls in (("rawiq_seg16_d128_L6", torch.randn(4, 2, 1024), 11),
+                           ("vit_p16_d256_L6", torch.randn(4, 1, 32, 64), 19)):
+        ref = bench.ReferenceStep(bench.WORKLOADS[name])
+        y = torch.randint(0, n_cls, (4,))
+        l0 = ref.step(x, y).item()
+        l1 = ref.step(x, y).item()
+        assert math.isfinite(l0) and math.isfinite(l1)
+        yield name, ref
+
+
+def test_vendored_reference_is_a_byte_copy_and_runs(tmp_path, monkeypatch):
+    """oracle/make_ref.py copies the reference's model code unmodified (sha256 manifest) and the copy is importable; the
+    reference arm's train step is the reference's own loop body (R/training/train.py:258-271).  The copy is made from a
+    stand-in tree; where the reference itself has been vendored into oracle/_ref, that copy is run too."""
+    import hashlib
+
     import torch
     import bench
-    if not bench.reference_available():
-        pytest.skip("oracle/_ref not built")
-    w = bench.WORKLOADS["rawiq_seg16_d128_L6"]
-    ref = bench.ReferenceStep(w)
-    assert sum(p.numel() for p in ref.model.parameters()) == 1985163          # SURVEY §8d cross-check for cfg-1
-    x, y = torch.randn(4, 2, 1024), torch.randint(0, 11, (4,))
-    l0 = ref.step(x, y).item()
-    l1 = ref.step(x, y).item()
-    assert math.isfinite(l0) and math.isfinite(l1)
+    from oracle import make_ref
+    if bench.reference_available():
+        _forget_vendored_modules()
+        for name, ref in _run_reference_steps(bench, torch):
+            if name == "rawiq_seg16_d128_L6":
+                assert sum(p.numel() for p in ref.model.parameters()) == 1985163     # SURVEY §8d cross-check for cfg-1
+        _forget_vendored_modules()
+
+    src = tmp_path / "src"
+    for rel, text in {**_STAND_IN_MODELS, **_STAND_IN_OTHER}.items():
+        f = src / "Transformer_Thesis" / rel
+        f.parent.mkdir(parents=True, exist_ok=True)
+        f.write_text(text)
+    dst = tmp_path / "_ref"
+    m = make_ref.vendor(str(src), str(dst))
+    assert sorted(m) == sorted(_STAND_IN_MODELS)
+    for rel, digest in m.items():
+        data = (src / "Transformer_Thesis" / rel).read_bytes()
+        assert (dst / rel).read_bytes() == data and digest == hashlib.sha256(data).hexdigest()
+    assert json.loads((dst / "MANIFEST.json").read_text())["files"] == m
+    assert not (dst / "transformer_rawIQ" / "models" / "notes.txt").exists() and not (dst / "ViT" / "training").exists()
+    make_ref.vendor(str(src), str(dst), check=True)
+    edited = dst / "ViT" / "models" / "amc_transformer.py"
+    edited.write_text(_STAND_IN_MODELS["ViT/models/amc_transformer.py"] + "# edited\n")
+    with pytest.raises(SystemExit, match="differs from the reference"):
+        make_ref.vendor(str(src), str(dst), check=True)
+    edited.write_text(_STAND_IN_MODELS["ViT/models/amc_transformer.py"])
+
+    monkeypatch.setattr(make_ref, "HERE", str(tmp_path))            # load_reference() -> <tmp_path>/_ref
+    monkeypatch.setattr(sys, "path", list(sys.path))
+    _forget_vendored_modules()
+    try:
+        for _, ref in _run_reference_steps(bench, torch):
+            assert os.path.dirname(sys.modules[type(ref.model).__module__].__file__).startswith(str(dst))
+    finally:
+        _forget_vendored_modules()
 
 
 def test_roofline_traffic_is_scaled_to_the_run_batch():
@@ -127,3 +188,50 @@ def test_ncu_full_summary_reads_the_raw_csv_made_on_the_gpu_box(tmp_path, monkey
     assert tj["gemm_wgrad"]["report"] == "cap.csv" and tj["gemm_wgrad"]["launches"] == 2 and tj["gemm_wgrad"]["frames"] == 4096
     assert abs(tj["gemm_wgrad"]["dram_bytes_per_launch"] - 400e6) < 1.0
     assert tj["attn_bwd"]["kernels"] == ["attn_tc5_bwd_kernel<2>"] and abs(tj["attn_bwd"]["dram_bytes_per_launch"] - 510e6) < 1.0
+
+
+def test_dump_outputs_writes_float32_arrays_and_samples_the_large_ones(tmp_path, monkeypatch):
+    """--dump-outputs: the last step's logits and updated parameters as DIR/<name>.npy; an array over its element budget
+    becomes the same seeded sample of its elements on every run."""
+    import types
+
+    import numpy as np
+    import torch
+    import bench
+    model = torch.nn.Sequential(torch.nn.Linear(8, 6), torch.nn.Linear(6, 3))
+    logits = torch.randn(5, 3, dtype=torch.float64)
+    trainer = types.SimpleNamespace(model=model, _logits=logits)
+    bench.dump_outputs(str(tmp_path / "a"), trainer)
+    flat = torch.cat([p.detach().reshape(-1) for p in model.parameters()]).numpy()
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("logits", "parameters")}
+    assert got["logits"].dtype == np.float32 and np.array_equal(got["logits"], logits.float().numpy())
+    assert got["parameters"].dtype == np.float32 and np.array_equal(got["parameters"], flat)
+    assert sum(bench.DUMP_ELEMS.values()) * 4 <= 64 << 20
+    monkeypatch.setitem(bench.DUMP_ELEMS, "parameters", 20)
+    bench.dump_outputs(str(tmp_path / "b"), trainer)
+    bench.dump_outputs(str(tmp_path / "c"), trainer)
+    b, c = np.load(tmp_path / "b" / "parameters.npy"), np.load(tmp_path / "c" / "parameters.npy")
+    assert b.shape == (20,) and np.array_equal(b, c) and np.isin(b, flat).all()
+    assert np.array_equal(np.load(tmp_path / "b" / "logits.npy"), got["logits"])
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_end_to_end(tmp_path):
+    """bench.py --steps 3 --dump-outputs DIR on the GPU: the JSON line reports the 3 timed steps and DIR holds the last
+    step's logits [batch, classes] and every parameter of the workload's model as finite float32."""
+    import numpy as np
+    import bench
+    from oracle import amc_oracle as O
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "3", "--batch", "512",
+                          "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True,
+                         timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 3 and line["config"]["frames_per_gpu_per_step"] == 512
+    w = bench.WORKLOADS[bench.DEFAULT_WORKLOAD]
+    logits = np.load(tmp_path / "logits.npy")
+    params = np.load(tmp_path / "parameters.npy")
+    assert logits.dtype == params.dtype == np.float32
+    assert logits.shape == (512, w["kw"]["num_classes"]) and np.isfinite(logits).all()
+    kw = {k: v for k, v in w["kw"].items() if k != "drop_prob"}
+    assert params.shape == (O.param_count(O.Config(kind=w["kind"], **kw)),) and np.isfinite(params).all()

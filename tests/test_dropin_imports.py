@@ -8,7 +8,6 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/Transformer_Thesis"
 
 CASES = {
     "rawiq": ("transformer_rawIQ", "from models.transformer_rawIQ import AMCTransformer", "RawIQAMCTransformer",
@@ -21,33 +20,47 @@ CASES = {
 }
 
 
-def _run(kind, with_reference_root):
+def _reference_layout(root, kind):
+    """A stand-in for the reference's project directory with the layout dropin/README.md describes: ``models/`` has no
+    ``__init__.py`` (a namespace package) and holds a module of the name the reference's scripts import -- one that fails
+    if it is ever imported instead of the shim -- next to the reference's own ``training/``."""
+    sub, stmt = CASES[kind][:2]
+    base = root / sub
+    (base / "models").mkdir(parents=True)
+    (base / "models" / (stmt.split()[1].split(".")[1] + ".py")).write_text(
+        "raise ImportError('the reference module was imported instead of the shim')\n")
+    (base / "training").mkdir()
+    (base / "training" / "train.py").write_text("")
+    return str(base)
+
+
+def _run(kind, cwd, reference_root=None):
     sub, stmt, cls, ctor, n_params = CASES[kind]
     code = "import sys\n"
-    if with_reference_root:
+    if reference_root:
         # what the reference scripts do before importing (train.py: sys.path.append(str(Path(__file__).parent.parent)))
-        code += f"sys.path.append({os.path.join(REF, sub)!r})\n"
+        code += f"sys.path.append({reference_root!r})\n"
     code += (f"{stmt}\nm = {ctor}\n"
              "print(type(m).__module__, type(m).__name__, sum(p.numel() for p in m.parameters()))\n")
-    if with_reference_root:
+    if reference_root:
         code += "import training\nprint(list(training.__path__)[0])\n"
     env = dict(os.environ, PYTHONPATH=os.pathsep.join([ROOT, os.path.join(ROOT, "dropin", kind)]))
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, cwd="/tmp", timeout=300)
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, cwd=cwd, timeout=300)
     assert r.returncode == 0, r.stderr[-2000:]
     return r.stdout.strip().splitlines()
 
 
 @pytest.mark.parametrize("kind", ["rawiq", "vit"])
-def test_shim_resolves_the_reference_import_statement(kind):
-    out = _run(kind, with_reference_root=False)
+def test_shim_resolves_the_reference_import_statement(kind, tmp_path):
+    out = _run(kind, tmp_path)
     mod, cls, n = out[0].split()
     assert mod.startswith("vit_vs_raw_iq_b200") and cls == CASES[kind][2] and int(n) == CASES[kind][4]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
 @pytest.mark.parametrize("kind", ["rawiq", "vit"])
-def test_shim_wins_over_the_reference_namespace_package(kind):
-    out = _run(kind, with_reference_root=True)
+def test_shim_wins_over_the_reference_namespace_package(kind, tmp_path):
+    ref_root = _reference_layout(tmp_path / "Transformer_Thesis", kind)
+    out = _run(kind, tmp_path, reference_root=ref_root)
     mod, cls, n = out[0].split()
     assert mod.startswith("vit_vs_raw_iq_b200") and cls == CASES[kind][2] and int(n) == CASES[kind][4]
-    assert out[1].startswith(os.path.join(REF, CASES[kind][0]))          # training.* is still the reference's
+    assert out[1].startswith(ref_root)          # training.* is still the reference's

@@ -3,19 +3,16 @@ error behaviour, and that the C-ABI library exports every symbol the header decl
 import ctypes
 import os
 import re
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN_CASES, ROOT, load_golden
+from conftest import GOLDEN_CASES, GOLDEN_DIR, ROOT, load_golden
 from oracle import amc_oracle as O
 
 import vit_vs_raw_iq_b200 as amc
 from vit_vs_raw_iq_b200 import _lib
-
-REF = "/root/reference/Transformer_Thesis"
 
 
 def build_ours(name, **extra):
@@ -70,29 +67,29 @@ def test_known_answer_param_counts():
     assert sum(p.numel() for p in m.encoder.layers[0].parameters()) == 789_760
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
 @pytest.mark.parametrize("kind", ["rawiq", "vit"])
 def test_same_seed_gives_reference_initial_weights(kind):
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    from make_golden import import_reference
-    RefAMC = import_reference(kind)
+    """The reference's modules constructed after torch.manual_seed(s) (tests/golden/make_golden.py trajectory_case /
+    trajectory_vit_case: seed 5 / 6, dropout 0) stored their initial state_dict as the trajectories' param/*; ours
+    must draw the same weights from the same seed.  Dropout has no parameters and draws nothing at construction, so
+    building ours with dropout on must not change them."""
     if kind == "rawiq":
-        kw = dict(in_channels=2, seq_length=256, num_classes=11, d_model=32, n_head=4, n_layers=2, ffn_hidden=64,
+        seed, golden = 5, "trajectory_rawiq.npz"
+        kw = dict(in_channels=2, seq_length=256, num_classes=4, d_model=32, n_head=4, n_layers=2, ffn_hidden=64,
                   drop_prob=0.1, device="cpu", use_cls_token=True, embedding_type="segment", segment_size=16)
         ours_cls = amc.RawIQAMCTransformer
     else:
-        kw = dict(in_channels=1, img_size_h=32, img_size_w=64, patch_size=8, num_classes=19, d_model=32, n_head=4,
-                  n_layers=2, ffn_hidden=64, drop_prob=0.1, device="cpu")
+        seed, golden = 6, "trajectory_vit.npz"
+        kw = dict(in_channels=1, img_size_h=32, img_size_w=64, patch_size=16, num_classes=4, d_model=64, n_head=8,
+                  n_layers=2, ffn_hidden=128, drop_prob=0.1, device="cpu")
         ours_cls = amc.ViTAMCTransformer
-    torch.manual_seed(7)
-    ref = RefAMC(**kw)
-    torch.manual_seed(7)
-    ours = ours_cls(**kw)
-    rsd, osd = ref.state_dict(), ours.state_dict()
+    z = np.load(os.path.join(GOLDEN_DIR, golden))
+    rsd = {k[len("param/"):]: z[k] for k in z.files if k.startswith("param/")}
+    torch.manual_seed(seed)
+    osd = ours_cls(**kw).state_dict()
     assert list(rsd) == list(osd)
     for k in rsd:
-        assert torch.equal(rsd[k], osd[k]), k
-    sys.path[:] = [p for p in sys.path if not p.startswith(REF)]
+        assert np.array_equal(rsd[k], osd[k].numpy()), k
 
 
 def test_constructor_errors_match_reference():
