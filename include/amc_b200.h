@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AMC_ABI_VERSION 6
+#define AMC_ABI_VERSION 7
 
 enum { AMC_KIND_RAWIQ = 0, AMC_KIND_VIT = 1 };
 enum { AMC_F32 = 0, AMC_BF16 = 1 };
@@ -129,6 +129,24 @@ int amc_model_fwd(const AmcDesc* desc, const float* src, const float* params, co
 int amc_model_bwd(const AmcDesc* desc, const float* src, const float* params, void* workspace,
                   const float* dlogits, const float* denc_out, float* grads,
                   int stage_begin, int stage_end, amc_stream_t stream);
+
+/* The same backward with the gradient w.r.t. the input frames (saliency maps, FGSM/PGD adversarial examples and
+ * adversarial training on a trained classifier): autograd of R/models/embedding/patch_embedding.py:47-60,
+ * V/models/embedding/patch_embedding.py:11-15 and, for AMC_INPUT_RAW, R/dataloader/dataset.py:215-222.
+ * amc_model_bwd(...) is amc_model_bwd_ex(..., grads, NULL, ...).
+ *   grads  as above, or NULL: no parameter gradients at all (a frozen model).  Only the data-gradient chain runs: no
+ *          weight-gradient GEMMs, no bias / LayerNorm / CLS / head parameter sums.  The data gradients are bit-identical
+ *          to a run with grads (that chain has no atomics).
+ *   dsrc   NULL, or the gradient w.r.t. src, written by stage n_layers+1: fp32, the shape and layout of src as
+ *          desc->input_layout defines it ([B,C,L] / [B,C,H,W], or [B,L,2] w.r.t. the UN-normalised dataset frames, i.e.
+ *          chained through the fused z-score, 1/std per channel, and the framing).  Overwritten, not accumulated; every
+ *          element is written (samples no patch covers get 0).  The CLS token and the positional encoding contribute
+ *          nothing to it.
+ *   grads and dsrc may not both be NULL. */
+int amc_model_bwd_ex(const AmcDesc* desc, const float* src, const float* params, void* workspace,
+                     const float* dlogits, const float* denc_out,
+                     float* grads, float* dsrc,
+                     int stage_begin, int stage_end, amc_stream_t stream);
 
 /* nn.CrossEntropyLoss(label_smoothing) + argmax statistics (R/training/train.py:260,274-277,504).
  *   stats[0] += sum of per-frame losses * loss_scale, stats[1] += #correct (fp32 accumulators)

@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libamc_b200.so")
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 KIND_RAWIQ, KIND_VIT = 0, 1
 F32, BF16 = 0, 1
 INPUT_MODEL, INPUT_RAW = 0, 1
@@ -59,6 +59,7 @@ def _load():
         "amc_model_workspace": [C.POINTER(AmcDesc), C.POINTER(AmcWorkspaceInfo)],
         "amc_model_fwd": [C.POINTER(AmcDesc), vp, vp, vp, vp, vp, vp, vp],
         "amc_model_bwd": [C.POINTER(AmcDesc), vp, vp, vp, vp, vp, vp, i32, i32, vp],
+        "amc_model_bwd_ex": [C.POINTER(AmcDesc), vp, vp, vp, vp, vp, vp, vp, i32, i32, vp],
         "amc_ce_loss": [i32, i32, vp, vp, f32, f32, f32, vp, vp, vp],
         "amc_argmax": [i32, i32, vp, vp, vp],
         "amc_zero": [vp, C.c_size_t, vp],

@@ -143,6 +143,9 @@ struct Work {
   // backward scratch
   float *dy32, *dw32, *t32, *du32;
   void *dw16, *da, *du16, *dO, *dqkv, *demb;
+  // input gradient: dX [B*Ttok, K] fp32 and (bf16) W_emb^T [K, d]
+  float* dx = nullptr;
+  bf16* wembT = nullptr;
   size_t bytes = 0;
 };
 
@@ -220,6 +223,7 @@ void carve(const AmcDesc& D, const Dims& m, const AmcParamLayout& L, char* base,
     }
   }
   if (D.training) {
+    const size_t dead0 = off;   // dy32 .. dqkv: layer-gradient scratch, dead once stage n_layers+1 has gathered demb
     w.dy32 = (float*)take(M * d * 4);
     w.dw32 = (float*)take(M * d * 4);
     w.t32 = (float*)take(M * d * 4);
@@ -229,6 +233,13 @@ void carve(const AmcDesc& D, const Dims& m, const AmcParamLayout& L, char* base,
     w.du16 = take(M * d * e);
     w.dO = take(M * d * e);
     w.dqkv = take(M * 3 * d * e);
+    // the input gradient's dX and W_emb^T live in that scratch; a buffer of their own only where the patches outgrow it
+    // (patch width K well above d * T / Ttok), so the workspace of every geometry that fits is unchanged
+    const size_t dx_bytes = align_up((size_t)m.B * m.Ttok * m.K * 4, 256);
+    const size_t need = dx_bytes + (bf ? (size_t)m.K * d * 2 : 0);
+    char* dx = need <= off - dead0 ? (base ? base + dead0 : nullptr) : take(need);
+    w.dx = (float*)dx;
+    w.wembT = bf && dx ? (bf16*)(dx + dx_bytes) : nullptr;
     w.demb = take((size_t)m.B * m.Ttok * d * e);
   }
   w.bytes = off;
@@ -271,6 +282,7 @@ struct Model {
   const float* params;
   cudaStream_t st;
   DropoutCfg drop;
+  float* grads = nullptr;   // backward: parameter-gradient blob, NULL = input gradient only
 
   Model(const AmcDesc& D_, const float* params_, cudaStream_t st_) : D(D_), params(params_), st(st_) {}
 
@@ -297,6 +309,9 @@ struct Model {
     return reinterpret_cast<const E*>(params + L.emb_w);
   }
   const LayerBuf& LB(int l) const { return w.lay[D.training ? l : 0]; }
+  // gradient slots (NULL when no parameter gradients are wanted: every parameter output then takes its null path)
+  float* GP(int64_t off) const { return grads ? grads + off : nullptr; }
+  float* GL(int l, int64_t off) const { return grads ? grads + L.layer0 + (int64_t)l * L.layer_stride + off : nullptr; }
   // (amc_gemm_ln also takes 256 < N <= 512 -- one single-buffered 512-column accumulator -- but measured inside the d512 L12
   //  step it loses to GEMM + ln_fwd: 4.97 vs 4.54 ms per step for the two LayerNorm sites, the epilogue of a tile no longer
   //  overlapping the next tile's main loop; the model path therefore fuses up to d = 256 only)
@@ -503,6 +518,7 @@ struct Model {
   // weight-gradient GEMM: dW[No, Ki] += dY[M, No]^T X[M, Ki]
   // ... and db[No] += column sums of dY: inside the same kernel on the bf16 path, a colsum launch in fp32
   int wgrad(int No, int Ki, const void* dY, int ldy, const void* X, int ldx, float* dW, float* db) {
+    if (!dW) return 0;
     if (db && sizeof(E) != 2) AMC_PROF("colsum", 0.0, 0.0, colsum<E>((int)m.M, No, (const E*)dY, ldy, db, st));
     GemmArgs g;
     if (sizeof(E) == 2) g.epi.colsum_out = db;
@@ -527,6 +543,7 @@ struct Model {
 
   // wgrad with an explicit token count (the CLS view has B token rows)
   int wgrad_n(int Ktok, int No, int Ki, const void* dY, int ldy, const void* X, int ldx, float* dW, float* db) {
+    if (!dW) return 0;
     if (db && sizeof(E) != 2) AMC_PROF("colsum", 0.0, 0.0, colsum<E>(Ktok, No, (const E*)dY, ldy, db, st));
     GemmArgs g;
     if (sizeof(E) == 2) g.epi.colsum_out = db;
@@ -541,16 +558,15 @@ struct Model {
 
   // backward of post_fwd_part on the same row view: consumes r.dy32, leaves the out-proj input gradient in
   // r.dO (row pitch r.lddO) and the skip gradient of the layer input in r.du32
-  int post_bwd_part(int l, const Rows& r, float* grads) {
+  int post_bwd_part(int l, const Rows& r) {
     const int d = m.d, F = m.F, Mr = r.n;
     const int64_t dd = (int64_t)d * d;
-    float* G = grads + L.layer0 + (int64_t)l * L.layer_stride;
     GemmArgs g;
     // norm2 backward; dw16 carries dropout2's mask (operand of the FFN2 gradients), dw32 is the skip path
     AMC_PROF("ln_bwd", 0.0, (double)Mr * d * (8 + 2 * sizeof(E)),
-             ln_bwd<E>(Mr, d, r.dy32, (const E*)r.xhat2, r.rstd2, PL(l, L.g2), (E*)r.dw16, r.dw32, G + L.g2, G + L.be2,
-                       G + L.b2, drop, site_ffn(l), st));
-    AMC_TRY(wgrad_n(Mr, d, F, r.dw16, d, r.hid, F, G + L.w2, nullptr));
+             ln_bwd<E>(Mr, d, r.dy32, (const E*)r.xhat2, r.rstd2, PL(l, L.g2), (E*)r.dw16, r.dw32, GL(l, L.g2),
+                       GL(l, L.be2), GL(l, L.b2), drop, site_ffn(l), st));
+    AMC_TRY(wgrad_n(Mr, d, F, r.dw16, d, r.hid, F, GL(l, L.w2), nullptr));
     // dgrad FFN2 with the ReLU/dropout mask taken from the stored hidden
     g.M = Mr; g.N = F; g.K = d; g.A = r.dw16; g.lda = d;
     dgrad_operand(g, l, L.w2, 4 * dd + (int64_t)d * F, d, F);
@@ -558,9 +574,9 @@ struct Model {
     g.epi.mask_src = r.hid; g.epi.ldmask = F; g.epi.mask_scale = drop.scale;
     g.epi.D16 = r.da; g.epi.ldd16 = F;
     const bool fuse_db1 = sizeof(E) == 2 && F % 32 == 0 && F <= 2048;   // bias gradient summed in the mask epilogue
-    if (fuse_db1) g.epi.colsum_out = G + L.b1;
+    if (fuse_db1) g.epi.colsum_out = GL(l, L.b1);
     AMC_TRY(gemm<E>(g, st));
-    AMC_TRY(wgrad_n(Mr, F, d, r.da, F, r.x1_16, d, G + L.w1, fuse_db1 ? nullptr : G + L.b1));
+    AMC_TRY(wgrad_n(Mr, F, d, r.da, F, r.x1_16, d, GL(l, L.w1), fuse_db1 ? nullptr : GL(l, L.b1)));
     // dgrad FFN1 + skip -> gradient w.r.t. x1
     g = GemmArgs();
     g.M = Mr; g.N = d; g.K = F; g.A = r.da; g.lda = F;
@@ -570,9 +586,9 @@ struct Model {
     AMC_TRY(gemm<E>(g, st));
     // norm1 backward
     AMC_PROF("ln_bwd", 0.0, (double)Mr * d * (8 + 2 * sizeof(E)),
-             ln_bwd<E>(Mr, d, r.t32, (const E*)r.xhat1, r.rstd1, PL(l, L.g1), (E*)r.du16, r.du32, G + L.g1, G + L.be1,
-                       G + L.bo, drop, site_attn(l), st));
-    AMC_TRY(wgrad_n(Mr, d, d, r.du16, d, r.o, r.ldo, G + L.wo, nullptr));
+             ln_bwd<E>(Mr, d, r.t32, (const E*)r.xhat1, r.rstd1, PL(l, L.g1), (E*)r.du16, r.du32, GL(l, L.g1),
+                       GL(l, L.be1), GL(l, L.bo), drop, site_attn(l), st));
+    AMC_TRY(wgrad_n(Mr, d, d, r.du16, d, r.o, r.ldo, GL(l, L.wo), nullptr));
     g = GemmArgs();
     g.M = Mr; g.N = d; g.K = d; g.A = r.du16; g.lda = d;
     dgrad_operand(g, l, L.wo, 3 * dd, d, d);
@@ -582,26 +598,25 @@ struct Model {
     return 0;
   }
 
-  int layer_bwd(int l, float* grads, bool cls_only) {
+  int layer_bwd(int l, bool cls_only) {
     const int M = (int)m.M, d = m.d;
     const LayerBuf& b = LB(l);
-    float* G = grads + L.layer0 + (int64_t)l * L.layer_stride;
     const bool cls_kernel = cls_only && cls_attn();
     if (cls_only) {
       // every non-CLS row of the attention-output gradient is exactly zero (the CLS-row kernel never reads them)
       if (!cls_kernel) AMC_CUDA(cudaMemsetAsync(w.dO, 0, (size_t)M * d * sizeof(E), st));
-      AMC_TRY(post_bwd_part(l, cls_rows_view(l), grads));
+      AMC_TRY(post_bwd_part(l, cls_rows_view(l)));
     } else {
-      AMC_TRY(post_bwd_part(l, all_rows(l), grads));
+      AMC_TRY(post_bwd_part(l, all_rows(l)));
     }
     if (cls_kernel) {
       ProfScope ps("attn_cls_bwd", st, 10.0 * m.M * d, (double)M * 5 * d * sizeof(E));
-      AMC_TRY(attn_cls_bwd(m.B, m.T, m.h, m.dh, (const bf16*)b.qkv, (const bf16*)w.dO, (bf16*)w.dqkv, G + L.bq, st));
+      AMC_TRY(attn_cls_bwd(m.B, m.T, m.h, m.dh, (const bf16*)b.qkv, (const bf16*)w.dO, (bf16*)w.dqkv, GL(l, L.bq), st));
     } else {
       ProfScope ps("attn_bwd", st, 10.0 * m.M * m.T * d, (double)M * 7 * d * sizeof(E));
-      AMC_TRY(attention_bwd<E>(m.B, m.T, m.h, m.dh, (const E*)b.qkv, (const E*)b.o, b.lse, (const E*)w.dO, (E*)w.dqkv, G + L.bq, st));
+      AMC_TRY(attention_bwd<E>(m.B, m.T, m.h, m.dh, (const E*)b.qkv, (const E*)b.o, b.lse, (const E*)w.dO, (E*)w.dqkv, GL(l, L.bq), st));
     }
-    AMC_TRY(wgrad(3 * d, d, w.dqkv, 3 * d, w.x16[l], d, G + L.wq, nullptr));
+    AMC_TRY(wgrad(3 * d, d, w.dqkv, 3 * d, w.x16[l], d, GL(l, L.wq), nullptr));
     // dgrad QKV + skip -> gradient w.r.t. the layer input
     GemmArgs g;
     g.M = M; g.N = d; g.K = 3 * d; g.A = w.dqkv; g.lda = 3 * d;
@@ -617,10 +632,39 @@ struct Model {
     return 0;
   }
 
-  int backward(const float* dlogits, const float* denc_out, float* grads, int s0, int s1) {
+  // Input gradient (stage n_layers+1), autograd of the patch embedding and of the dataset z-score + framing:
+  // dX = demb W_emb, then the transpose of the patch map into dsrc (caller's layout, * 1/std_c for dataset input).
+  int input_grad(float* dsrc) {
+    const int Mt = m.B * m.Ttok;
+    if (sizeof(E) == 2 && m.K % 8 != 0) {
+      AMC_PROF("frontend_bwd_dsrc", 2.0 * Mt * m.d * m.K, (double)Mt * (m.d * 2 + m.K * 4),
+               embed_smallk_dgrad(D, m.Ttok, m.d, m.K, (const bf16*)w.demb, (const bf16*)Wemb(), dsrc, st));
+      return 0;
+    }
+    GemmArgs g;
+    g.M = Mt; g.N = m.K; g.K = m.d;
+    g.A = w.demb; g.lda = m.d;
+    if (sizeof(E) == 2) {   // tcgen05 needs both operands K-major: W_emb [d, K] -> [K, d]
+      TransposeBatch tb;
+      tb.n = 1;
+      tb.t[0] = {P(L.emb_w), w.wembT, m.d, m.K, 0};
+      AMC_PROF("frontend_bwd_dsrc", 0.0, (double)m.d * m.K * 6, transpose_batch(tb, st));
+      g.B = w.wembT; g.ldb = m.d;
+    } else {
+      g.B = P(L.emb_w); g.ldb = m.K; g.transB = 1;   // [d, K] read as [K=d, N=K]
+    }
+    g.name = "frontend_bwd_dsrc";
+    g.epi.D32 = w.dx; g.epi.ldd32 = m.K;
+    AMC_TRY(gemm<E>(g, st));
+    AMC_PROF("frontend_bwd_dsrc", 0.0, (double)Mt * m.K * 8, patch_scatter(D, m.Ttok, m.K, w.dx, dsrc, st));
+    return 0;
+  }
+
+  int backward(const float* dlogits, const float* denc_out, float* grads_, float* dsrc, int s0, int s1) {
     AMC_CHECK_ARG(D.training, "amc_model_bwd needs a forward run with desc.training=1");
     AMC_CHECK_ARG(0 <= s0 && s0 <= s1 && s1 <= m.L + 2, "bad stage range [%d,%d)", s0, s1);
     if (m.B == 0) return 0;
+    grads = grads_;
     const size_t nx = (size_t)m.M * m.d;
     const bool cls_top = m.has_cls && dlogits && !denc_out && m.L >= 1;   // must mirror forward()
     for (int s = s0; s < s1; ++s) {
@@ -630,8 +674,8 @@ struct Model {
           AMC_PROF("head", 0.0, 0.0, head_bwd(m.B, cls_top ? 1 : m.T, m.d, m.C, m.has_cls, D.head_ln, dlogits, P(L.head_w),
                            D.head_ln ? P(L.head_ln_w) : nullptr, w.hl, w.hxhat, w.hrstd, w.dhl,
                            cls_top ? w.c.dy32 : w.dy32,
-                           grads + L.head_w, grads + L.head_b, D.head_ln ? grads + L.head_ln_w : nullptr,
-                           D.head_ln ? grads + L.head_ln_b : nullptr, st));
+                           GP(L.head_w), GP(L.head_b), D.head_ln ? GP(L.head_ln_w) : nullptr,
+                           D.head_ln ? GP(L.head_ln_b) : nullptr, st));
           if (denc_out) {
             add_inplace_kernel<<<148 * 4, 256, 0, st>>>(nx, w.dy32, denc_out);
             AMC_LAUNCH_CHECK();
@@ -640,28 +684,29 @@ struct Model {
           AMC_CUDA(cudaMemcpyAsync(w.dy32, denc_out, nx * 4, cudaMemcpyDeviceToDevice, st));
         }
       } else if (s <= m.L) {
-        AMC_TRY(layer_bwd(m.L - s, grads, cls_top && s == 1));
+        AMC_TRY(layer_bwd(m.L - s, cls_top && s == 1));
       } else {
-        // embedding front end: dcls, dW_emb, db_emb (input never needs a gradient: Appendix B)
-        if (m.has_cls) AMC_PROF("frontend_bwd_misc", 0.0, 0.0, cls_grad(m.B, m.T, m.d, w.dy32, grads + L.cls, drop, st));
+        // embedding front end: dcls, dW_emb, db_emb (when parameter gradients are wanted) and the input gradient
+        if (m.has_cls && grads) AMC_PROF("frontend_bwd_misc", 0.0, 0.0, cls_grad(m.B, m.T, m.d, w.dy32, GP(L.cls), drop, st));
         AMC_PROF("frontend_bwd_misc", 0.0, 0.0, gather_tok_rows<E>(m.B, m.T, m.Ttok, m.d, m.has_cls, w.dy32, (E*)w.demb, drop, st));
         const int Mt = m.B * m.Ttok;
-        if (sizeof(E) == 2 && m.K % 8 != 0) {
+        if (grads && sizeof(E) == 2 && m.K % 8 != 0) {
           AMC_PROF("embed_smallk", 2.0 * Mt * m.d * m.K, (double)Mt * (m.K + m.d) * 2,
-                   embed_smallk_bwd(Mt, m.d, m.K, (const bf16*)w.demb, m.d, (const bf16*)w.Apatch, grads + L.emb_w,
-                                    grads + L.emb_b, st));
-        } else {
-          if (sizeof(E) != 2) AMC_PROF("colsum", 0.0, 0.0, colsum<E>(Mt, m.d, (const E*)w.demb, m.d, grads + L.emb_b, st));
+                   embed_smallk_bwd(Mt, m.d, m.K, (const bf16*)w.demb, m.d, (const bf16*)w.Apatch, GP(L.emb_w),
+                                    GP(L.emb_b), st));
+        } else if (grads) {
+          if (sizeof(E) != 2) AMC_PROF("colsum", 0.0, 0.0, colsum<E>(Mt, m.d, (const E*)w.demb, m.d, GP(L.emb_b), st));
           GemmArgs g;
-          if (sizeof(E) == 2) g.epi.colsum_out = grads + L.emb_b;
+          if (sizeof(E) == 2) g.epi.colsum_out = GP(L.emb_b);
           g.M = m.d; g.N = m.K; g.K = Mt;
           g.A = w.demb; g.lda = m.d; g.transA = 1;
           g.B = w.Apatch; g.ldb = m.K; g.transB = 1;
           g.split_k = pick_split_k(m.d, m.K, Mt);
           g.name = "gemm_wgrad";
-          g.epi.D32 = grads + L.emb_w; g.epi.ldd32 = m.K; g.epi.accumulate = 1;
+          g.epi.D32 = GP(L.emb_w); g.epi.ldd32 = m.K; g.epi.accumulate = 1;
           AMC_TRY(gemm<E>(g, st));
         }
+        if (dsrc) AMC_TRY(input_grad(dsrc));
       }
     }
     return 0;
@@ -716,20 +761,28 @@ int amc_model_fwd(const AmcDesc* desc, const float* src, const float* params, co
   return mdl.forward(src, pos, logits, enc_out);
 }
 
-int amc_model_bwd(const AmcDesc* desc, const float* src, const float* params, void* workspace, const float* dlogits,
-                  const float* denc_out, float* grads, int stage_begin, int stage_end, amc_stream_t stream) {
+int amc_model_bwd_ex(const AmcDesc* desc, const float* src, const float* params, void* workspace, const float* dlogits,
+                     const float* denc_out, float* grads, float* dsrc, int stage_begin, int stage_end,
+                     amc_stream_t stream) {
   DeviceGuard dev_guard(params);
-  (void)src;
-  AMC_CHECK_ARG(desc && params && grads, "NULL argument");
+  (void)src;   // the input gradient's shape follows from desc; the kernels never read src in backward
+  AMC_CHECK_ARG(desc && params && (grads || dsrc), "NULL argument");
   cudaStream_t st = (cudaStream_t)stream;
   if (desc->dtype == AMC_BF16) {
     Model<bf16> mdl(*desc, params, st);
     AMC_TRY(mdl.init(workspace));
-    return mdl.backward(dlogits, denc_out, grads, stage_begin, stage_end);
+    return mdl.backward(dlogits, denc_out, grads, dsrc, stage_begin, stage_end);
   }
   Model<float> mdl(*desc, params, st);
   AMC_TRY(mdl.init(workspace));
-  return mdl.backward(dlogits, denc_out, grads, stage_begin, stage_end);
+  return mdl.backward(dlogits, denc_out, grads, dsrc, stage_begin, stage_end);
+}
+
+int amc_model_bwd(const AmcDesc* desc, const float* src, const float* params, void* workspace, const float* dlogits,
+                  const float* denc_out, float* grads, int stage_begin, int stage_end, amc_stream_t stream) {
+  AMC_CHECK_ARG(grads, "NULL argument");
+  return amc_model_bwd_ex(desc, src, params, workspace, dlogits, denc_out, grads, nullptr, stage_begin, stage_end,
+                          stream);
 }
 
 int amc_ce_loss(int B, int C, const float* logits, const int64_t* labels, float label_smoothing, float grad_scale,

@@ -3,10 +3,12 @@
 // A [M, 2] operand has no 16-byte rows for TMA and 2 FLOP per output byte is nothing for a tensor core to do: the
 // forward is an HBM-bound elementwise kernel (x0 = a . W[n, :] + bias + PE, dropout -> fp32 + bf16 rows) that shares
 // the GEMM epilogue, the backward a column reduction (dW[n, k] += sum_m dY[m, n] A[m, k], db[n] += sum_m dY[m, n]).
-// Operands are the same bf16 values the tensor-core path would see, accumulation is fp32.
+// Operands are the same bf16 values the tensor-core path would see, accumulation is fp32.  The input gradient
+// (dX[m, k] = sum_n dY[m, n] W[n, k]) is HBM-bound on reading dY and is written straight into the caller's layout.
 #include <algorithm>
 
 #include "gemm_common.cuh"
+#include "rowops.cuh"
 
 namespace amc {
 namespace {
@@ -60,6 +62,42 @@ __global__ void __launch_bounds__(256) embed_smallk_bwd_kernel(int M, int N, int
   }
 }
 
+// a warp per token row: the row of dY is read once, K <= 16 partial sums per lane are reduced across the warp in a
+// fixed order (no atomics: deterministic), lane k writes element k of the patch through the front end's map
+__global__ void __launch_bounds__(256) embed_smallk_dgrad_kernel(int M, int N, int K, const bf16* __restrict__ dY,
+                                                                 const bf16* __restrict__ W, PatchP p,
+                                                                 float* __restrict__ dsrc) {
+  extern __shared__ float sw[];   // W [N, K] in fp32
+  for (int i = threadIdx.x; i < N * K; i += blockDim.x) sw[i] = to_f(W[i]);
+  __syncthreads();
+  const int lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+  for (int m = blockIdx.x * nw + (threadIdx.x >> 5); m < M; m += gridDim.x * nw) {
+    float acc[SK_MAX];
+#pragma unroll
+    for (int k = 0; k < SK_MAX; ++k) acc[k] = 0.f;
+    for (int n = lane; n < N; n += 32) {
+      const float g = to_f(dY[(size_t)m * N + n]);
+#pragma unroll
+      for (int k = 0; k < SK_MAX; ++k)
+        if (k < K) acc[k] = fmaf(g, sw[n * K + k], acc[k]);
+    }
+    float v = 0.f;
+#pragma unroll
+    for (int k = 0; k < SK_MAX; ++k) {
+      if (k < K) {
+        const float s = warp_sum(acc[k]);
+        if (lane == k) v = s;
+      }
+    }
+    if (lane < K) {
+      const int b = m / p.Ttok, t = m - b * p.Ttok;
+      int ch;
+      const size_t o = patch_src_offset(p, b, t, lane, &ch);
+      dsrc[o] = ch < 0 ? v : v * p.inv_std[ch];
+    }
+  }
+}
+
 }  // namespace
 
 bool embed_smallk_supported(int K) { return K >= 1 && K <= SK_MAX; }
@@ -82,6 +120,20 @@ int embed_smallk_bwd(int M, int N, int K, const bf16* dY, int ldy, const bf16* A
   const int rpb = ceil_div(M, blocks);
   blocks = ceil_div(M, rpb);
   embed_smallk_bwd_kernel<<<blocks, 256, 0, st>>>(M, N, K, dY, ldy, A, dW, db, rpb);
+  AMC_LAUNCH_CHECK();
+  return 0;
+}
+
+int embed_smallk_dgrad(const AmcDesc& D, int Ttok, int N, int K, const bf16* dY, const bf16* W, float* dsrc,
+                       cudaStream_t st) {
+  AMC_CHECK_ARG(embed_smallk_supported(K), "small-K embedding: K=%d unsupported (1..%d)", K, SK_MAX);
+  const int M = D.B * Ttok;
+  if (M == 0) return 0;
+  if ((int64_t)Ttok * K != frame_floats(D))
+    AMC_CUDA(cudaMemsetAsync(dsrc, 0, (size_t)D.B * frame_floats(D) * sizeof(float), st));
+  const int blocks = std::min(ceil_div(M, 8), 148 * 8);
+  embed_smallk_dgrad_kernel<<<blocks, 256, (size_t)N * K * sizeof(float), st>>>(M, N, K, dY, W, make_patchp(D, Ttok, K),
+                                                                                 dsrc);
   AMC_LAUNCH_CHECK();
   return 0;
 }

@@ -143,6 +143,9 @@ int gemm_bf16(const GemmArgs& g, cudaStream_t st);  // gemm_tc.cu (tcgen05)
 bool embed_smallk_supported(int K);
 int embed_smallk_fwd(int M, int N, int K, const bf16* A, const bf16* W, const Epi& epi, cudaStream_t st);
 int embed_smallk_bwd(int M, int N, int K, const bf16* dY, int ldy, const bf16* A, float* dW, float* db, cudaStream_t st);
+// input gradient dsrc (caller's layout per D.input_layout, overwritten) from dY [B*Ttok, N] and W [N, K]
+int embed_smallk_dgrad(const AmcDesc& D, int Ttok, int N, int K, const bf16* dY, const bf16* W, float* dsrc,
+                       cudaStream_t st);
 
 // frontend_tc.cu: fused normalise + frame + patchify + embedding GEMM (+bias, +PE, dropout) for the bf16 path.
 // *handled = false when the geometry is outside what the fused kernel covers (caller: patchify + gemm);

@@ -265,31 +265,6 @@ __global__ void __launch_bounds__(256) colsum_kernel(int M, int N, const E* __re
 // Front end, step 1: dataset z-score + framing + patchify into the embedding GEMM's A operand.
 //   A[b*Ttok + t, k]  (SURVEY §8 a1-a4)
 // ---------------------------------------------------------------------------------------
-struct PatchP {
-  int kind, input_layout, B, Ttok, K, in_ch, seq_len, seg, img_h, img_w, patch;
-  float mean[2], inv_std[2];
-};
-__device__ __forceinline__ float patch_fetch(const PatchP& p, const float* __restrict__ src, int b, int t, int k) {
-  if (p.kind == AMC_KIND_RAWIQ) {
-    const int c = k / p.seg, s = k - c * p.seg;
-    const int pos = t * p.seg + s;
-    if (p.input_layout == AMC_INPUT_MODEL) return __ldg(src + ((size_t)b * p.in_ch + c) * p.seq_len + pos);
-    const float x = __ldg(src + ((size_t)b * p.seq_len + pos) * 2 + c);  // dataset.py:215-222
-    return (x - p.mean[c]) * p.inv_std[c];
-  } else {
-    const int pp = p.patch * p.patch, wp = p.img_w / p.patch;
-    const int c = k / pp, rem = k - c * pp, r = rem / p.patch, cc = rem - r * p.patch;
-    const int ph = t / wp, pw = t - ph * wp;
-    const int y = ph * p.patch + r, x = pw * p.patch + cc;
-    if (p.input_layout == AMC_INPUT_MODEL)
-      return __ldg(src + (((size_t)b * p.in_ch + c) * p.img_h + y) * p.img_w + x);
-    // V/dataloader/dataset.py:216-224: image = cat(I, Q).view(1, H, W)
-    const int L = p.img_h * p.img_w / 2, f = y * p.img_w + x;
-    const int ch = f >= L ? 1 : 0, n = f - ch * L;
-    const float v = __ldg(src + ((size_t)b * L + n) * 2 + ch);
-    return (v - p.mean[ch]) * p.inv_std[ch];
-  }
-}
 template <typename E>
 __global__ void __launch_bounds__(256) patchify_kernel(PatchP p, const float* __restrict__ src, E* __restrict__ A) {
   const size_t total = (size_t)p.B * p.Ttok * p.K;
@@ -297,7 +272,24 @@ __global__ void __launch_bounds__(256) patchify_kernel(PatchP p, const float* __
     const int k = (int)(i % p.K);
     const size_t row = i / p.K;
     const int t = (int)(row % p.Ttok), b = (int)(row / p.Ttok);
-    A[i] = from_f<E>(patch_fetch(p, src, b, t, k));
+    int ch;
+    const float x = __ldg(src + patch_src_offset(p, b, t, k, &ch));
+    A[i] = from_f<E>(ch < 0 ? x : (x - p.mean[ch]) * p.inv_std[ch]);
+  }
+}
+
+// Input gradient, last step: the transpose of patchify.  d(x - mean) * inv_std / dx = inv_std in dataset layout.
+__global__ void __launch_bounds__(256) patch_scatter_kernel(PatchP p, const float* __restrict__ dX,
+                                                            float* __restrict__ dsrc) {
+  const size_t total = (size_t)p.B * p.Ttok * p.K;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    const int k = (int)(i % p.K);
+    const size_t row = i / p.K;
+    const int t = (int)(row % p.Ttok), b = (int)(row / p.Ttok);
+    int ch;
+    const size_t o = patch_src_offset(p, b, t, k, &ch);
+    const float g = dX[i];
+    dsrc[o] = ch < 0 ? g : g * p.inv_std[ch];
   }
 }
 
@@ -832,7 +824,7 @@ template int ln_bwd<bf16>(int, int, const float*, const bf16*, const float*, con
                           float*, float*, const DropoutCfg&, uint32_t, cudaStream_t);
 
 
-static PatchP make_patchp(const AmcDesc& D, int Ttok, int K) {
+PatchP make_patchp(const AmcDesc& D, int Ttok, int K) {
   PatchP p;
   p.kind = D.kind;
   p.input_layout = D.input_layout;
@@ -877,6 +869,17 @@ int patchify(const AmcDesc& D, int Ttok, int K, const float* src, E* A, cudaStre
 }
 template int patchify<float>(const AmcDesc&, int, int, const float*, float*, cudaStream_t);
 template int patchify<bf16>(const AmcDesc&, int, int, const float*, bf16*, cudaStream_t);
+
+int patch_scatter(const AmcDesc& D, int Ttok, int K, const float* dX, float* dsrc, cudaStream_t st) {
+  if (D.B == 0) return 0;
+  if ((int64_t)Ttok * K != frame_floats(D))
+    AMC_CUDA(cudaMemsetAsync(dsrc, 0, (size_t)D.B * frame_floats(D) * sizeof(float), st));
+  const size_t total = (size_t)D.B * Ttok * K;
+  const int blocks = (int)std::min<size_t>((total + 255) / 256, 148 * 16);
+  patch_scatter_kernel<<<blocks, 256, 0, st>>>(make_patchp(D, Ttok, K), dX, dsrc);
+  AMC_LAUNCH_CHECK();
+  return 0;
+}
 
 template <typename E>
 int cls_rows(int B, int T, int d, const float* cls, const float* pos, E* y16, float* y32, const DropoutCfg& drop,
@@ -954,8 +957,9 @@ int head_bwd(int B, int T, int d, int C, int has_cls, int head_ln, const float* 
              float* dxL, float* dW, float* dbias, float* dlnw, float* dlnb, cudaStream_t st) {
   if (B == 0) return 0;
   head_bwd_rows_kernel<<<ceil_div(B, 4), 128, 0, st>>>(B, T, d, C, has_cls, head_ln, dlogits, W, lnw, s_xhat,
-                                                       s_rstd, dxL, dhl_scratch);
+                                                       s_rstd, dxL, dW ? dhl_scratch : nullptr);
   AMC_LAUNCH_CHECK();
+  if (!dW) return 0;   // input gradient only: no parameter outputs
   const int chunks = ceil_div(B, 32);       // 32 rows per block (the kernel's shared-memory staging size)
   head_bwd_params_kernel<<<dim3(ceil_div(d, 128), chunks), 128, 0, st>>>(B, d, C, head_ln, dlogits, s_hl, dhl_scratch, s_xhat,
                                                               dW, dbias, dlnw, dlnb);

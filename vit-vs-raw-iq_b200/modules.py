@@ -147,8 +147,10 @@ class PositionalEncoding(_ParamContainer):
 # the autograd boundary
 # ----------------------------------------------------------------------------------------------
 class _EncoderPathFn(torch.autograd.Function):
-    """forward = amc_model_fwd, backward = amc_model_bwd.  ``params`` are passed only so autograd
-    routes gradients to them; the kernels read the flat blob they are views of."""
+    """forward = amc_model_fwd, backward = amc_model_bwd_ex.  ``params`` are passed only so autograd
+    routes gradients to them; the kernels read the flat blob they are views of.  The input gradient (``src.grad``,
+    saliency maps, adversarial examples) comes out of the same backward; when no parameter needs a gradient (a frozen
+    model) the backward runs the data-gradient chain alone, without weight-gradient GEMMs or a gradient blob."""
 
     @staticmethod
     def forward(ctx, owner, src, want_logits, need_grad, *params):
@@ -171,16 +173,19 @@ class _EncoderPathFn(torch.autograd.Function):
     def backward(ctx, dout):
         core = ctx.owner._core
         dout = dout.contiguous().float()
-        grads = torch.zeros(core.layout.total, dtype=torch.float32, device=dout.device)
+        # a partially frozen model still gets every parameter gradient; only a fully frozen one skips them
+        want_params = any(ctx.needs_input_grad[4:])
+        grads = torch.zeros(core.layout.total, dtype=torch.float32, device=dout.device) if want_params else None
+        dsrc = torch.empty_like(ctx.src) if ctx.needs_input_grad[1] else None
         stream = torch.cuda.current_stream(dout.device).cuda_stream
         dl = dout.data_ptr() if ctx.want_logits else 0
         de = 0 if ctx.want_logits else dout.data_ptr()
-        _lib.check(_lib.lib.amc_model_bwd(C.byref(ctx.desc), ctx.src.data_ptr(), core.flat.data_ptr(),
-                                          ctx.ws.data_ptr(), dl, de, grads.data_ptr(), 0,
-                                          core.n_layers + 2, stream), "amc_model_bwd")
+        _lib.check(_lib.lib.amc_model_bwd_ex(C.byref(ctx.desc), ctx.src.data_ptr(), core.flat.data_ptr(),
+                                             ctx.ws.data_ptr(), dl, de, _lib.ptr(grads), _lib.ptr(dsrc), 0,
+                                             core.n_layers + 2, stream), "amc_model_bwd_ex")
         ctx.ws = None
-        views = [grads[o:o + n].view(shape) for (o, n, shape) in core.slots]
-        return (None, None, None, None, *views)
+        views = [grads[o:o + n].view(shape) for (o, n, shape) in core.slots] if want_params else [None] * len(core.slots)
+        return (None, dsrc, None, None, *views)
 
 
 class _Core:
@@ -362,7 +367,7 @@ class _AMCBase(nn.Module):
 
     def _run(self, src, want_logits):
         # grad mode is switched off inside Function.forward, so decide here whether to keep activations
-        need_grad = torch.is_grad_enabled() and any(p.requires_grad for p in self._core.params)
+        need_grad = torch.is_grad_enabled() and (src.requires_grad or any(p.requires_grad for p in self._core.params))
         return _EncoderPathFn.apply(self, src, want_logits, need_grad, *self._core.params)
 
 
