@@ -152,7 +152,9 @@ int amc_model_bwd_ex(const AmcDesc* desc, const float* src, const float* params,
  *   stats[0] += sum of per-frame losses * loss_scale, stats[1] += #correct (fp32 accumulators)
  *   dlogits = (softmax - smoothed one-hot) * grad_scale   (grad_scale = 1/global_batch)
  *   labels: device int64 [B].  A label outside [0, C) -- where the reference raises -- makes that frame's loss NaN, so
- *   stats[0] is NaN from then on and the host mirror raises when it reads the statistics. */
+ *   stats[0] is NaN from then on and the host mirror raises when it reads the statistics; that frame is not counted in
+ *   stats[1] and its dlogits row uses the all-smoothing target (softmax - ls/C) * grad_scale.
+ *   dlogits and stats may each be NULL. */
 int amc_ce_loss(int B, int C, const float* logits, const int64_t* labels, float label_smoothing,
                 float grad_scale, float loss_scale, float* dlogits, float* stats, amc_stream_t stream);
 
@@ -166,8 +168,9 @@ int amc_zero(void* p, size_t bytes, amc_stream_t stream);
 
 /* clip_grad_norm_(max_norm) + AdamW.step fused over the flat blobs (R/training/train.py:266-271,506-511).
  * grads are first multiplied by grad_scale (1/world_size after an all-reduce SUM).  norm_ws: >= 2 floats
- * of device scratch (zeroed by the call); norm_ws[1] holds the pre-clip global norm afterwards.
- * max_norm <= 0 disables clipping. */
+ * of device scratch; with clipping (max_norm > 0) the call zeroes it and norm_ws[1] holds the pre-clip global norm of
+ * grad_scale * grads afterwards.  max_norm <= 0 disables clipping: no norm is computed and norm_ws is neither read
+ * nor written. */
 int amc_adamw_clip_step(int64_t n, float* params, float* grads, float* exp_avg, float* exp_avg_sq,
                         float lr, float beta1, float beta2, float eps, float weight_decay,
                         float max_norm, float grad_scale, int64_t step, float* norm_ws,

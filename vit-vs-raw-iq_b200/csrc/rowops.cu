@@ -594,10 +594,13 @@ __global__ void ce_loss_kernel(int B, int C, const float* __restrict__ logits, c
     for (int k = 0; k < C; ++k) se += expf(z[k] - mx);
     const float lse = logf(se);
     const int64_t y64 = labels[b];
-    const int y = (int)y64;
     // nn.CrossEntropyLoss raises on a target outside [0, C); an asynchronous kernel cannot, so the frame's loss becomes
-    // NaN: the running loss statistic is NaN from then on and the host raises when it reads it (trainer.read_stats)
-    const float poison = (y64 < 0 || y64 >= (int64_t)C) ? __int_as_float(0x7fc00000) : 0.f;
+    // NaN: the running loss statistic is NaN from then on and the host raises when it reads it (trainer.read_stats).
+    // Such a frame matches no class (y = -1): it is never counted correct -- a label of 2^32 + 3 truncated to 32 bits
+    // would otherwise read as class 3 -- and its gradient has the all-smoothing target.
+    const bool valid = y64 >= 0 && y64 < (int64_t)C;
+    const int y = valid ? (int)y64 : -1;
+    const float poison = valid ? 0.f : __int_as_float(0x7fc00000);
     float sum_logp = 0.f;
     for (int k = 0; k < C; ++k) {
       const float logp = z[k] - mx - lse;
