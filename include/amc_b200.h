@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AMC_ABI_VERSION 7
+#define AMC_ABI_VERSION 8
 
 enum { AMC_KIND_RAWIQ = 0, AMC_KIND_VIT = 1 };
 enum { AMC_F32 = 0, AMC_BF16 = 1 };
@@ -189,6 +189,31 @@ int amc_adamw_clip_step_graph(int64_t n, float* params, float* grads, float* exp
  * frames x [n_frames, frame_len, 2] fp32, acc4 (device, fp64, zeroed by the caller) += {sum I, sum I^2, sum Q,
  * sum Q^2}.  mean = s/n, unbiased std = sqrt((ss - s^2/n)/(n-1)), floored at 1e-8 like the reference. */
 int amc_iq_stats(int64_t n_frames, int64_t frame_len, const float* x, double* acc4, amc_stream_t stream);
+
+/* ---- projected-gradient adversarial attacks (FGSM / PGD) -------------------------------
+ * A frame is the n contiguous fp32 values the model reads for one example in the caller's input layout: [C,L] /
+ * [1,H,W] model layout, or [L,2] dataset layout, in which case the attack works on the physical, un-normalised IQ
+ * samples.  Frames start 16-byte aligned only when n % 4 == 0; other sizes take a scalar path.  A targeted attack needs
+ * no flag here: amc_ce_loss with grad_scale = -1 and the target labels makes the step descend the target's loss. */
+enum { AMC_NORM_LINF = 0, AMC_NORM_L2 = 1 };
+
+/* One projected-gradient ascent step on B frames of n floats (x updated in place):
+ *   a_b = step_frac * eps[b]                                  (one fp32 multiply)
+ *   LINF: x = min(max(x + a_b * sign(g), x0 - eps[b]), x0 + eps[b])      sign(0) = 0
+ *   L2:   v = x + a_b * g / ||g_b||  (v = x when ||g_b|| = 0);  d = v - x0;
+ *         x = ||d|| > eps[b] ? x0 + d * (eps[b] / ||d||) : v
+ * The L2 norms are fp32 tree reductions inside the CTA that owns the frame (deterministic, one launch).
+ * x0, g, x: device fp32 [B, n]; eps: device fp32 [B], >= 0 (eps[b] = 0 gives exactly x0). */
+int amc_adv_step(int64_t B, int64_t n, int norm, const float* x0, const float* g, const float* eps,
+                 float step_frac, float* x, amc_stream_t stream);
+
+/* Random start: x = x0 + a draw from the norm ball of radius eps[b]
+ *   LINF: eps[b] * (2u - 1) per element, u in [0,1) from 24 hash bits
+ *   L2:   eps[b] * r * z / ||z||, z standard normal per element, r = u^(1/n) per frame
+ * keyed by (seed, offset + *step_counter, element index b*n+i) with the dropout counter hash (its own site constants).
+ * step_counter: device or NULL, as in AmcDesc, so a captured CUDA graph draws a fresh start on every replay. */
+int amc_adv_init(int64_t B, int64_t n, int norm, const float* x0, const float* eps, uint64_t seed,
+                 uint64_t offset, const uint32_t* step_counter, float* x, amc_stream_t stream);
 
 /* ---- operator-level calls (used by the block tests; the whole-path calls are built from
  *      the same kernels) ------------------------------------------------------------- */

@@ -6,5 +6,6 @@ importable name onto this directory).  Importing this package loads the in-tree 
 """
 from . import _lib  # noqa: F401  (loads the shared library; raises ImportError if missing)
 from .modules import (RawIQAMCTransformer, ViTAMCTransformer, default_compute_dtype)  # noqa: F401
+from .adversarial import PGDAttack  # noqa: F401
 
-__all__ = ["RawIQAMCTransformer", "ViTAMCTransformer", "default_compute_dtype"]
+__all__ = ["RawIQAMCTransformer", "ViTAMCTransformer", "default_compute_dtype", "PGDAttack"]

@@ -12,10 +12,11 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libamc_b200.so")
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 KIND_RAWIQ, KIND_VIT = 0, 1
 F32, BF16 = 0, 1
 INPUT_MODEL, INPUT_RAW = 0, 1
+NORM_LINF, NORM_L2 = 0, 1
 
 
 class AmcDesc(C.Structure):
@@ -66,6 +67,8 @@ def _load():
         "amc_adamw_clip_step": [i64, vp, vp, vp, vp, f32, f32, f32, f32, f32, f32, f32, i64, vp, vp],
         "amc_adamw_clip_step_graph": [i64, vp, vp, vp, vp, f32, f32, f32, f32, f32, f32, f32, vp, vp, vp],
         "amc_iq_stats": [i64, i64, vp, vp, vp],
+        "amc_adv_step": [i64, i64, i32, vp, vp, vp, f32, vp, vp],
+        "amc_adv_init": [i64, i64, i32, vp, vp, C.c_uint64, C.c_uint64, vp, vp, vp],
         "amc_gemm": [i32, i32, i32, i32, vp, i32, i32, vp, i32, i32, vp, vp, i32, i32, vp, i32, vp, i32, i32, vp],
         "amc_gemm_ln": [i32, i32, i32, vp, i32, vp, i32, vp, vp, vp, vp, f32, vp, vp, vp, vp, vp],
         "amc_gemm_relu_mask": [i32, i32, i32, vp, i32, vp, i32, vp, f32, vp, vp],

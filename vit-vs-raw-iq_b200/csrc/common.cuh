@@ -118,12 +118,12 @@ inline DropoutCfg make_dropout(float p, uint64_t seed, uint64_t offset, bool tra
 // not the tensor pipe, bound the K = 256 GEMMs.  Statistics (4M groups, p in {0.1, 0.2, 0.5}): drop rate of every
 // field within 3e-4 of p; |correlation| between fields, neighbouring groups, rows, seeds, steps and sites < 2e-3.
 // Dropout only needs an unbiased, well-mixed keep decision per element; it is not a cryptographic stream.
-// keep-multipliers (0 or scale) for elements [4*q4, 4*q4+4) of dropout site `site`
-__device__ __forceinline__ float4 dropout_mult4(const DropoutCfg& c, uint32_t site, uint64_t q4) {
+// the two hash words (h, b) of counter q under key (seed, offset + *ctr, site)
+__device__ __forceinline__ uint2 counter_hash2(const DropoutCfg& c, uint32_t site, uint64_t q) {
   const uint32_t off = c.off_lo + (c.ctr != nullptr ? __ldg(c.ctr) : 0u);
   const uint32_t key = c.seed_lo ^ (off * 0x9E3779B9u) ^ (site * 0x85EBCA6Bu) ^ (c.seed_hi * 0x27D4EB2Fu) ^
                        (c.off_hi * 0x165667B1u);                                        // loop-invariant
-  uint32_t h = (uint32_t)q4 * 0x9E3779B1u + ((uint32_t)(q4 >> 32) * 0x7FEB352Du + key);
+  uint32_t h = (uint32_t)q * 0x9E3779B1u + ((uint32_t)(q >> 32) * 0x7FEB352Du + key);
   h ^= h >> 16;                                   // murmur3 finaliser: keys that differ in one bit (seed, step, site)
   h *= 0x85EBCA6Bu;                               // must give uncorrelated masks -- a single multiply left 10 %
   h ^= h >> 13;                                   // correlation between neighbouring seeds
@@ -131,6 +131,12 @@ __device__ __forceinline__ float4 dropout_mult4(const DropoutCfg& c, uint32_t si
   h ^= h >> 16;
   uint32_t b = h * 0x27D4EB2Fu;                   // second word derived from the first
   b ^= b >> 15;
+  return make_uint2(h, b);
+}
+// keep-multipliers (0 or scale) for elements [4*q4, 4*q4+4) of dropout site `site`
+__device__ __forceinline__ float4 dropout_mult4(const DropoutCfg& c, uint32_t site, uint64_t q4) {
+  const uint2 hb = counter_hash2(c, site, q4);
+  const uint32_t h = hb.x, b = hb.y;
   const uint32_t t = c.thresh & 0xFFFF0000u;      // keep iff the 16-bit field >= thresh >> 16
   return make_float4((h << 16) >= t ? c.scale : 0.f, h >= t ? c.scale : 0.f, (b << 16) >= t ? c.scale : 0.f,
                      b >= t ? c.scale : 0.f);
@@ -142,6 +148,9 @@ __host__ __device__ __forceinline__ uint32_t site_pe() { return 0; }
 __host__ __device__ __forceinline__ uint32_t site_attn(int l) { return 1 + 3 * l; }
 __host__ __device__ __forceinline__ uint32_t site_hidden(int l) { return 2 + 3 * l; }
 __host__ __device__ __forceinline__ uint32_t site_ffn(int l) { return 3 + 3 * l; }
+// random starts of projected-gradient attacks (adversarial.cu): far above every dropout site (n_layers is small)
+__host__ __device__ __forceinline__ uint32_t site_adv_elem() { return 0xADF00000u; }
+__host__ __device__ __forceinline__ uint32_t site_adv_radius() { return 0xADF00001u; }
 
 // Every entry point runs on the device that owns its buffers, whatever the caller's current device is (a model on
 // cuda:1 while cuda:0 is current is plain `.to(device)` usage in the reference): kernels, cudaFuncSetAttribute and tensor-

@@ -53,9 +53,15 @@ def _report_from_confusion(cm: np.ndarray, class_names: Sequence[str], digits: i
 @torch.no_grad()
 def evaluate_model_with_confusion(model: _AMCBase, batches: Iterable[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]],
                                   class_names: List[str], save_dir, prefix: str = "test",
-                                  device: Optional[torch.device] = None) -> Dict:
+                                  device: Optional[torch.device] = None, attack=None) -> Dict:
     """``batches`` yields (images, labels, snrs) like the reference DataLoader (host tensors, or device tensors).
-    Returns overall / per-SNR accuracy and confusion matrices and writes ``{prefix}_classification_report.txt``."""
+    Returns overall / per-SNR accuracy and confusion matrices and writes ``{prefix}_classification_report.txt``.
+
+    ``attack`` (an ``adversarial.PGDAttack`` on ``model``): robust evaluation.  Each batch is moved to the device and
+    replaced by ``attack(images, labels)`` before the prediction; the report has the same format."""
+    if attack is not None and attack.model is not model:
+        raise ValueError("the attack must be bound to the model being evaluated (a transfer attack crafts the frames "
+                         "beforehand and evaluates them without attack=)")
     save_dir = Path(save_dir)
     save_dir.mkdir(parents=True, exist_ok=True)
     model.eval()
@@ -76,6 +82,8 @@ def evaluate_model_with_confusion(model: _AMCBase, batches: Iterable[Tuple[torch
             cm_snr[s].add_(torch.bincount(idx[sel], minlength=C * C))
 
     for images, labels, snrs in batches:
+        if attack is not None:      # the attack runs no autograd, so no_grad does not get in its way
+            images = attack(images.to(dev, non_blocking=True).contiguous(), labels.to(dev, non_blocking=True))
         if images.is_cuda:
             account(predict(model, images.contiguous()), labels, snrs)
             continue

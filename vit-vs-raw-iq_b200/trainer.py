@@ -18,12 +18,29 @@ from . import _lib
 from .modules import _AMCBase, _DTYPES
 
 
+def _check_labels(labels, B: int, dev: torch.device) -> None:
+    # the kernel reads `labels` as B contiguous int64 on the model's device: anything else is an out-of-bounds or
+    # garbage device read (nn.CrossEntropyLoss raises in these cases too)
+    if not (isinstance(labels, torch.Tensor) and labels.is_cuda and labels.device == dev):
+        raise ValueError(f"labels must be a CUDA tensor on {dev}")
+    if labels.dtype != torch.int64 or labels.dim() != 1 or labels.numel() != B or not labels.is_contiguous():
+        raise ValueError(f"labels must be a contiguous int64 tensor of shape [{B}], got {labels.dtype} "
+                         f"{tuple(labels.shape)}")
+
+
 class TrainStep:
     def __init__(self, model: _AMCBase, lr: float = 1e-4, weight_decay: float = 1e-4, betas=(0.9, 0.99),
                  eps: float = 1e-8, max_norm: float = 1.0, label_smoothing: float = 0.1,
-                 process_group=None, layers_per_bucket: int = 2, data_parallel: bool = True):
+                 process_group=None, layers_per_bucket: int = 2, data_parallel: bool = True, attack=None):
         """``data_parallel=False``: train this model on this rank alone even though ``torch.distributed`` is initialised
-        (rank-sharded hyper-parameter search: every rank holds DIFFERENT models, so no collective may be issued)."""
+        (rank-sharded hyper-parameter search: every rank holds DIFFERENT models, so no collective may be issued).
+
+        ``attack`` (an ``adversarial.PGDAttack`` on this model): adversarial training.  Each step first replaces the batch
+        by ``attack(src, labels)`` against the current parameters, reusing the step's workspace, then runs the unchanged
+        step on it (PGD training; ``steps=1, step_frac=1.25`` with a random start is "fast" FGSM-RS training)."""
+        if attack is not None and attack.model is not model:
+            raise ValueError("the attack must be bound to the model this TrainStep trains")
+        self.attack = attack
         self.model = model
         self.core = model._core
         self.lr, self.wd, self.betas, self.eps = lr, weight_decay, betas, eps
@@ -95,16 +112,12 @@ class TrainStep:
         self.model.train()
         desc = core.make_desc(src, training=True, module_training=True)
         B = desc.B
-        # the kernel reads `labels` as B contiguous int64 on the model's device: anything else is an out-of-bounds or
-        # garbage device read (nn.CrossEntropyLoss raises in these cases too)
-        if not (isinstance(labels, torch.Tensor) and labels.is_cuda and labels.device == self.dev):
-            raise ValueError(f"labels must be a CUDA tensor on {self.dev}")
-        if labels.dtype != torch.int64 or labels.dim() != 1 or labels.numel() != B or not labels.is_contiguous():
-            raise ValueError(f"labels must be a contiguous int64 tensor of shape [{B}], got {labels.dtype} "
-                             f"{tuple(labels.shape)}")
+        _check_labels(labels, B, self.dev)
         if src.device != self.dev:
             raise ValueError(f"src is on {src.device}, the model on {self.dev}")
         ws, logits, dlogits = self._buffers(B, desc)
+        if self.attack is not None:               # stream order: the attack is done before the forward reuses `ws`
+            src = self.attack._run(src, labels, ws)
         flat = self.model.flat_parameters()
         st = torch.cuda.current_stream(self.dev).cuda_stream
         lib = _lib.lib
@@ -178,6 +191,8 @@ class GraphTrainStep(TrainStep):
         desc = core.make_desc(src, training=True, module_training=True)
         B = desc.B
         ws, logits, dlogits = self._buffers(B, desc)
+        if self.attack is not None:               # captured too: the random start reads the device step counter
+            src = self.attack._run(src, labels, ws)
         flat = self.model.flat_parameters()
         st = torch.cuda.current_stream(self.dev).cuda_stream
         lib = _lib.lib
@@ -197,11 +212,7 @@ class GraphTrainStep(TrainStep):
     def step(self, src: torch.Tensor, labels: torch.Tensor) -> None:
         self.model.train()
         B = int(src.shape[0])
-        if not (isinstance(labels, torch.Tensor) and labels.is_cuda and labels.device == self.dev):
-            raise ValueError(f"labels must be a CUDA tensor on {self.dev}")
-        if labels.dtype != torch.int64 or labels.dim() != 1 or labels.numel() != B or not labels.is_contiguous():
-            raise ValueError(f"labels must be a contiguous int64 tensor of shape [{B}], got {labels.dtype} "
-                             f"{tuple(labels.shape)}")
+        _check_labels(labels, B, self.dev)
         key = (tuple(src.shape), src.dtype, self.core.compute_dtype, self.core.drop_prob > 0)
         if self._gkey != key:                              # new shape: this call runs eagerly, the next one captures
             self._graph, self._gkey = None, key
