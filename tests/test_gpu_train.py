@@ -283,21 +283,29 @@ def test_labels_are_validated_like_cross_entropy_loss():
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 def test_model_on_a_non_current_device():
     """The reference's plain `.to(device)` usage: model and batch on cuda:1 while cuda:0 is the current device (ADVICE r1:
-    the ABI switches to the device that owns the buffers)."""
+    the ABI switches to the device that owns the buffers).  bf16 runs the tcgen05 kernels, whose shared-memory attributes are
+    per device: a bf16 forward on cuda:0 comes first, so cuda:1 must get them too."""
     z, params, grads, _ = load_golden("vit_p16")
     torch.cuda.set_device(0)
     dev1 = torch.device("cuda", 1)
     kind, kw = GOLDEN_CASES["vit_p16"]
-    model = amc.ViTAMCTransformer(**kw, drop_prob=0.0, device=dev1, compute_dtype="fp32")
-    model.load_state_dict({k: torch.from_numpy(v) for k, v in params.items()}, strict=True)
-    src = torch.from_numpy(z["src"]).to(dev1)
-    labels = torch.from_numpy(z["labels"]).to(dev1)
-    assert torch.cuda.current_device() == 0
-    ts = TrainStep(model, lr=1e-3)
-    ts.step(src, labels)
-    loss, _ = ts.read_stats()
-    assert abs(loss - float(z["loss"])) < 1e-4
-    assert torch.cuda.current_device() == 0
+    state = {k: torch.from_numpy(v) for k, v in params.items()}
+    model0 = amc.ViTAMCTransformer(**kw, drop_prob=0.0, device=DEV, compute_dtype="bf16")
+    model0.load_state_dict(state, strict=True)
+    with torch.no_grad():
+        model0(torch.from_numpy(z["src"]).to(DEV))
+    torch.cuda.synchronize(0)
+    for dtype, tol in (("fp32", 1e-4), ("bf16", 2e-2)):
+        model = amc.ViTAMCTransformer(**kw, drop_prob=0.0, device=dev1, compute_dtype=dtype)
+        model.load_state_dict(state, strict=True)
+        src = torch.from_numpy(z["src"]).to(dev1)
+        labels = torch.from_numpy(z["labels"]).to(dev1)
+        assert torch.cuda.current_device() == 0
+        ts = TrainStep(model, lr=1e-3)
+        ts.step(src, labels)
+        loss, _ = ts.read_stats()
+        assert abs(loss - float(z["loss"])) < tol, dtype
+        assert torch.cuda.current_device() == 0
 
 
 @pytest.mark.parametrize("name,dtype", [("rawiq_seg16", "fp32"), ("vit_p16", "bf16")])

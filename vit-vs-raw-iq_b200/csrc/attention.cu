@@ -20,6 +20,7 @@
 #include <cstdlib>
 
 #include "attention.cuh"
+#include "ptx.cuh"
 #include "rowops.cuh"
 
 #include <type_traits>
@@ -259,54 +260,21 @@ __device__ __forceinline__ void rows_copy(E* smem_blk, int smem_stride, E* gmem_
 }
 
 // ---- 1-D bulk (TMA) row copies: one elected thread moves whole rows, completion on an mbarrier ----
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init1(uint64_t* bar) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(bar)));
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_parity(uint64_t* bar, uint32_t parity) {
-  uint32_t ok = 0, spins = 0;
-  while (!ok) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_addr(bar)), "r"(parity)
-        : "memory");
-    if (!ok && ++spins > (1u << 24)) __trap();
-  }
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   smem_addr(dst)),
-               "l"(src), "r"(bytes), "r"(smem_addr(bar))
-               : "memory");
-}
-__device__ __forceinline__ void bulk_s2g(void* dst, const void* src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_addr(src)), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_all0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 // load `rows` dense global rows into padded smem rows (called by ONE thread)
 template <typename E>
 __device__ __forceinline__ void bulk_rows_in(E* smem_blk, int smem_stride, const E* gmem_blk, int rows, int row_elems,
                                              uint64_t* bar) {
   const uint32_t rb = (uint32_t)(row_elems * sizeof(E));
-  mbar_expect(bar, rb * (uint32_t)rows);
-  for (int r = 0; r < rows; ++r) bulk_g2s(smem_blk + (size_t)r * smem_stride, gmem_blk + (size_t)r * row_elems, rb, bar);
+  mbar_expect_tx(bar, rb * (uint32_t)rows);
+  for (int r = 0; r < rows; ++r)
+    bulk_g2s(smem_u32(smem_blk + (size_t)r * smem_stride), gmem_blk + (size_t)r * row_elems, rb, bar);
 }
 template <typename E>
 __device__ __forceinline__ void bulk_rows_out(E* gmem_blk, const E* smem_blk, int smem_stride, int rows, int row_elems) {
   const uint32_t rb = (uint32_t)(row_elems * sizeof(E));
-  for (int r = 0; r < rows; ++r) bulk_s2g(gmem_blk + (size_t)r * row_elems, smem_blk + (size_t)r * smem_stride, rb);
-  bulk_commit_group();
+  for (int r = 0; r < rows; ++r)
+    bulk_s2g(gmem_blk + (size_t)r * row_elems, smem_u32(smem_blk + (size_t)r * smem_stride), rb);
+  bulk_commit();
 }
 
 // row (<= 32 elements) <-> registers; only the first nq float4 are live
@@ -362,8 +330,10 @@ __global__ void __launch_bounds__(256) attn_frames_fwd_kernel(int B, int T, int 
   const int hT = h * T;
   const int f = tid / hT, rem = tid - f * hT, hh = rem / T, i = rem - hh * T;
   if (tid == 0) {
-    mbar_init1(bars);
-    mbar_init1(bars + 1);
+    mbar_init(bars, 1);
+    fence_barrier_init();
+    mbar_init(bars + 1, 1);
+    fence_barrier_init();
   }
   __syncthreads();
   const int stride_f = gridDim.x * F;
@@ -377,7 +347,7 @@ __global__ void __launch_bounds__(256) attn_frames_fwd_kernel(int B, int T, int 
       if (fn < B) bulk_rows_in(blk0 + ((it + 1) & 1) * in_elems, s_in, qkv + (size_t)fn * T * ld, min(F, B - fn) * T, ld,
                                bars + ((it + 1) & 1));
     }
-    mbar_wait_parity(bars + (it & 1), (it >> 1) & 1);
+    mbar_wait(bars + (it & 1), (it >> 1) & 1);
     float4 o[8];
     if (f < nf) {
       const E* fb = blk + (size_t)f * T * s_in + hh * dh;
@@ -402,14 +372,14 @@ __global__ void __launch_bounds__(256) attn_frames_fwd_kernel(int B, int T, int 
       for (int j = 0; j < MAXT; ++j)
         if (j < T) row_axpy(o, s[j] * inv, fb + (size_t)j * s_in + 2 * d, nq);
     }
-    if (tid == 0) bulk_wait_read0();          // previous iteration's output rows have left oblk
+    if (tid == 0) bulk_wait_read<0>();          // previous iteration's output rows have left oblk
     __syncthreads();                          // ... and everyone is done reading blk (it may be refilled next iteration)
     if (f < nf) row_store(oblk + ((size_t)f * T + i) * s_out + hh * dh, o, nq);
-    fence_async_smem();
+    fence_proxy_async();
     __syncthreads();
     if (tid == 0) bulk_rows_out(out + (size_t)f0 * T * d, oblk, s_out, nf * T, d);
   }
-  if (tid == 0) bulk_wait_all0();
+  if (tid == 0) bulk_wait_all();
 }
 
 template <typename E, int MAXT>
@@ -427,21 +397,24 @@ __global__ void __launch_bounds__(256) attn_frames_bwd_kernel(int B, int T, int 
   const int tid = threadIdx.x;
   const int hT = h * T;
   const int f = tid / hT, rem = tid - f * hT, hh = rem / T, i = rem - hh * T;
-  if (tid == 0) mbar_init1(bar);
+  if (tid == 0) {
+    mbar_init(bar, 1);
+    fence_barrier_init();
+  }
   __syncthreads();
   const int stride_f = gridDim.x * F;
   int f0 = blockIdx.x * F;
   if (tid == 0 && f0 < B) {
     const int rows = min(F, B - f0) * T;
-    mbar_expect(bar, (uint32_t)(rows * (ld + d) * sizeof(E)));
+    mbar_expect_tx(bar, (uint32_t)(rows * (ld + d) * sizeof(E)));
     for (int r = 0; r < rows; ++r) {
-      bulk_g2s(blk + (size_t)r * s_in, qkv + ((size_t)f0 * T + r) * ld, (uint32_t)(ld * sizeof(E)), bar);
-      bulk_g2s(doblk + (size_t)r * s_do, dout + ((size_t)f0 * T + r) * d, (uint32_t)(d * sizeof(E)), bar);
+      bulk_g2s(smem_u32(blk + (size_t)r * s_in), qkv + ((size_t)f0 * T + r) * ld, (uint32_t)(ld * sizeof(E)), bar);
+      bulk_g2s(smem_u32(doblk + (size_t)r * s_do), dout + ((size_t)f0 * T + r) * d, (uint32_t)(d * sizeof(E)), bar);
     }
   }
   for (uint32_t it = 0; f0 < B; f0 += stride_f, ++it) {
     const int nf = min(F, B - f0);
-    mbar_wait_parity(bar, it & 1);
+    mbar_wait(bar, it & 1);
     const bool act = f < nf;
     const E* fb = blk + (size_t)(act ? f : 0) * T * s_in + hh * dh;          // q at +0, k at +d, v at +2d
     const E* fo = doblk + (size_t)(act ? f : 0) * T * s_do + hh * dh;
@@ -489,16 +462,16 @@ __global__ void __launch_bounds__(256) attn_frames_bwd_kernel(int B, int T, int 
         row_axpy(dv, P[j * (T + 1) + i], fo + (size_t)j * s_do, nq);
       }
     }
-    if (tid == 0) bulk_wait_read0();          // previous iteration's gradient rows have left oblk
+    if (tid == 0) bulk_wait_read<0>();          // previous iteration's gradient rows have left oblk
     __syncthreads();                          // every read of q/k/v/dO is done: inputs may be refilled
     if (tid == 0) {
       const int fn = f0 + stride_f;
       if (fn < B) {
         const int rows = min(F, B - fn) * T;
-        mbar_expect(bar, (uint32_t)(rows * (ld + d) * sizeof(E)));
+        mbar_expect_tx(bar, (uint32_t)(rows * (ld + d) * sizeof(E)));
         for (int r = 0; r < rows; ++r) {
-          bulk_g2s(blk + (size_t)r * s_in, qkv + ((size_t)fn * T + r) * ld, (uint32_t)(ld * sizeof(E)), bar);
-          bulk_g2s(doblk + (size_t)r * s_do, dout + ((size_t)fn * T + r) * d, (uint32_t)(d * sizeof(E)), bar);
+          bulk_g2s(smem_u32(blk + (size_t)r * s_in), qkv + ((size_t)fn * T + r) * ld, (uint32_t)(ld * sizeof(E)), bar);
+          bulk_g2s(smem_u32(doblk + (size_t)r * s_do), dout + ((size_t)fn * T + r) * d, (uint32_t)(d * sizeof(E)), bar);
         }
       }
     }
@@ -508,11 +481,11 @@ __global__ void __launch_bounds__(256) attn_frames_bwd_kernel(int B, int T, int 
       row_store(ob + d, dk, nq);
       row_store(ob + 2 * d, dv, nq);
     }
-    fence_async_smem();
+    fence_proxy_async();
     __syncthreads();
     if (tid == 0) bulk_rows_out(dqkv + (size_t)f0 * T * ld, oblk, s_in, nf * T, ld);
   }
-  if (tid == 0) bulk_wait_all0();
+  if (tid == 0) bulk_wait_all();
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -524,24 +497,6 @@ __global__ void __launch_bounds__(256) attn_frames_bwd_kernel(int B, int T, int 
 // needed (dK = dS^T Q, dV = P^T dO).  Rows/keys >= T are padding: their addresses are clamped to row T-1,
 // key columns are masked to -inf, query rows are zeroed in backward and never written.
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void ldsm_x4(uint32_t (&r)[4], uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ void ldsm_x4_t(uint32_t (&r)[4], uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ void mma_bf16(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, "
-               "{%0, %1, %2, %3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ uint32_t pack2(float a, float b) {
-  __nv_bfloat162 t = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&t);
-}
 // A-operand address (rows r0.., 16 columns at col0) / "K-pattern" B address (rows = n, cols = k) for lane
 __device__ __forceinline__ uint32_t addr_a(uint32_t base, int pitch_b, int T, int col0, int lane) {
   const int r = min((lane & 7) + ((lane >> 3) & 1) * 8, T - 1);
@@ -609,8 +564,10 @@ __global__ void __launch_bounds__(256) attn_mma_fwd_kernel(int B, int T, int h, 
   bf16* oblk = blk0 + 2 * in_elems;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nw = blockDim.x >> 5;
   if (tid == 0) {
-    mbar_init1(bars);
-    mbar_init1(bars + 1);
+    mbar_init(bars, 1);
+    fence_barrier_init();
+    mbar_init(bars + 1, 1);
+    fence_barrier_init();
   }
   __syncthreads();
   const int stride_f = gridDim.x * F;
@@ -619,9 +576,9 @@ __global__ void __launch_bounds__(256) attn_mma_fwd_kernel(int B, int T, int h, 
   // iteration cost about a quarter of it.  Thread 0 arms the barrier with the byte count, the copies may land first.
   auto rows_in = [&](bf16* dst, int fs, uint64_t* bar) {      // called by lane 0 of each warp
     const int rows = min(F, B - fs) * T;
-    if (warp == 0) mbar_expect(bar, (uint32_t)(rows * ld * 2));
+    if (warp == 0) mbar_expect_tx(bar, (uint32_t)(rows * ld * 2));
     for (int r = warp; r < rows; r += nw)
-      bulk_g2s(dst + (size_t)r * s_in, qkv + ((size_t)fs * T + r) * ld, (uint32_t)(ld * 2), bar);
+      bulk_g2s(smem_u32(dst + (size_t)r * s_in), qkv + ((size_t)fs * T + r) * ld, (uint32_t)(ld * 2), bar);
   };
   if (lane == 0 && f0 < B) rows_in(blk0, f0, bars);
   for (uint32_t it = 0; f0 < B; f0 += stride_f, ++it) {
@@ -630,13 +587,13 @@ __global__ void __launch_bounds__(256) attn_mma_fwd_kernel(int B, int T, int h, 
     if (lane == 0) {
       const int fn = f0 + stride_f;
       if (fn < B) rows_in(blk0 + ((it + 1) & 1) * in_elems, fn, bars + ((it + 1) & 1));
-      bulk_wait_read0();                       // this warp's output rows of the previous iteration have left oblk
+      bulk_wait_read<0>();                       // this warp's output rows of the previous iteration have left oblk
     }
-    mbar_wait_parity(bars + (it & 1), (it >> 1) & 1);
+    mbar_wait(bars + (it & 1), (it >> 1) & 1);
     __syncthreads();
     for (int pr = warp; pr < nf * h; pr += nw) {
       const int f = pr / h, hh = pr - f * h;
-      const uint32_t qb = smem_addr(blk + (size_t)f * T * s_in + hh * dh);
+      const uint32_t qb = smem_u32(blk + (size_t)f * T * s_in + hh * dh);
       const uint32_t kb = qb + d * 2, vb = qb + 2 * d * 2;
       float c[2][4] = {};
 #pragma unroll
@@ -666,15 +623,15 @@ __global__ void __launch_bounds__(256) attn_mma_fwd_kernel(int B, int T, int h, 
         if (g + 8 < T) *reinterpret_cast<uint32_t*>(ob + (size_t)(g + 8) * s_out + nt * 8) = pack2(o[nt][2], o[nt][3]);
       }
     }
-    fence_async_smem();
+    fence_proxy_async();
     __syncthreads();
     if (lane == 0) {
       for (int r = warp; r < nf * T; r += nw)
-        bulk_s2g(out + ((size_t)f0 * T + r) * d, oblk + (size_t)r * s_out, (uint32_t)(d * 2));
-      bulk_commit_group();
+        bulk_s2g(out + ((size_t)f0 * T + r) * d, smem_u32(oblk + (size_t)r * s_out), (uint32_t)(d * 2));
+      bulk_commit();
     }
   }
-  if (lane == 0) bulk_wait_all0();
+  if (lane == 0) bulk_wait_all();
 }
 
 template <int KD>
@@ -695,17 +652,20 @@ __global__ void __launch_bounds__(256) attn_mma_bwd_kernel(int B, int T, int h, 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nw = blockDim.x >> 5;
   bf16* tP = tiles + (size_t)warp * 2 * 16 * TP;
   bf16* tS = tP + 16 * TP;
-  if (tid == 0) mbar_init1(bar);
+  if (tid == 0) {
+    mbar_init(bar, 1);
+    fence_barrier_init();
+  }
   __syncthreads();
   const int stride_f = gridDim.x * F;
   int f0 = blockIdx.x * F;
   // row copies dealt round-robin to lane 0 of every warp (see the forward kernel); thread 0 arms the barrier
   auto issue = [&](int fs) {                                  // called by lane 0 of each warp
     const int rows = min(F, B - fs) * T;
-    if (warp == 0) mbar_expect(bar, (uint32_t)(rows * (ld + d) * 2));
+    if (warp == 0) mbar_expect_tx(bar, (uint32_t)(rows * (ld + d) * 2));
     for (int r = warp; r < rows; r += nw) {
-      bulk_g2s(blk + (size_t)r * s_in, qkv + ((size_t)fs * T + r) * ld, (uint32_t)(ld * 2), bar);
-      bulk_g2s(doblk + (size_t)r * s_do, dout + ((size_t)fs * T + r) * d, (uint32_t)(d * 2), bar);
+      bulk_g2s(smem_u32(blk + (size_t)r * s_in), qkv + ((size_t)fs * T + r) * ld, (uint32_t)(ld * 2), bar);
+      bulk_g2s(smem_u32(doblk + (size_t)r * s_do), dout + ((size_t)fs * T + r) * d, (uint32_t)(d * 2), bar);
     }
   };
   if (lane == 0 && f0 < B) issue(f0);
@@ -715,15 +675,15 @@ __global__ void __launch_bounds__(256) attn_mma_bwd_kernel(int B, int T, int h, 
   const int ngroups = ld >> 2;
   for (uint32_t it = 0; f0 < B; f0 += stride_f, ++it) {
     const int nf = min(F, B - f0);
-    if (lane == 0) bulk_wait_read0();         // this warp's gradient rows of the previous iteration have left oblk
-    mbar_wait_parity(bar, it & 1);
+    if (lane == 0) bulk_wait_read<0>();         // this warp's gradient rows of the previous iteration have left oblk
+    mbar_wait(bar, it & 1);
     __syncthreads();
     const int g = lane >> 2, cb = (lane & 3) * 2;
     for (int pr = warp; pr < nf * h; pr += nw) {
       const int f = pr / h, hh = pr - f * h;
-      const uint32_t qb = smem_addr(blk + (size_t)f * T * s_in + hh * dh);
+      const uint32_t qb = smem_u32(blk + (size_t)f * T * s_in + hh * dh);
       const uint32_t kb = qb + d * 2, vb = qb + 2 * d * 2;
-      const uint32_t ob = smem_addr(doblk + (size_t)f * T * s_do + hh * dh);
+      const uint32_t ob = smem_u32(doblk + (size_t)f * T * s_do + hh * dh);
       float c[2][4] = {}, dp[2][4] = {};
 #pragma unroll
       for (int ks = 0; ks < KD; ++ks) {
@@ -777,8 +737,8 @@ __global__ void __launch_bounds__(256) attn_mma_bwd_kernel(int B, int T, int h, 
       uint32_t pta[4], sta[4];     // A fragments of P^T and dS^T: rows = keys, k = queries
       {
         const int r = (lane & 7) + (lane >> 4) * 8, cc = ((lane >> 3) & 1) * 8;
-        ldsm_x4_t(pta, smem_addr(tP + r * TP + cc));
-        ldsm_x4_t(sta, smem_addr(tS + r * TP + cc));
+        ldsm_x4_t(pta, smem_u32(tP + r * TP + cc));
+        ldsm_x4_t(sta, smem_u32(tS + r * TP + cc));
       }
       bf16* og = oblk + (size_t)f * T * s_in + hh * dh + cb;
 #pragma unroll
@@ -810,12 +770,12 @@ __global__ void __launch_bounds__(256) attn_mma_bwd_kernel(int B, int T, int h, 
         }
       }
     }
-    fence_async_smem();
+    fence_proxy_async();
     __syncthreads();                          // all reads of q/k/v/dO done, all gradient rows staged
     if (lane == 0) {
       for (int r = warp; r < nf * T; r += nw)
-        bulk_s2g(dqkv + ((size_t)f0 * T + r) * ld, oblk + (size_t)r * s_in, (uint32_t)(ld * 2));
-      bulk_commit_group();
+        bulk_s2g(dqkv + ((size_t)f0 * T + r) * ld, smem_u32(oblk + (size_t)r * s_in), (uint32_t)(ld * 2));
+      bulk_commit();
       const int fn = f0 + stride_f;
       if (fn < B) issue(fn);
     }
@@ -843,7 +803,7 @@ __global__ void __launch_bounds__(256) attn_mma_bwd_kernel(int B, int T, int h, 
       }
     }
   }
-  if (lane == 0) bulk_wait_all0();
+  if (lane == 0) bulk_wait_all();
 }
 
 inline bool use_mma(int T, int h, int dh) {

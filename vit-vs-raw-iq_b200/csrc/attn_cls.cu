@@ -10,29 +10,24 @@
 // The q / v bias gradients are dq_0 and dO_0 summed over frames (sum_j p_j = 1); the k bias gradient is exactly 0
 // (sum_j ds_j = 0: the dead parameter of SURVEY Appendix B).
 #include "attention.cuh"
+#include "ptx.cuh"
 
 namespace amc {
 namespace {
 
 constexpr int KPL_MAX = 9;     // keys per lane: T <= 288 with 32-lane groups
 
-__device__ __forceinline__ float lo16(uint32_t w) { return __uint_as_float(w << 16); }
-__device__ __forceinline__ float hi16(uint32_t w) { return __uint_as_float(w & 0xFFFF0000u); }
-__device__ __forceinline__ uint32_t pk2(float a, float b) {
-  __nv_bfloat162 t = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&t);
-}
 __device__ __forceinline__ float dot8(const uint4& a, const uint4& b) {
-  return lo16(a.x) * lo16(b.x) + hi16(a.x) * hi16(b.x) + lo16(a.y) * lo16(b.y) + hi16(a.y) * hi16(b.y) +
-         lo16(a.z) * lo16(b.z) + hi16(a.z) * hi16(b.z) + lo16(a.w) * lo16(b.w) + hi16(a.w) * hi16(b.w);
+  return bf_lo(a.x) * bf_lo(b.x) + bf_hi(a.x) * bf_hi(b.x) + bf_lo(a.y) * bf_lo(b.y) + bf_hi(a.y) * bf_hi(b.y) +
+         bf_lo(a.z) * bf_lo(b.z) + bf_hi(a.z) * bf_hi(b.z) + bf_lo(a.w) * bf_lo(b.w) + bf_hi(a.w) * bf_hi(b.w);
 }
 __device__ __forceinline__ void axpy8(float (&o)[8], float a, const uint4& x) {
-  o[0] = fmaf(a, lo16(x.x), o[0]); o[1] = fmaf(a, hi16(x.x), o[1]); o[2] = fmaf(a, lo16(x.y), o[2]); o[3] = fmaf(a, hi16(x.y), o[3]);
-  o[4] = fmaf(a, lo16(x.z), o[4]); o[5] = fmaf(a, hi16(x.z), o[5]); o[6] = fmaf(a, lo16(x.w), o[6]); o[7] = fmaf(a, hi16(x.w), o[7]);
+  o[0] = fmaf(a, bf_lo(x.x), o[0]); o[1] = fmaf(a, bf_hi(x.x), o[1]); o[2] = fmaf(a, bf_lo(x.y), o[2]); o[3] = fmaf(a, bf_hi(x.y), o[3]);
+  o[4] = fmaf(a, bf_lo(x.z), o[4]); o[5] = fmaf(a, bf_hi(x.z), o[5]); o[6] = fmaf(a, bf_lo(x.w), o[6]); o[7] = fmaf(a, bf_hi(x.w), o[7]);
 }
 __device__ __forceinline__ uint4 scale8(float a, const uint4& x) {
-  return make_uint4(pk2(a * lo16(x.x), a * hi16(x.x)), pk2(a * lo16(x.y), a * hi16(x.y)), pk2(a * lo16(x.z), a * hi16(x.z)),
-                    pk2(a * lo16(x.w), a * hi16(x.w)));
+  return make_uint4(pack2(a * bf_lo(x.x), a * bf_hi(x.x)), pack2(a * bf_lo(x.y), a * bf_hi(x.y)), pack2(a * bf_lo(x.z), a * bf_hi(x.z)),
+                    pack2(a * bf_lo(x.w), a * bf_hi(x.w)));
 }
 template <int GS> __device__ __forceinline__ float group_sum(float v) {
 #pragma unroll
@@ -122,7 +117,7 @@ __global__ void __launch_bounds__(256) attn_cls_fwd_kernel(int B, int T, int h, 
       // every lane holds every sum; lane gl stores chunk gl (selected without dynamic register indexing)
 #pragma unroll
       for (int c = 0; c < C8; ++c)
-        if (c == gl) w = make_uint4(pk2(o[c][0], o[c][1]), pk2(o[c][2], o[c][3]), pk2(o[c][4], o[c][5]), pk2(o[c][6], o[c][7]));
+        if (c == gl) w = make_uint4(pack2(o[c][0], o[c][1]), pack2(o[c][2], o[c][3]), pack2(o[c][4], o[c][5]), pack2(o[c][6], o[c][7]));
       *(reinterpret_cast<uint4*>(out + (size_t)b * T * d + hh * dh) + gl) = w;
     }
   }
@@ -209,9 +204,9 @@ __global__ void __launch_bounds__(256) attn_cls_bwd_kernel(int B, int T, int h, 
       for (int c = 0; c < C8; ++c)
         if (c == gl) {
           *(reinterpret_cast<uint4*>(gbase) + gl) =
-              make_uint4(pk2(dq[c][0], dq[c][1]), pk2(dq[c][2], dq[c][3]), pk2(dq[c][4], dq[c][5]), pk2(dq[c][6], dq[c][7]));
-          const float g8[8] = {lo16(go[c].x), hi16(go[c].x), lo16(go[c].y), hi16(go[c].y),
-                               lo16(go[c].z), hi16(go[c].z), lo16(go[c].w), hi16(go[c].w)};
+              make_uint4(pack2(dq[c][0], dq[c][1]), pack2(dq[c][2], dq[c][3]), pack2(dq[c][4], dq[c][5]), pack2(dq[c][6], dq[c][7]));
+          const float g8[8] = {bf_lo(go[c].x), bf_hi(go[c].x), bf_lo(go[c].y), bf_hi(go[c].y),
+                               bf_lo(go[c].z), bf_hi(go[c].z), bf_lo(go[c].w), bf_hi(go[c].w)};
 #pragma unroll
           for (int e = 0; e < 8; ++e) { bq[e] += dq[c][e]; bv[e] += g8[e]; }
           my_head = hh;
@@ -300,7 +295,7 @@ __global__ void __launch_bounds__(256) attn_cls_long_fwd_kernel(int B, int T, in
       uint4 wv = make_uint4(0u, 0u, 0u, 0u);
 #pragma unroll
       for (int c = 0; c < C8; ++c)
-        if (c == lane) wv = make_uint4(pk2(o[c][0], o[c][1]), pk2(o[c][2], o[c][3]), pk2(o[c][4], o[c][5]), pk2(o[c][6], o[c][7]));
+        if (c == lane) wv = make_uint4(pack2(o[c][0], o[c][1]), pack2(o[c][2], o[c][3]), pack2(o[c][4], o[c][5]), pack2(o[c][6], o[c][7]));
       *(reinterpret_cast<uint4*>(out + (size_t)b * T * d + hh * dh) + lane) = wv;
     }
   }
@@ -389,10 +384,10 @@ __global__ void __launch_bounds__(256) attn_cls_long_bwd_kernel(int B, int T, in
       for (int c = 0; c < C8; ++c)
         if (c == lane) {
           *(reinterpret_cast<uint4*>(gbase) + lane) =
-              make_uint4(pk2(dq[c][0], dq[c][1]), pk2(dq[c][2], dq[c][3]), pk2(dq[c][4], dq[c][5]), pk2(dq[c][6], dq[c][7]));
+              make_uint4(pack2(dq[c][0], dq[c][1]), pack2(dq[c][2], dq[c][3]), pack2(dq[c][4], dq[c][5]), pack2(dq[c][6], dq[c][7]));
           if (dbias) {
-            const float g8[8] = {lo16(go[c].x), hi16(go[c].x), lo16(go[c].y), hi16(go[c].y),
-                                 lo16(go[c].z), hi16(go[c].z), lo16(go[c].w), hi16(go[c].w)};
+            const float g8[8] = {bf_lo(go[c].x), bf_hi(go[c].x), bf_lo(go[c].y), bf_hi(go[c].y),
+                                 bf_lo(go[c].z), bf_hi(go[c].z), bf_lo(go[c].w), bf_hi(go[c].w)};
 #pragma unroll
             for (int e = 0; e < 8; ++e) {
               atomicAdd(&sbias[hh * dh + lane * 8 + e], dq[c][e]);

@@ -20,8 +20,6 @@
 namespace amc {
 namespace {
 
-using namespace attn_ptx;
-
 constexpr float LOG2E = 1.4426950408889634f;
 constexpr float LN2 = 0.6931471805599453f;
 
@@ -380,7 +378,7 @@ attn_long_mma_fwd_kernel(const __grid_constant__ CUtensorMap mOwn, const __grid_
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~(uintptr_t)1023);
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem);     // [0] own tile, [1], [2] stream stages
-  const uint32_t qtile = s_u32(smem + M_HDR), st0 = qtile + OWN_B;
+  const uint32_t qtile = smem_u32(smem + M_HDR), st0 = qtile + OWN_B;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int g = lane >> 2, cb = (lane & 3) * 2;
   const int T = gm.T;
@@ -483,7 +481,7 @@ attn_long_mma_dq_kernel(const __grid_constant__ CUtensorMap mOwn, const __grid_c
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~(uintptr_t)1023);
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem);
-  const uint32_t qtile = s_u32(smem + M_HDR), gtile = qtile + OWN_B, st0 = gtile + OWN_B;
+  const uint32_t qtile = smem_u32(smem + M_HDR), gtile = qtile + OWN_B, st0 = gtile + OWN_B;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int g = lane >> 2, cb = (lane & 3) * 2;
   const int T = gm.T;
@@ -592,9 +590,9 @@ attn_long_mma_dkdv_kernel(const __grid_constant__ CUtensorMap mOwn, const __grid
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~(uintptr_t)1023);
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem);
-  const uint32_t ktile = s_u32(smem + M_HDR), vtile = ktile + OWN_B, st0 = vtile + OWN_B;
+  const uint32_t ktile = smem_u32(smem + M_HDR), vtile = ktile + OWN_B, st0 = vtile + OWN_B;
   float2* s_stat = reinterpret_cast<float2*>(smem + M_HDR + 2 * OWN_B + 6 * CH_B);    // [M_CR] {lse2, delta * scale}
-  const uint32_t stat_u = s_u32(s_stat);
+  const uint32_t stat_u = smem_u32(s_stat);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nt = blockDim.x;
   const int g = lane >> 2, cb = (lane & 3) * 2;
   const int T = gm.T;

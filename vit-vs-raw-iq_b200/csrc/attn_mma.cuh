@@ -1,111 +1,13 @@
-// PTX helpers of the mma.sync / TMA attention kernels (attn_tiles.cu, attn_long.cu): mbarrier + TMA tensor copies,
-// ldmatrix / mma.sync / movmatrix wrappers and the swizzled-tile addressing both files share.
+// Building blocks of the mma.sync / TMA attention kernels (attn_tiles.cu, attn_long.cu, and the leftover rows of
+// attn_tc5.cu): the swizzled-tile addressing and the forward chunk of a 16-query-row item.
 #pragma once
-#include <cuda.h>
-
-#include "common.cuh"
+#include "ptx.cuh"
 
 namespace amc {
 // bf16 tensor [B][T][cols] (row pitch = cols) as a 3-D TMA map, box = {dh, box_rows, 1}, swizzle span = dh * 2 bytes
 int attn_make_map3(CUtensorMap* map, const void* base, int B, int T, int cols, int dh, int box_rows);
-int attn_sm_count();
 
-namespace attn_ptx {
-
-// ---- PTX helpers -----------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t s_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(s_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(s_u32(bar)), "r"(bytes) : "memory");
-}
-// Bounded wait: a protocol bug must surface as a trap (launch error), never as a hung GPU.
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t ok = 0, spins = 0;
-  while (!ok) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(s_u32(bar)), "r"(parity)
-        : "memory");
-    if (!ok && ++spins > (1u << 24)) __trap();
-  }
-}
-__device__ __forceinline__ void tma_load_3d(const CUtensorMap* map, uint64_t* bar, uint32_t dst, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(dst), "l"(map), "r"(s_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, uint32_t src, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(map), "r"(src),
-               "r"(c0), "r"(c1), "r"(c2)
-               : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
-  asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_all0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-__device__ __forceinline__ void ldsm_x4(uint32_t (&r)[4], uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ void ldsm_x4_t(uint32_t (&r)[4], uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ void mma_bf16(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, "
-               "{%0, %1, %2, %3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ uint32_t movm_t(uint32_t a) {   // 8x8 b16 transpose across the warp
-  uint32_t d;
-  asm volatile("movmatrix.sync.aligned.m8n8.trans.b16 %0, %1;" : "=r"(d) : "r"(a));
-  return d;
-}
-__device__ __forceinline__ uint32_t pack2(float a, float b) {
-  __nv_bfloat162 t = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&t);
-}
-__device__ __forceinline__ float ex2(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-__device__ __forceinline__ void sts32(uint32_t addr, uint32_t v) { asm volatile("st.shared.b32 [%0], %1;" ::"r"(addr), "r"(v) : "memory"); }
-__device__ __forceinline__ void sts128(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-__device__ __forceinline__ uint4 lds128(uint32_t addr) {
-  uint4 v;
-  asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
-  return v;
-}
-__device__ __forceinline__ float2 lds64f(uint32_t addr) {
-  float2 v;
-  asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(addr));
-  return v;
-}
-__device__ __forceinline__ float4 lds128f(uint32_t addr) {
-  float4 v;
-  asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
-  return v;
-}
-__device__ __forceinline__ void sts64f(uint32_t addr, float a, float b) {
-  asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(addr), "f"(a), "f"(b) : "memory");
-}
-__device__ __forceinline__ float bf_lo(uint32_t w) { return __uint_as_float(w << 16); }
-__device__ __forceinline__ float bf_hi(uint32_t w) { return __uint_as_float(w & 0xFFFF0000u); }
+namespace {
 
 // ---- swizzled tile addressing --------------------------------------------------------------------------------
 // A tile is Tpad rows of RB = 32*KD bytes written by TMA with SWIZZLE_{32,64,128}B: the 16-byte chunk index is
@@ -202,5 +104,5 @@ __device__ __forceinline__ void fwd_chunk(uint32_t kb, uint32_t vb, int k0, int 
   }
 }
 
-}  // namespace attn_ptx
+}  // namespace
 }  // namespace amc

@@ -32,11 +32,10 @@
 
 #include "attention.cuh"
 #include "attn_mma.cuh"
-#include "tc_ptx.cuh"
+#include "ptx.cuh"
 
 namespace amc {
 namespace {
-namespace ap = attn_ptx;
 
 struct Tc5Geom {
   int T, Tk, NT, rem, Tmain;      // tokens, keys padded to 16, 128-row main tiles per unit, leftover rows, main rows
@@ -51,90 +50,8 @@ struct Tc5Geom {
 
 constexpr int TC5_HDR = 4096;     // mbarriers + TMEM slot (256 B), then the split-row exchange: [max | sum][half][128 rows] floats
 
-// ---- PTX not in tc_ptx.cuh ------------------------------------------------------------------------------------
-// shared-memory matrix descriptor with an explicit swizzle mode (2 = 128B, 4 = 64B, 6 = 32B)
-__device__ __forceinline__ uint64_t make_desc_sw(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t layout) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)layout << 61;
-  return d;
-}
+// UMMA swizzle layout of a tile whose rows are 32 * KD bytes (make_smem_desc: 6 = 32B, 4 = 64B, 2 = 128B)
 template <int KD> __device__ __forceinline__ constexpr uint32_t sw_layout() { return KD == 1 ? 6u : (KD == 2 ? 4u : 2u); }
-// kind::f16 instruction descriptor: fp32 accumulate, bf16 operands, separate operand majors (1 = MN-major)
-__host__ __device__ constexpr uint32_t make_idesc2(int M, int N, int a_mn, int b_mn) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) |
-         ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-// D[tmem] (+)= A[tmem] * B[smem]
-__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc,
-                                             uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&r)[8]) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait8(uint32_t (&r)[8]) {
-  asm volatile("tcgen05.wait::ld.sync.aligned;"
-               : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7])
-               :
-               : "memory");
-}
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait5() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-// tcgen05.wait::ld that also names the destination registers, so no use of them can be scheduled above the wait
-__device__ __forceinline__ void tmem_ld_wait32(uint32_t (&r)[32]) {
-  asm volatile("tcgen05.wait::ld.sync.aligned;"
-               : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]),
-                 "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]),
-                 "+r"(r[16]), "+r"(r[17]), "+r"(r[18]), "+r"(r[19]), "+r"(r[20]), "+r"(r[21]), "+r"(r[22]), "+r"(r[23]),
-                 "+r"(r[24]), "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31])
-               :
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait16(uint32_t (&r)[16]) {
-  asm volatile("tcgen05.wait::ld.sync.aligned;"
-               : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]),
-                 "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15])
-               :
-               : "memory");
-}
-
-// One lane of a converged warp.  The MMA issuer WARPS run their loops with all 32 lanes (warp-uniform control flow, so the
-// descriptors stay in uniform registers) and put only the tcgen05 instructions under this predicate: issued from inside
-// an `if (lane == 0)` region every MMA costs a register-to-uniform waterfall and ~45 issue cycles on an idle SM against
-// 14 (A in TMEM) .. 34 (A in shared memory) for this form (tools/probes/umma_probe.cu).
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(pred));
-  return pred != 0;
-}
 
 // ===============================================================================================================
 // Forward
@@ -200,9 +117,9 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
     // ============================ MMA issuer warp (all lanes run the loop, one elected lane issues) ============================
     {
       // descriptors differ only in the 14-bit start-address field: build the constant halves once
-      constexpr uint32_t idPV = make_idesc2(128, dh, 0, 1);
-      const uint64_t hiK = make_desc_sw(0, 16, SBO, LAY), hiV = make_desc_sw(0, SBO, SBO, LAY);
-      const uint32_t idS0 = make_idesc2(128, min(256, Tk), 0, 0), idS1 = make_idesc2(128, max(16, Tk - 256), 0, 0);
+      constexpr uint32_t idPV = make_idesc(128, dh, 0, 1);
+      const uint64_t hiK = make_smem_desc(0, 16, SBO, LAY), hiV = make_smem_desc(0, SBO, SBO, LAY);
+      const uint32_t idS0 = make_idesc(128, min(256, Tk), 0, 0), idS1 = make_idesc(128, max(16, Tk - 256), 0, 0);
       const int npv = Tk / 16;
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
       int it = 0, s = 0;
@@ -262,12 +179,12 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
         const int col = hh * dh;
         mbar_expect_tx(bars->full + s, (uint32_t)(NT * RM * RB + 2 * Tk * RB + (has_lo ? 16 * RB : 0)));
         for (int t = 0; t < NT; ++t)
-          ap::tma_load_3d(&mQ, bars->full + s, q_tile(s) + (uint32_t)(t * 128 * RB), col, t * 128, b);
-        if (has_lo) ap::tma_load_3d(&mQlo, bars->full + s, qlo_tile(s), col, gm.Tmain, b);
+          tma_load_3d(&mQ, bars->full + s, q_tile(s) + (uint32_t)(t * 128 * RB), col, t * 128, b);
+        if (has_lo) tma_load_3d(&mQlo, bars->full + s, qlo_tile(s), col, gm.Tmain, b);
         for (int bx = 0; bx < gm.kbox_n; ++bx) {
           const uint32_t off = (uint32_t)(bx * gm.kbox_rows * RB);
-          ap::tma_load_3d(&mKV, bars->full + s, k_tile(s) + off, gm.d + col, bx * gm.kbox_rows, b);
-          ap::tma_load_3d(&mKV, bars->full + s, v_tile(s) + off, 2 * gm.d + col, bx * gm.kbox_rows, b);
+          tma_load_3d(&mKV, bars->full + s, k_tile(s) + off, gm.d + col, bx * gm.kbox_rows, b);
+          tma_load_3d(&mKV, bars->full + s, v_tile(s) + off, 2 * gm.d + col, bx * gm.kbox_rows, b);
         }
       };
       for (int k = 0; k < NST; ++k)
@@ -278,11 +195,11 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
         const int b = u / gm.h, hh = u - b * gm.h;
         mbar_wait(bars->o_staged + s, ph);                    // every softmax warp has staged its rows of this unit
         tr(trace, 1, it, 0);
-        for (int t = 0; t < NT; ++t) ap::tma_store_3d(&mO, q_tile(s) + (uint32_t)(t * 128 * RB), hh * dh, t * 128, b);
-        ap::bulk_commit();
+        for (int t = 0; t < NT; ++t) tma_store_3d(&mO, q_tile(s) + (uint32_t)(t * 128 * RB), hh * dh, t * 128, b);
+        bulk_commit();
         const int un = u + NST * (int)gridDim.x;
         if (un < gm.units) {
-          ap::bulk_wait_read0();                              // the store has read the staging rows
+          bulk_wait_read<0>();                              // the store has read the staging rows
           tr(trace, 1, it, 1);
           mbar_wait(bars->empty + s, ph);                     // MMAs (and the leftover warp) are done with K / V
           tr(trace, 1, it, 2);
@@ -290,7 +207,7 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
         }
         if (++s == NST) { s = 0; ph ^= 1; }
       }
-      ap::bulk_wait_all0();
+      bulk_wait_all();
     }
   } else if (warp == NSW + 1) {
     // ============================ leftover rows: one mma.sync 16-row block per unit ============================
@@ -307,14 +224,14 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
         const uint32_t qb = qlo_tile(s), kb = k_tile(s), vb = v_tile(s);
         uint32_t aq[KD][4];
 #pragma unroll
-        for (int ks = 0; ks < KD; ++ks) ap::ldsm_x4(aq[ks], ap::addrA<KD>(qb, 0, ks, lane));
+        for (int ks = 0; ks < KD; ++ks) ldsm_x4(aq[ks], addrA<KD>(qb, 0, ks, lane));
         float o[2 * KD][4];
 #pragma unroll
         for (int n = 0; n < 2 * KD; ++n) { o[n][0] = 0.f; o[n][1] = 0.f; o[n][2] = 0.f; o[n][3] = 0.f; }
         float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;
         for (int k0 = 0; k0 < last_k0; k0 += NBC)
-          ap::fwd_chunk<KD, NBC, false>(kb, vb, k0, NBC, T, aq, o, m0, m1, l0, l1, gm.sl2, lane);
-        ap::fwd_chunk<KD, NBC, true>(kb, vb, last_k0, NQ - last_k0, T, aq, o, m0, m1, l0, l1, gm.sl2, lane);
+          fwd_chunk<KD, NBC, false>(kb, vb, k0, NBC, T, aq, o, m0, m1, l0, l1, gm.sl2, lane);
+        fwd_chunk<KD, NBC, true>(kb, vb, last_k0, NQ - last_k0, T, aq, o, m0, m1, l0, l1, gm.sl2, lane);
         __syncwarp();
         if (lane == 0) mbar_arrive(bars->empty + s);       // this warp is done with the stage's tiles
         if (lane == 0) tr(trace, 3, it, 1);
@@ -325,8 +242,8 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
         bf16* ob = out + ((size_t)b * T) * gm.d + hh * dh + cb;
 #pragma unroll
         for (int n = 0; n < 2 * KD; ++n) {
-          if (r0 < T) *reinterpret_cast<uint32_t*>(ob + (size_t)r0 * gm.d + n * 8) = ap::pack2(o[n][0] * i0, o[n][1] * i0);
-          if (r1 < T) *reinterpret_cast<uint32_t*>(ob + (size_t)r1 * gm.d + n * 8) = ap::pack2(o[n][2] * i1, o[n][3] * i1);
+          if (r0 < T) *reinterpret_cast<uint32_t*>(ob + (size_t)r0 * gm.d + n * 8) = pack2(o[n][0] * i0, o[n][1] * i0);
+          if (r1 < T) *reinterpret_cast<uint32_t*>(ob + (size_t)r1 * gm.d + n * 8) = pack2(o[n][2] * i1, o[n][3] * i1);
         }
         if (lse != nullptr && (lane & 3) == 0) {
           float* lp = lse + ((size_t)b * gm.h + hh) * T;
@@ -347,7 +264,7 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
     // swap a partial row statistic with the thread that holds the other half of the row
     auto swap_half = [&](int which, float mine) -> float {
       xch[(which * SP + hf) * 128 + row] = mine;
-      asm volatile("bar.sync %0, 64;" ::"r"(1 + q) : "memory");
+      bar_sync(1 + q, 64);
       return xch[(which * SP + (hf ^ 1)) * 128 + row];
     };
     int it = 0, s = 0;
@@ -379,11 +296,11 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
         auto col = [&](int k) { return (uint32_t)((hf + SP * k) * 32); };      // first S column of this thread's k-th chunk
         if (nmine > 0) tmem_ld32(trow + col(0), ra);
         for (int k = 0; k < nmine; k += 2) {
-          tmem_ld_wait32(ra);
+          tmem_ld_wait(ra);
           if (k + 1 < nmine) tmem_ld32(trow + col(k + 1), rb);
           max32(ra, hf + SP * k);
           if (k + 1 < nmine) {
-            tmem_ld_wait32(rb);
+            tmem_ld_wait(rb);
             if (k + 2 < nmine) tmem_ld32(trow + col(k + 2), ra);
             max32(rb, hf + SP * (k + 1));
           }
@@ -406,22 +323,22 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
           }
 #pragma unroll
           for (int j = 0; j < 16; ++j) {
-            const float p0 = ap::ex2(fmaf(__uint_as_float(r[2 * j]), sl2, -ms));
-            const float p1 = ap::ex2(fmaf(__uint_as_float(r[2 * j + 1]), sl2, -ms));
+            const float p0 = ex2(fmaf(__uint_as_float(r[2 * j]), sl2, -ms));
+            const float p1 = ex2(fmaf(__uint_as_float(r[2 * j + 1]), sl2, -ms));
             sum0 += p0; sum1 += p1;
-            pk[j] = ap::pack2(p0, p1);
+            pk[j] = pack2(p0, p1);
           }
         };
         if (SP == 1) {
           uint32_t pk[16];
           if (nmine > 0) tmem_ld32(trow, ra);
           for (int c = 0; c < nch; c += 2) {
-            tmem_ld_wait32(ra);
+            tmem_ld_wait(ra);
             if (c + 1 < nch) tmem_ld32(trow + (uint32_t)((c + 1) * 32), rb);
             exp32(ra, c, pk);
             tmem_st16(trow + (uint32_t)(c * 16), pk);
             if (c + 1 < nch) {
-              tmem_ld_wait32(rb);
+              tmem_ld_wait(rb);
               if (c + 2 < nch) tmem_ld32(trow + (uint32_t)((c + 2) * 32), ra);
               exp32(rb, c + 1, pk);
               tmem_st16(trow + (uint32_t)((c + 1) * 16), pk);
@@ -438,24 +355,24 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
           uint32_t pk[16];
           if (nmine > 0) tmem_ld32(trow + col(0), ra);
           for (int k = 0; k < nmine; k += 2) {
-            tmem_ld_wait32(ra);
+            tmem_ld_wait(ra);
             if (k + 1 < nmine) tmem_ld32(trow + col(k + 1), rb);
             // every chunk pair (2k, 2k + 1) is in registers on both sides before its P -- which overlaps S chunk k <= 2k --
             // is stored: one 64-thread barrier per pair (the partner may have one chunk less: it still takes the barrier)
-            asm volatile("bar.sync %0, 64;" ::"r"(1 + q) : "memory");
+            bar_sync(1 + q, 64);
             exp32(ra, hf + SP * k, pk);
             tmem_st16(trow + (uint32_t)((hf + SP * k) * 16), pk);
             if (k + 1 < nmine) {
-              tmem_ld_wait32(rb);
+              tmem_ld_wait(rb);
               if (k + 2 < nmine) tmem_ld32(trow + col(k + 2), ra);
-              asm volatile("bar.sync %0, 64;" ::"r"(1 + q) : "memory");
+              bar_sync(1 + q, 64);
               exp32(rb, hf + SP * (k + 1), pk);
               tmem_st16(trow + (uint32_t)((hf + SP * (k + 1)) * 16), pk);
             }
           }
-          if (nmine < (nch + SP - 1) / SP) asm volatile("bar.sync %0, 64;" ::"r"(1 + q) : "memory");   // odd chunk count: keep the pair's barrier count equal
+          if (nmine < (nch + SP - 1) / SP) bar_sync(1 + q, 64);   // odd chunk count: keep the pair's barrier count equal
         }
-        tmem_st_wait5();
+        tmem_st_wait();
         tc_fence_before();
         mbar_arrive(&bars->p_full);
         if (tid == 0 && t == 0) tr(trace, 2, it, 2);
@@ -476,20 +393,20 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
         if (CW == 8) {
           uint32_t t8[8];
           tmem_ld8(trow + oc0, t8);
-          tmem_ld_wait8(t8);
+          tmem_ld_wait(t8);
 #pragma unroll
           for (int j = 0; j < CW; ++j) o[j] = t8[j % 8];
         } else if (CW == 16) {
           uint32_t t16[16];
           tmem_ld16(trow + oc0, t16);
-          tmem_ld_wait16(t16);
+          tmem_ld_wait(t16);
 #pragma unroll
           for (int j = 0; j < CW; ++j) o[j] = t16[j % 16];
         } else {
           tmem_ld32(trow + oc0, ra);
           if (CW == 64) tmem_ld32(trow + oc0 + 32u, rb);
-          tmem_ld_wait32(ra);
-          if (CW == 64) tmem_ld_wait32(rb);
+          tmem_ld_wait(ra);
+          if (CW == 64) tmem_ld_wait(rb);
 #pragma unroll
           for (int j = 0; j < CW; ++j) o[j] = j < 32 ? ra[j % 32] : rb[j % 32];
         }
@@ -498,11 +415,11 @@ attn_tc5_fwd_kernel(const __grid_constant__ CUtensorMap mQ, const __grid_constan
         if (lane == 0) mbar_arrive(&bars->t_empty);
 #pragma unroll
         for (int ch = 0; ch < NCH; ++ch)
-          sts128(ap::chunk_addr<KD>(ot, row, hf * NCH + ch),
-                 ap::pack2(__uint_as_float(o[8 * ch]) * inv, __uint_as_float(o[8 * ch + 1]) * inv),
-                 ap::pack2(__uint_as_float(o[8 * ch + 2]) * inv, __uint_as_float(o[8 * ch + 3]) * inv),
-                 ap::pack2(__uint_as_float(o[8 * ch + 4]) * inv, __uint_as_float(o[8 * ch + 5]) * inv),
-                 ap::pack2(__uint_as_float(o[8 * ch + 6]) * inv, __uint_as_float(o[8 * ch + 7]) * inv));
+          sts128(chunk_addr<KD>(ot, row, hf * NCH + ch),
+                 pack2(__uint_as_float(o[8 * ch]) * inv, __uint_as_float(o[8 * ch + 1]) * inv),
+                 pack2(__uint_as_float(o[8 * ch + 2]) * inv, __uint_as_float(o[8 * ch + 3]) * inv),
+                 pack2(__uint_as_float(o[8 * ch + 4]) * inv, __uint_as_float(o[8 * ch + 5]) * inv),
+                 pack2(__uint_as_float(o[8 * ch + 6]) * inv, __uint_as_float(o[8 * ch + 7]) * inv));
         fence_proxy_async();
         __syncwarp();
         if (lane == 0) mbar_arrive(bars->o_staged + s);
@@ -614,20 +531,20 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
   if (warp == NRW) {
     // ============================ MMA issuer warp (all lanes run the loop, one elected lane issues) ============================
     {
-      const uint64_t hiK = make_desc_sw(0, 16, SBO, LAY);          // K-major view of an input tile (rows of RB bytes)
-      const uint64_t hiM = make_desc_sw(0, SBO, SBO, LAY);         // MN-major view of an input tile
+      const uint64_t hiK = make_smem_desc(0, 16, SBO, LAY);          // K-major view of an input tile (rows of RB bytes)
+      const uint64_t hiM = make_smem_desc(0, SBO, SBO, LAY);         // MN-major view of an input tile
       // [Q | dO] as one MN-major B operand: two dh-wide atoms 3 tiles apart (stage order Q, K, V, dO)
-      const uint64_t hiM2 = make_desc_sw(0, 3u * (uint32_t)gm.tile_bytes, SBO, LAY);
-      const uint64_t hiPK = make_desc_sw(0, 16, 1024, 2u);         // dS tile (128-byte rows), K-major
+      const uint64_t hiM2 = make_smem_desc(0, 3u * (uint32_t)gm.tile_bytes, SBO, LAY);
+      const uint64_t hiPK = make_smem_desc(0, 16, 1024, 2u);         // dS tile (128-byte rows), K-major
       // [P ; dS] as one MN-major A operand: two 64-key atoms ps_bytes apart
-      const uint64_t hiPM2 = make_desc_sw(0, (uint32_t)gm.ps_bytes, 1024, 2u);
-      constexpr uint32_t idG = make_idesc2(128, 2 * dh, 1, 1);     // [dK_c | . ; . | dV_c] : both operands MN-major
-      constexpr uint32_t idQ = make_idesc2(128, dh, 0, 1);         // dQ : A = dS K-major, B = K MN-major
+      const uint64_t hiPM2 = make_smem_desc(0, (uint32_t)gm.ps_bytes, 1024, 2u);
+      constexpr uint32_t idG = make_idesc(128, 2 * dh, 1, 1);     // [dK_c | . ; . | dV_c] : both operands MN-major
+      constexpr uint32_t idQ = make_idesc(128, dh, 0, 1);         // dQ : A = dS K-major, B = K MN-major
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
       // S and dP of item (c, t) of the unit staged in s -> TMEM buffer gi & 1
       auto issue_sdp = [&](int s, int c, int t, int gi) {
         const int k0 = c * CK, wc = min(CK, Tk - k0);
-        const uint32_t idS = make_idesc2(128, wc, 0, 0);
+        const uint32_t idS = make_idesc(128, wc, 0, 0);
         const uint32_t qa = (q_tile(s) + (uint32_t)(t * 128 * RB)) >> 4, da = (do_tile(s) + (uint32_t)(t * 128 * RB)) >> 4;
         const uint32_t kb = (k_tile(s) + (uint32_t)(k0 * RB)) >> 4, vb = (v_tile(s) + (uint32_t)(k0 * RB)) >> 4;
         const uint32_t td = tmem_u + (uint32_t)((gi & 1) * 128);
@@ -653,10 +570,10 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
           for (int bx = 0; bx < gm.kbox_n; ++bx) {
             const uint32_t off = (uint32_t)(bx * gm.kbox_rows * RB);
             const int r0 = bx * gm.kbox_rows;
-            ap::tma_load_3d(&mQKV, bars->full + s, q_tile(s) + off, col, r0, b);
-            ap::tma_load_3d(&mQKV, bars->full + s, k_tile(s) + off, gm.d + col, r0, b);
-            ap::tma_load_3d(&mQKV, bars->full + s, v_tile(s) + off, 2 * gm.d + col, r0, b);
-            ap::tma_load_3d(&mDO, bars->full + s, do_tile(s) + off, col, r0, b);
+            tma_load_3d(&mQKV, bars->full + s, q_tile(s) + off, col, r0, b);
+            tma_load_3d(&mQKV, bars->full + s, k_tile(s) + off, gm.d + col, r0, b);
+            tma_load_3d(&mQKV, bars->full + s, v_tile(s) + off, 2 * gm.d + col, r0, b);
+            tma_load_3d(&mDO, bars->full + s, do_tile(s) + off, col, r0, b);
           }
         }
         __syncwarp();
@@ -667,7 +584,7 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
         if (elect_one()) {
           mbar_expect_tx(&bars->o_full, (uint32_t)(Tk * RB));
           for (int bx = 0; bx < gm.kbox_n; ++bx)
-            ap::tma_load_3d(&mOut, &bars->o_full, o_ring + (uint32_t)(bx * gm.kbox_rows * RB), hh * dh, bx * gm.kbox_rows, b);
+            tma_load_3d(&mOut, &bars->o_full, o_ring + (uint32_t)(bx * gm.kbox_rows * RB), hh * dh, bx * gm.kbox_rows, b);
         }
         __syncwarp();
       };
@@ -772,13 +689,13 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
 #pragma unroll
         for (int ks = 0; ks < KD; ++ks) {
           uint32_t ofr[4];
-          ap::ldsm_x4(aq[ks], ap::addrA<KD>(qb, rbase, ks, lane));
-          ap::ldsm_x4(ad[ks], ap::addrA<KD>(db, rbase, ks, lane));
-          ap::ldsm_x4(ofr, ap::addrA<KD>(o_ring, rbase, ks, lane));
-          d0 += ap::bf_lo(ad[ks][0]) * ap::bf_lo(ofr[0]) + ap::bf_hi(ad[ks][0]) * ap::bf_hi(ofr[0]) +
-                ap::bf_lo(ad[ks][2]) * ap::bf_lo(ofr[2]) + ap::bf_hi(ad[ks][2]) * ap::bf_hi(ofr[2]);
-          d1 += ap::bf_lo(ad[ks][1]) * ap::bf_lo(ofr[1]) + ap::bf_hi(ad[ks][1]) * ap::bf_hi(ofr[1]) +
-                ap::bf_lo(ad[ks][3]) * ap::bf_lo(ofr[3]) + ap::bf_hi(ad[ks][3]) * ap::bf_hi(ofr[3]);
+          ldsm_x4(aq[ks], addrA<KD>(qb, rbase, ks, lane));
+          ldsm_x4(ad[ks], addrA<KD>(db, rbase, ks, lane));
+          ldsm_x4(ofr, addrA<KD>(o_ring, rbase, ks, lane));
+          d0 += bf_lo(ad[ks][0]) * bf_lo(ofr[0]) + bf_hi(ad[ks][0]) * bf_hi(ofr[0]) +
+                bf_lo(ad[ks][2]) * bf_lo(ofr[2]) + bf_hi(ad[ks][2]) * bf_hi(ofr[2]);
+          d1 += bf_lo(ad[ks][1]) * bf_lo(ofr[1]) + bf_hi(ad[ks][1]) * bf_hi(ofr[1]) +
+                bf_lo(ad[ks][3]) * bf_lo(ofr[3]) + bf_hi(ad[ks][3]) * bf_hi(ofr[3]);
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(&bars->o_empty);
@@ -804,12 +721,12 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
 #pragma unroll
               for (int ks = 0; ks < KD; ++ks) {
                 uint32_t bfr[4];
-                ap::ldsm_x4(bfr, ap::addrB<KD>(kb, k0 + 16 * j, ks, lane));
-                ap::mma_bf16(st[2 * j], aq[ks], bfr[0], bfr[1]);
-                ap::mma_bf16(st[2 * j + 1], aq[ks], bfr[2], bfr[3]);
-                ap::ldsm_x4(bfr, ap::addrB<KD>(vb, k0 + 16 * j, ks, lane));
-                ap::mma_bf16(dp[2 * j], ad[ks], bfr[0], bfr[1]);
-                ap::mma_bf16(dp[2 * j + 1], ad[ks], bfr[2], bfr[3]);
+                ldsm_x4(bfr, addrB<KD>(kb, k0 + 16 * j, ks, lane));
+                mma_bf16(st[2 * j], aq[ks], bfr[0], bfr[1]);
+                mma_bf16(st[2 * j + 1], aq[ks], bfr[2], bfr[3]);
+                ldsm_x4(bfr, addrB<KD>(vb, k0 + 16 * j, ks, lane));
+                mma_bf16(dp[2 * j], ad[ks], bfr[0], bfr[1]);
+                mma_bf16(dp[2 * j + 1], ad[ks], bfr[2], bfr[3]);
               }
             }
           }
@@ -820,16 +737,16 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
           uint32_t sa[8][2];
 #pragma unroll
           for (int n = 0; n < 8; ++n) {
-            const float p0 = ap::ex2(fmaf(st[n][0], gm.sl2, -l0)), p1 = ap::ex2(fmaf(st[n][1], gm.sl2, -l0));
-            sa[n][0] = ap::pack2(p0 * fmaf(dp[n][0], gm.scale, -d0), p1 * fmaf(dp[n][1], gm.scale, -d0));
-            ap::sts32(ap::chunk_addr<4>(pt, pr0, n) + cb * 2, ap::pack2(p0, p1));
-            ap::sts32(ap::chunk_addr<4>(dt, pr0, n) + cb * 2, sa[n][0]);
+            const float p0 = ex2(fmaf(st[n][0], gm.sl2, -l0)), p1 = ex2(fmaf(st[n][1], gm.sl2, -l0));
+            sa[n][0] = pack2(p0 * fmaf(dp[n][0], gm.scale, -d0), p1 * fmaf(dp[n][1], gm.scale, -d0));
+            sts32(chunk_addr<4>(pt, pr0, n) + cb * 2, pack2(p0, p1));
+            sts32(chunk_addr<4>(dt, pr0, n) + cb * 2, sa[n][0]);
             sa[n][1] = 0u;
             if (two) {
-              const float p2 = ap::ex2(fmaf(st[n][2], gm.sl2, -l1)), p3 = ap::ex2(fmaf(st[n][3], gm.sl2, -l1));
-              sa[n][1] = ap::pack2(p2 * fmaf(dp[n][2], gm.scale, -d1), p3 * fmaf(dp[n][3], gm.scale, -d1));
-              ap::sts32(ap::chunk_addr<4>(pt, pr1, n) + cb * 2, ap::pack2(p2, p3));
-              ap::sts32(ap::chunk_addr<4>(dt, pr1, n) + cb * 2, sa[n][1]);
+              const float p2 = ex2(fmaf(st[n][2], gm.sl2, -l1)), p3 = ex2(fmaf(st[n][3], gm.sl2, -l1));
+              sa[n][1] = pack2(p2 * fmaf(dp[n][2], gm.scale, -d1), p3 * fmaf(dp[n][3], gm.scale, -d1));
+              sts32(chunk_addr<4>(pt, pr1, n) + cb * 2, pack2(p2, p3));
+              sts32(chunk_addr<4>(dt, pr1, n) + cb * 2, sa[n][1]);
             }
           }
           fence_proxy_async();
@@ -845,9 +762,9 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
 #pragma unroll
               for (int np = 0; np < KD; ++np) {
                 uint32_t bfr[4];
-                ap::ldsm_x4_t(bfr, ap::addrA<KD>(kb, k0 + 16 * j, np, lane));
-                ap::mma_bf16(dq[2 * np], a4, bfr[0], bfr[1]);
-                ap::mma_bf16(dq[2 * np + 1], a4, bfr[2], bfr[3]);
+                ldsm_x4_t(bfr, addrA<KD>(kb, k0 + 16 * j, np, lane));
+                mma_bf16(dq[2 * np], a4, bfr[0], bfr[1]);
+                mma_bf16(dq[2 * np + 1], a4, bfr[2], bfr[3]);
               }
             }
           }
@@ -861,7 +778,7 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
               *reinterpret_cast<float2*>(s_dqlo + (g + 8) * dh + n * 8 + cb) = make_float2(dq[n][2], dq[n][3]);
             }
           }
-          asm volatile("bar.sync 1, 64;" ::: "memory");
+          bar_sync(1, 64);
         }
         if (lw == 0) {
           __syncwarp();
@@ -874,8 +791,8 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
               a0 = *reinterpret_cast<const float2*>(s_dqlo + g * dh + n * 8 + cb);
               a1 = *reinterpret_cast<const float2*>(s_dqlo + (g + 8) * dh + n * 8 + cb);
             }
-            if (r0 < T) *reinterpret_cast<uint32_t*>(gp + (size_t)r0 * (3 * gm.d) + n * 8) = ap::pack2(dq[n][0] + a0.x, dq[n][1] + a0.y);
-            if (r1 < T) *reinterpret_cast<uint32_t*>(gp + (size_t)r1 * (3 * gm.d) + n * 8) = ap::pack2(dq[n][2] + a1.x, dq[n][3] + a1.y);
+            if (r0 < T) *reinterpret_cast<uint32_t*>(gp + (size_t)r0 * (3 * gm.d) + n * 8) = pack2(dq[n][0] + a0.x, dq[n][1] + a0.y);
+            if (r1 < T) *reinterpret_cast<uint32_t*>(gp + (size_t)r1 * (3 * gm.d) + n * 8) = pack2(dq[n][2] + a1.x, dq[n][3] + a1.y);
             if (dbias != nullptr) {        // q-bias gradient: column sums over the block's real rows
               float c0 = (r0 < T ? dq[n][0] + a0.x : 0.f) + (r1 < T ? dq[n][2] + a1.x : 0.f);
               float c1 = (r0 < T ? dq[n][1] + a0.y : 0.f) + (r1 < T ? dq[n][3] + a1.y : 0.f);
@@ -891,7 +808,7 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
             }
           }
         }
-        if (NLW == 2) asm volatile("bar.sync 2, 64;" ::: "memory");   // warp 0 has read the partial sums
+        if (NLW == 2) bar_sync(2, 64);   // warp 0 has read the partial sums
         if (++s == NST) { s = 0; ph ^= 1; }
       }
     }
@@ -913,19 +830,19 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
       if (KD == 4) {
         uint32_t a[32];
         tmem_ld32(ta, a);
-        tmem_ld_wait32(a);
+        tmem_ld_wait(a);
 #pragma unroll
         for (int j = 0; j < HC; ++j) v[j] = a[j % 32];
       } else if (KD == 2) {
         uint32_t a[16];
         tmem_ld16(ta, a);
-        tmem_ld_wait16(a);
+        tmem_ld_wait(a);
 #pragma unroll
         for (int j = 0; j < HC; ++j) v[j] = a[j % 16];
       } else {
         uint32_t a[8];
         tmem_ld8(ta, a);
-        tmem_ld_wait8(a);
+        tmem_ld_wait(a);
 #pragma unroll
         for (int j = 0; j < HC; ++j) v[j] = a[j % 8];
       }
@@ -934,10 +851,10 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
 #pragma unroll
       for (int ch = 0; ch < KD; ++ch)
         *reinterpret_cast<uint4*>(g + ch * 8) =
-            make_uint4(ap::pack2(__uint_as_float(v[8 * ch]), __uint_as_float(v[8 * ch + 1])),
-                       ap::pack2(__uint_as_float(v[8 * ch + 2]), __uint_as_float(v[8 * ch + 3])),
-                       ap::pack2(__uint_as_float(v[8 * ch + 4]), __uint_as_float(v[8 * ch + 5])),
-                       ap::pack2(__uint_as_float(v[8 * ch + 6]), __uint_as_float(v[8 * ch + 7])));
+            make_uint4(pack2(__uint_as_float(v[8 * ch]), __uint_as_float(v[8 * ch + 1])),
+                       pack2(__uint_as_float(v[8 * ch + 2]), __uint_as_float(v[8 * ch + 3])),
+                       pack2(__uint_as_float(v[8 * ch + 4]), __uint_as_float(v[8 * ch + 5])),
+                       pack2(__uint_as_float(v[8 * ch + 6]), __uint_as_float(v[8 * ch + 7])));
     };
     // column sums over the warp's 32 rows (rows that do not exist contribute 0): halving exchange, lane l ends with the
     // sum of column (l mod HC) over half (HC = 16) or a quarter (HC = 8) of the rows ... one global reduction per column
@@ -1017,11 +934,11 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
           float dl = 0.f;
 #pragma unroll
           for (int ch = 0; ch < 2 * KD; ++ch) {
-            const uint4 a = ap::lds128(ap::chunk_addr<KD>(do_tile(s), t * 128 + row, ch));
-            const uint4 o4 = ap::lds128(ap::chunk_addr<KD>(o_ring, t * 128 + row, ch));
-            dl += ap::bf_lo(a.x) * ap::bf_lo(o4.x) + ap::bf_hi(a.x) * ap::bf_hi(o4.x) + ap::bf_lo(a.y) * ap::bf_lo(o4.y) +
-                  ap::bf_hi(a.y) * ap::bf_hi(o4.y) + ap::bf_lo(a.z) * ap::bf_lo(o4.z) + ap::bf_hi(a.z) * ap::bf_hi(o4.z) +
-                  ap::bf_lo(a.w) * ap::bf_lo(o4.w) + ap::bf_hi(a.w) * ap::bf_hi(o4.w);
+            const uint4 a = lds128(chunk_addr<KD>(do_tile(s), t * 128 + row, ch));
+            const uint4 o4 = lds128(chunk_addr<KD>(o_ring, t * 128 + row, ch));
+            dl += bf_lo(a.x) * bf_lo(o4.x) + bf_hi(a.x) * bf_hi(o4.x) + bf_lo(a.y) * bf_lo(o4.y) +
+                  bf_hi(a.y) * bf_hi(o4.y) + bf_lo(a.z) * bf_lo(o4.z) + bf_hi(a.z) * bf_hi(o4.z) +
+                  bf_lo(a.w) * bf_lo(o4.w) + bf_hi(a.w) * bf_hi(o4.w);
           }
           dls[t] = dl * scale;
         }
@@ -1045,10 +962,10 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
           uint32_t pw[4], dw[4];
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
-            const float p0 = ap::ex2(fmaf(__uint_as_float(rs[2 * e]), sl2, -l2t));
-            const float p1 = ap::ex2(fmaf(__uint_as_float(rs[2 * e + 1]), sl2, -l2t));
-            pw[e] = ap::pack2(p0, p1);
-            dw[e] = ap::pack2(p0 * fmaf(__uint_as_float(rd[2 * e]), scale, -dlt), p1 * fmaf(__uint_as_float(rd[2 * e + 1]), scale, -dlt));
+            const float p0 = ex2(fmaf(__uint_as_float(rs[2 * e]), sl2, -l2t));
+            const float p1 = ex2(fmaf(__uint_as_float(rs[2 * e + 1]), sl2, -l2t));
+            pw[e] = pack2(p0, p1);
+            dw[e] = pack2(p0 * fmaf(__uint_as_float(rd[2 * e]), scale, -dlt), p1 * fmaf(__uint_as_float(rd[2 * e + 1]), scale, -dlt));
           }
           const uint32_t off = (uint32_t)(((hf * 4 + q4) ^ sw) << 4);
           if (!(gm.ablate & 8)) {
@@ -1061,16 +978,16 @@ attn_tc5_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_const
           uint32_t rs[32], rd[32];
           tmem_ld32(tb, rs);
           tmem_ld32(tb + 64u, rd);
-          tmem_ld_wait32(rs);
-          tmem_ld_wait32(rd);
+          tmem_ld_wait(rs);
+          tmem_ld_wait(rd);
 #pragma unroll
           for (int q4 = 0; q4 < 4; ++q4) emit8(rs + 8 * q4, rd + 8 * q4, q4);
         } else if (ncol > 0) {
           uint32_t rs[16], rd[16];
           tmem_ld16(tb, rs);
           tmem_ld16(tb + 64u, rd);
-          tmem_ld_wait16(rs);
-          tmem_ld_wait16(rd);
+          tmem_ld_wait(rs);
+          tmem_ld_wait(rd);
 #pragma unroll
           for (int q4 = 0; q4 < 2; ++q4) emit8(rs + 8 * q4, rd + 8 * q4, q4);
         }
@@ -1275,7 +1192,7 @@ int attn_tc5_fwd(int B, int T, int h, int dh, const bf16* qkv, bf16* out, float*
        resources; the hardware does co-schedule such CTAs -- measured -- so the limits are applied here) */           \
     int occ = tc5_ctas_per_sm((const void*)kern, threads, sm, g.tmem_cols);                                           \
     if (getenv("AMC_TC5_OCC")) occ = atoi(getenv("AMC_TC5_OCC"));                                                     \
-    const int grid = std::min(g.units, attn_sm_count() * occ);                                                        \
+    const int grid = std::min(g.units, device_sm_count() * occ);                                                      \
     if (trace) {                                                                                                      \
       cudaFuncAttributes fa;                                                                                          \
       cudaFuncGetAttributes(&fa, kern);                                                                               \
@@ -1320,7 +1237,7 @@ int attn_tc5_bwd(int B, int T, int h, int dh, const bf16* qkv, const bf16* out, 
     auto kern = attn_tc5_bwd_kernel<KD>;                                                                               \
     AMC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC5_SMEM_MAX));             \
     const int occ = 1;                                                                                                \
-    const int grid = std::min(g.units, attn_sm_count() * occ);                                                        \
+    const int grid = std::min(g.units, device_sm_count() * occ);                                                      \
     if (trace) fprintf(stderr, "[tc5 bwd] grid %d occ %d smem %zu nst %d units %d\n", grid, occ, sm, g.nst, g.units); \
     kern<<<grid, BWD_THREADS, sm, st>>>(mQKV, mDO, mOut, g, out, dout, lse, dqkv, dbias, trace);                                                 \
   } while (0)

@@ -30,8 +30,6 @@
 namespace amc {
 namespace {
 
-using namespace attn_ptx;
-
 struct TileGeom {
   int T, Tpad, NQ, h, d, G, ngrp, units;
   int BR, nbox;          // TMA box rows and boxes per tile (Tpad = BR * nbox)
@@ -53,7 +51,7 @@ attn_tile_fwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_cons
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~(uintptr_t)1023);
   uint64_t* full = reinterpret_cast<uint64_t*>(smem);
-  const uint32_t tiles = s_u32(smem + SMEM_HDR);
+  const uint32_t tiles = smem_u32(smem + SMEM_HDR);
   const uint32_t tb = (uint32_t)gm.tile_bytes, stage_bytes = 3u * gm.G * tb;
   const uint32_t so_base = tiles + gm.nst * stage_bytes;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nw = blockDim.x >> 5;
@@ -120,21 +118,21 @@ attn_tile_fwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_cons
         if (r1 < T) lp[r1] = fmaf(m1, gm.sl2, __log2f(l1));
       }
     }
-    fence_async_smem();
-    if (tid == 0) bulk_wait_read0();      // the previous unit's output tiles have left shared memory
+    fence_proxy_async();
+    if (tid == 0) bulk_wait_read<0>();      // the previous unit's output tiles have left shared memory
     __syncthreads();
     if (tid == 0) {
       for (int hh = 0; hh < gm.G; ++hh)
         for (int bx = 0; bx < gm.nbox; ++bx)
           tma_store_3d(&mO, so + hh * tb + bx * gm.BR * RB, (hg * gm.G + hh) * dh, bx * gm.BR, b);
       bulk_commit();
-      if (gm.nso == 1) bulk_wait_read0();
+      if (gm.nso == 1) bulk_wait_read<0>();
       if (gm.nst == 1 && u + (int)gridDim.x < gm.units) issue(u + gridDim.x, 0);
     }
     if (gm.nso == 1) __syncthreads();
     if (++s == gm.nst) { s = 0; ph ^= 1; }
   }
-  if (tid == 0) bulk_wait_all0();
+  if (tid == 0) bulk_wait_all();
 }
 
 // ===============================================================================================================
@@ -153,7 +151,7 @@ attn_tile_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_cons
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~(uintptr_t)1023);
   uint64_t* full = reinterpret_cast<uint64_t*>(smem);
-  const uint32_t tiles = s_u32(smem + SMEM_HDR);
+  const uint32_t tiles = smem_u32(smem + SMEM_HDR);
   const uint32_t tb = (uint32_t)gm.tile_bytes;
   const int T = gm.T, Tpad = gm.Tpad, NQ = gm.NQ, G = gm.G, items = G * NQ;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nt = blockDim.x, nw = nt >> 5;
@@ -163,7 +161,7 @@ attn_tile_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_cons
   float* s_colkv = reinterpret_cast<float*>(s_stat + G * Tpad);                     // [items][2][dh]
   float* s_colq = s_colkv + (size_t)items * 2 * dh;                                 // [nw][G][dh]
   float* s_bias = s_colq + (size_t)nw * G * dh;                                     // [3d]
-  const uint32_t sdq_u = s_u32(sdq), stat_u = s_u32(s_stat);
+  const uint32_t sdq_u = smem_u32(sdq), stat_u = smem_u32(s_stat);
   auto tile = [&](int hh, int which) { return tiles + (uint32_t)(hh * 7 + which) * tb; };
   // lane-constant ldmatrix offsets inside a 16-row block (block bases are multiples of 16 rows, the swizzle term
   // depends on the row modulo 8 only)
@@ -362,7 +360,7 @@ attn_tile_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_cons
         }
       }
     }
-    fence_async_smem();
+    fence_proxy_async();
     __syncthreads();
     if (tid == 0) {
       for (int hh = 0; hh < G; ++hh) {
@@ -375,7 +373,7 @@ attn_tile_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_cons
         }
       }
       bulk_commit();
-      bulk_wait_read0();
+      bulk_wait_read<0>();
       if (has_next) issue_o(u + gridDim.x);
     }
     if (dbias != nullptr) {                 // fold the slots into the CTA's running bias-gradient sums
@@ -391,7 +389,7 @@ attn_tile_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_cons
       }
     }
   }
-  if (tid == 0) bulk_wait_all0();
+  if (tid == 0) bulk_wait_all();
   if (dbias != nullptr) {
     __syncthreads();
     for (int c = tid; c < 3 * gm.d; c += nt) {
@@ -402,41 +400,6 @@ attn_tile_bwd_kernel(const __grid_constant__ CUtensorMap mQKV, const __grid_cons
 }
 
 // ---- host side -------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-int encode_fn(EncodeTiledFn* out) {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    AMC_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q));
-    AMC_CHECK_ARG(p != nullptr && q == cudaDriverEntryPointSuccess, "cuTensorMapEncodeTiled not available");
-    fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  *out = fn;
-  return 0;
-}
-// bf16 tensor [B][T][cols] (row pitch = cols), box = {dh, box_rows, 1}, swizzle span = dh * 2 bytes
-int make_map3(CUtensorMap* map, const void* base, int B, int T, int cols, int dh, int box_rows) {
-  EncodeTiledFn enc;
-  AMC_TRY(encode_fn(&enc));
-  AMC_CHECK_ARG((reinterpret_cast<uintptr_t>(base) & 15) == 0 && (cols * 2) % 16 == 0,
-                "attention tensors must be 16-byte aligned with a 16-byte row pitch");
-  cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)T, (cuuint64_t)B};
-  cuuint64_t strides[2] = {(cuuint64_t)cols * 2, (cuuint64_t)T * cols * 2};
-  cuuint32_t box[3] = {(cuuint32_t)dh, (cuuint32_t)box_rows, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  const CUtensorMapSwizzle sw = dh == 16 ? CU_TENSOR_MAP_SWIZZLE_32B : (dh == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B);
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  AMC_CHECK_ARG(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled (attention) failed (%d) B=%d T=%d cols=%d dh=%d box=%d", (int)r, B,
-                T, cols, dh, box_rows);
-  return 0;
-}
-
-int sm_count() { return device_sm_count(); }
-
 constexpr size_t SMEM_MAX = 227 * 1024;
 
 size_t fwd_bytes(const TileGeom& g) { return 1024 + SMEM_HDR + (size_t)(3 * g.nst + g.nso) * g.G * g.tile_bytes; }
@@ -465,9 +428,15 @@ int pick_warps(int items) {
 }  // namespace
 
 int attn_make_map3(CUtensorMap* map, const void* base, int B, int T, int cols, int dh, int box_rows) {
-  return make_map3(map, base, B, T, cols, dh, box_rows);
+  AMC_CHECK_ARG((reinterpret_cast<uintptr_t>(base) & 15) == 0 && (cols * 2) % 16 == 0,
+                "attention tensors must be 16-byte aligned with a 16-byte row pitch");
+  const cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)T, (cuuint64_t)B};
+  const cuuint64_t strides[2] = {(cuuint64_t)cols * 2, (cuuint64_t)T * cols * 2};
+  const cuuint32_t box[3] = {(cuuint32_t)dh, (cuuint32_t)box_rows, 1};
+  const CUtensorMapSwizzle sw = dh == 16 ? CU_TENSOR_MAP_SWIZZLE_32B : (dh == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B);
+  return encode_tiled_map(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base, dims, strides, box, sw,
+                          CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
 }
-int attn_sm_count() { return sm_count(); }
 
 bool attn_tiles_supported(int T, int h, int dh) {
   return T > 16 && T <= 288 && (dh == 16 || dh == 32 || dh == 64) && h >= 1;
@@ -501,15 +470,15 @@ int attn_tiles_fwd(int B, int T, int h, int dh, const bf16* qkv, bf16* out, floa
   const size_t sm = fwd_bytes(g);
   const int threads = 32 * pick_warps(G * g.NQ);
   CUtensorMap mQKV, mO;
-  AMC_TRY(make_map3(&mQKV, qkv, B, T, 3 * g.d, dh, g.BR));
-  AMC_TRY(make_map3(&mO, out, B, T, g.d, dh, g.BR));
+  AMC_TRY(attn_make_map3(&mQKV, qkv, B, T, 3 * g.d, dh, g.BR));
+  AMC_TRY(attn_make_map3(&mO, out, B, T, g.d, dh, g.BR));
 #define AMC_TILE_FWD(KD, NBC)                                                                                         \
   do {                                                                                                                \
     auto kern = attn_tile_fwd_kernel<KD, NBC, 2>;                                                                      \
     AMC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_MAX));                 \
     int occ = 1;                                                                                                      \
     AMC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, sm));                                 \
-    const int grid = std::min(g.units, sm_count() * std::max(occ, 1));                                                \
+    const int grid = std::min(g.units, device_sm_count() * std::max(occ, 1));                                         \
     kern<<<grid, threads, sm, st>>>(mQKV, mO, g, lse);                                                                \
   } while (0)
 #define AMC_TILE_FWD_KD(KD)                            \
@@ -547,17 +516,17 @@ int attn_tiles_bwd(int B, int T, int h, int dh, const bf16* qkv, const bf16* out
   const size_t sm = bwd_bytes(g, dh);
   const int threads = 32 * pick_warps(G * g.NQ);
   CUtensorMap mQKV, mOut, mDO, mDQKV;
-  AMC_TRY(make_map3(&mQKV, qkv, B, T, 3 * g.d, dh, g.BR));
-  AMC_TRY(make_map3(&mOut, out, B, T, g.d, dh, g.BR));
-  AMC_TRY(make_map3(&mDO, dout, B, T, g.d, dh, g.BR));
-  AMC_TRY(make_map3(&mDQKV, dqkv, B, T, 3 * g.d, dh, g.BR));
+  AMC_TRY(attn_make_map3(&mQKV, qkv, B, T, 3 * g.d, dh, g.BR));
+  AMC_TRY(attn_make_map3(&mOut, out, B, T, g.d, dh, g.BR));
+  AMC_TRY(attn_make_map3(&mDO, dout, B, T, g.d, dh, g.BR));
+  AMC_TRY(attn_make_map3(&mDQKV, dqkv, B, T, 3 * g.d, dh, g.BR));
 #define AMC_TILE_BWD(KD, MINB)                                                                                        \
   do {                                                                                                                \
     auto kern = attn_tile_bwd_kernel<KD, MINB>;                                                                        \
     AMC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_MAX));                 \
     int occ = 1;                                                                                                      \
     AMC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, sm));                                 \
-    const int grid = std::min(g.units, sm_count() * std::max(occ, 1));                                                \
+    const int grid = std::min(g.units, device_sm_count() * std::max(occ, 1));                                         \
     kern<<<grid, threads, sm, st>>>(mQKV, mOut, mDO, mDQKV, g, lse, dbias);                                           \
   } while (0)
   const bool two = 2 * (sm + 1024) <= SMEM_MAX + 1024;      // two CTAs per SM fit: cap registers for it

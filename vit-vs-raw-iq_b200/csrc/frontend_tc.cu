@@ -18,7 +18,7 @@
 
 #include "gemm_common.cuh"
 #include "rowops.cuh"
-#include "tc_ptx.cuh"
+#include "ptx.cuh"
 
 namespace amc {
 namespace {
@@ -52,16 +52,6 @@ template <int BN> struct FrontCfg {
   }
 };
 
-__device__ __forceinline__ void sts32(uint32_t addr, uint32_t v) {
-  asm volatile("st.shared.b32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
-}
-__device__ __forceinline__ void sts64(uint32_t addr, uint32_t a, uint32_t b) {
-  asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(addr), "r"(a), "r"(b) : "memory");
-}
-__device__ __forceinline__ uint32_t pk(float a, float b) {
-  __nv_bfloat162 t = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&t);
-}
 // byte offset of element (row, kcol) inside a 128-row x 64-column K-major SWIZZLE_128B tile
 __device__ __forceinline__ uint32_t a_off(int row, int kcol) {
   return (uint32_t)(row * 128 + ((((kcol >> 3) ^ (row & 7)) << 4) | ((kcol & 7) << 1)));
@@ -208,8 +198,8 @@ __device__ __forceinline__ void store_block(const FrontParams& p, const LaneSlot
     if (p.raw) {
       uint32_t wi = 0u, wq = 0u;
       if (ok) {
-        wi = pk((v[j].x - p.mean[0]) * p.inv_std[0], (v[j].z - p.mean[0]) * p.inv_std[0]);
-        wq = pk((v[j].y - p.mean[1]) * p.inv_std[1], (v[j].w - p.mean[1]) * p.inv_std[1]);
+        wi = pack2((v[j].x - p.mean[0]) * p.inv_std[0], (v[j].z - p.mean[0]) * p.inv_std[0]);
+        wq = pack2((v[j].y - p.mean[1]) * p.inv_std[1], (v[j].w - p.mean[1]) * p.inv_std[1]);
         if (p.Aout) {
           *reinterpret_cast<uint32_t*>(p.Aout + (size_t)(m0 + row0) * p.K + kbase + k0) = wi;
           *reinterpret_cast<uint32_t*>(p.Aout + (size_t)(m0 + row1) * p.K + kbase + k1) = wq;
@@ -218,7 +208,7 @@ __device__ __forceinline__ void store_block(const FrontParams& p, const LaneSlot
       sts32(sa + (ls.soff[j] & 0xFFFFu), wi);
       sts32(sa + (ls.soff[j] >> 16), wq);
     } else {
-      const uint32_t w0_ = pk(v[j].x, v[j].y), w1_ = pk(v[j].z, v[j].w);
+      const uint32_t w0_ = pack2(v[j].x, v[j].y), w1_ = pack2(v[j].z, v[j].w);
       if (ok && p.Aout)
         *reinterpret_cast<uint2*>(p.Aout + (size_t)(m0 + row0) * p.K + kbase + k0) = make_uint2(w0_, w1_);
       sts64(sa + (ls.soff[j] & 0xFFFFu), w0_, w1_);
@@ -274,11 +264,12 @@ frontend_tc_kernel(const __grid_constant__ CUtensorMap mapW, const FrontParams p
   if (warp == 0) {
     if (lane == 0) {
       mbar_expect_tx(wfull, (uint32_t)(p.kb_total * C::W_BLOCK));
-      for (int kb = 0; kb < p.kb_total; ++kb) tma_load_2d(&mapW, wfull, sW + (size_t)kb * C::W_BLOCK, kb * FBK, n0);
+      for (int kb = 0; kb < p.kb_total; ++kb)
+        tma_load_2d(&mapW, wfull, smem_u32(sW + (size_t)kb * C::W_BLOCK), kb * FBK, n0);
     }
   } else if (warp == 1) {
     if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc(FBM, BN, 0);
+      constexpr uint32_t idesc = make_idesc(FBM, BN, 0, 0);
       mbar_wait(wfull, 0);
       int stage = 0, as = 0;
       uint32_t phase = 0, aphase = 0;
@@ -293,7 +284,7 @@ frontend_tc_kernel(const __grid_constant__ CUtensorMap mapW, const FrontParams p
           const uint32_t sb = smem_u32(sW + (size_t)kb * C::W_BLOCK);
           const int ksteps = min(FBK, p.K - kb * FBK + 15) / 16;
           for (int k = 0; k < ksteps; ++k)
-            umma_bf16(tmem_d, make_smem_desc(sa + k * 32, 16, 1024), make_smem_desc(sb + k * 32, 16, 1024), idesc,
+            umma_bf16(tmem_d, make_smem_desc(sa + k * 32, 16, 1024, 2), make_smem_desc(sb + k * 32, 16, 1024, 2), idesc,
                       (kb > 0 || k > 0) ? 1u : 0u);
           umma_commit(empty_bar + stage);
           if (++stage == nstage) { stage = 0; phase ^= 1; }
@@ -354,7 +345,7 @@ frontend_tc_kernel(const __grid_constant__ CUtensorMap mapW, const FrontParams p
       if (c_begin < c_end) tmem_ld32(taddr + c_begin, r);
 #pragma unroll 1
       for (int c = c_begin; c < c_end; c += 32) {
-        tmem_ld_wait();
+        tmem_ld_wait(r);
 #pragma unroll
         for (int j = 0; j < 32; j += 4)
           sts128(stg + (uint32_t)(lane * F_STG_LD + (((j >> 2) ^ (lane & 7)) << 2)) * 4, r[j], r[j + 1], r[j + 2], r[j + 3]);
@@ -369,7 +360,7 @@ frontend_tc_kernel(const __grid_constant__ CUtensorMap mapW, const FrontParams p
 #pragma unroll
           for (int it = 0; it < 8; ++it) {
             const int rr = it * 4 + sub_r;
-            float4 v = lds128(stg + (uint32_t)(rr * F_STG_LD + ((((lane & 7)) ^ (rr & 7)) << 2)) * 4);
+            float4 v = lds128f(stg + (uint32_t)(rr * F_STG_LD + ((((lane & 7)) ^ (rr & 7)) << 2)) * 4);
             if (orow[it] < 0) continue;
             v.x += bias.x + pe[it].x; v.y += bias.y + pe[it].y; v.z += bias.z + pe[it].z; v.w += bias.w + pe[it].w;
             const size_t o = (size_t)orow[it] * p.d + n;
@@ -397,51 +388,26 @@ frontend_tc_kernel(const __grid_constant__ CUtensorMap mapW, const FrontParams p
   }
 }
 
-int encode_fn(EncodeTiledFn* out) {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    AMC_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q));
-    AMC_CHECK_ARG(p != nullptr && q == cudaDriverEntryPointSuccess, "cuTensorMapEncodeTiled not available");
-    fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  *out = fn;
-  return 0;
-}
-
 inline bool pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
 
 template <int BN>
 int launch_front(const AmcDesc& D, FrontParams p, const Epi& epi, const float* src, const bf16* W, cudaStream_t st) {
   using C = FrontCfg<BN>;
-  EncodeTiledFn enc;
-  AMC_TRY(encode_fn(&enc));
   CUtensorMap mapW;
-  cuuint64_t dims[2] = {(cuuint64_t)p.K, (cuuint64_t)p.d};
-  cuuint64_t strides[1] = {(cuuint64_t)p.K * 2};
-  cuuint32_t box[2] = {(cuuint32_t)FBK, (cuuint32_t)BN};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(&mapW, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<bf16*>(W), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  AMC_CHECK_ARG(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled (embedding weight) failed (%d)", (int)r);
+  const cuuint64_t dims[2] = {(cuuint64_t)p.K, (cuuint64_t)p.d};
+  const cuuint64_t strides[1] = {(cuuint64_t)p.K * 2};
+  const cuuint32_t box[2] = {(cuuint32_t)FBK, (cuuint32_t)BN};
+  AMC_TRY(encode_tiled_map(&mapW, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, W, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B));
   p.tiles_n = ceil_div(p.d, BN);
   p.tiles_m = ceil_div(p.M, FBM);
   int nstage = std::min(8, std::max(2, 2 * p.kb_total));
   while (nstage > 2 && C::smem(p.kb_total, nstage) > 227 * 1024) --nstage;
   const size_t smem = C::smem(p.kb_total, nstage);
   AMC_CHECK_ARG(smem <= 227 * 1024, "front end: K=%d d=%d needs %zu bytes of shared memory", p.K, p.d, smem);
-  int sms = 148, dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  const int per_n = std::max(1, std::min(p.tiles_m, sms / p.tiles_n));
+  const int per_n = std::max(1, std::min(p.tiles_m, device_sm_count() / p.tiles_n));
   auto kern = frontend_tc_kernel<BN>;
-  static bool attr_done = false;
-  if (!attr_done) {
-    AMC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    attr_done = true;
-  }
+  AMC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
   kern<<<per_n * p.tiles_n, F_THREADS, smem, st>>>(mapW, p, epi, src, nstage);
   AMC_LAUNCH_CHECK();
   (void)D;

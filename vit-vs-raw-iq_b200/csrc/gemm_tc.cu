@@ -23,7 +23,7 @@
 #include <initializer_list>
 
 #include "gemm_common.cuh"
-#include "tc_ptx.cuh"
+#include "ptx.cuh"
 
 namespace amc {
 namespace {
@@ -72,16 +72,16 @@ __device__ __forceinline__ void producer_loop(const CUtensorMap* mapA, const CUt
       unsigned char* sb = sa + A_BYTES;
       mbar_expect_tx(full_bar + stage, STAGE_BYTES);
       if (MODE_MN == 0) {
-        tma_load_2d(mapA, full_bar + stage, sa, kb * BK, m0);       // box {64 k, 128 rows}
-        tma_load_2d(mapB, full_bar + stage, sb, kb * BK, n0);       // box {64 k, min(BN, 256) rows}
-        if (BN > 256) tma_load_2d(mapB, full_bar + stage, sb + 256 * BK * 2, kb * BK, n0 + 256);
+        tma_load_2d(mapA, full_bar + stage, smem_u32(sa), kb * BK, m0);   // box {64 k, 128 rows}
+        tma_load_2d(mapB, full_bar + stage, smem_u32(sb), kb * BK, n0);   // box {64 k, min(BN, 256) rows}
+        if (BN > 256) tma_load_2d(mapB, full_bar + stage, smem_u32(sb + 256 * BK * 2), kb * BK, n0 + 256);
       } else {
 #pragma unroll
         for (int j = 0; j < BM / 64; ++j)                            // boxes {64 m, 64 tokens}
-          tma_load_2d(mapA, full_bar + stage, sa + j * 8192, m0 + 64 * j, kb * BK);
+          tma_load_2d(mapA, full_bar + stage, smem_u32(sa + j * 8192), m0 + 64 * j, kb * BK);
 #pragma unroll
         for (int j = 0; j < BN / 64; ++j)
-          tma_load_2d(mapB, full_bar + stage, sb + j * 8192, n0 + 64 * j, kb * BK);
+          tma_load_2d(mapB, full_bar + stage, smem_u32(sb + j * 8192), n0 + 64 * j, kb * BK);
       }
       if (++stage == STAGES) { stage = 0; phase ^= 1; }
     }
@@ -95,7 +95,7 @@ __device__ __forceinline__ void mma_loop(const TcParams& p, unsigned char* smem,
   constexpr int A_BYTES = BM * BK * 2, STAGE_BYTES = A_BYTES + BN * BK * 2;
   constexpr int UN = BN > 256 ? 256 : BN;          // UMMA N (<= 256): a 512-column tile is two MMAs per k-step
   constexpr int NACC = BN > 256 ? 1 : 2;           // accumulator stages in TMEM (512 columns in all)
-  constexpr uint32_t idesc = make_idesc(BM, UN, MODE_MN);
+  constexpr uint32_t idesc = make_idesc(BM, UN, MODE_MN, MODE_MN);
   const int total_tiles = p.tiles_m * p.tiles_n * p.splits;
   int stage = 0;
   uint32_t phase = 0;
@@ -116,15 +116,15 @@ __device__ __forceinline__ void mma_loop(const TcParams& p, unsigned char* smem,
       for (int k = 0; k < BK / UMMA_K; ++k) {
         uint64_t adesc, bdesc;
         if (MODE_MN == 0) {
-          adesc = make_smem_desc(sa + k * (UMMA_K * 2), 16, 1024);
-          bdesc = make_smem_desc(sb + k * (UMMA_K * 2), 16, 1024);
+          adesc = make_smem_desc(sa + k * (UMMA_K * 2), 16, 1024, 2);
+          bdesc = make_smem_desc(sb + k * (UMMA_K * 2), 16, 1024, 2);
         } else {
-          adesc = make_smem_desc(sa + k * (UMMA_K * 128), 8192, 1024);
-          bdesc = make_smem_desc(sb + k * (UMMA_K * 128), 8192, 1024);
+          adesc = make_smem_desc(sa + k * (UMMA_K * 128), 8192, 1024, 2);
+          bdesc = make_smem_desc(sb + k * (UMMA_K * 128), 8192, 1024, 2);
         }
         umma_bf16(tmem_d, adesc, bdesc, idesc, (kb > kb0 || k > 0) ? 1u : 0u);
         if (BN > 256)          // (K-major only: the row kernel) second half of the N columns: B rows 256.. of the stage
-          umma_bf16(tmem_d + 256u, adesc, make_smem_desc(sb + 256 * BK * 2 + k * (UMMA_K * 2), 16, 1024), idesc,
+          umma_bf16(tmem_d + 256u, adesc, make_smem_desc(sb + 256 * BK * 2 + k * (UMMA_K * 2), 16, 1024, 2), idesc,
                     (kb > kb0 || k > 0) ? 1u : 0u);
       }
       umma_commit(empty_bar + stage);            // frees the smem stage when the MMAs retire
@@ -217,13 +217,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_tc_kernel(const __grid_const
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
               const int k = grp * 4 + t;
-              uint32_t w0, w1, w2, w3;
-              asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(w0), "=r"(w1), "=r"(w2), "=r"(w3)
-                           : "r"(sa + (uint32_t)k * 128u + (uint32_t)(((q & 7) ^ (k & 7)) << 4)));
-              acc[0] += __uint_as_float(w0 << 16); acc[1] += __uint_as_float(w0 & 0xFFFF0000u);
-              acc[2] += __uint_as_float(w1 << 16); acc[3] += __uint_as_float(w1 & 0xFFFF0000u);
-              acc[4] += __uint_as_float(w2 << 16); acc[5] += __uint_as_float(w2 & 0xFFFF0000u);
-              acc[6] += __uint_as_float(w3 << 16); acc[7] += __uint_as_float(w3 & 0xFFFF0000u);
+              const uint4 w = lds128(sa + (uint32_t)k * 128u + (uint32_t)(((q & 7) ^ (k & 7)) << 4));
+              acc[0] += bf_lo(w.x); acc[1] += bf_hi(w.x);
+              acc[2] += bf_lo(w.y); acc[3] += bf_hi(w.y);
+              acc[4] += bf_lo(w.z); acc[5] += bf_hi(w.z);
+              acc[6] += bf_lo(w.w); acc[7] += bf_hi(w.w);
             }
           }
           __syncwarp();
@@ -233,14 +231,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_tc_kernel(const __grid_const
         if (mine) {
 #pragma unroll
           for (int j = 0; j < 8; ++j) atomicAdd(sred + q * 8 + j, acc[j]);
-          asm volatile("bar.sync 1, 256;" ::: "memory");
+          bar_sync(1, 256);
           if (et < 128) {
             const float v = sred[et];
             sred[et] = 0.f;
             const int mrow = tm * BM + et;
             if (mrow < p.M && v != 0.f) atomicAdd(epi.colsum_out + mrow, v);
           }
-          asm volatile("bar.sync 1, 256;" ::: "memory");
+          bar_sync(1, 256);
         }
       }
       mbar_wait(tfull_bar + as, aphase);
@@ -258,7 +256,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_tc_kernel(const __grid_const
       if (c_begin < c_end) tmem_ld32(taddr + c_begin, r);
 #pragma unroll 1
       for (int c = c_begin; c < c_end; c += 32) {
-        tmem_ld_wait();
+        tmem_ld_wait(r);
 #pragma unroll
         for (int j = 0; j < 32; j += 4)
           sts128(stg + (uint32_t)(lane * STG_LD + (((j >> 2) ^ (lane & 7)) << 2)) * 4, r[j], r[j + 1], r[j + 2],
@@ -269,7 +267,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_tc_kernel(const __grid_const
 #pragma unroll
         for (int it = 0; it < 8; ++it) {
           const int rr = it * 4 + sub_r;
-          v[it] = lds128(stg + (uint32_t)(rr * STG_LD + ((((lane & 7)) ^ (rr & 7)) << 2)) * 4);
+          v[it] = lds128f(stg + (uint32_t)(rr * STG_LD + ((((lane & 7)) ^ (rr & 7)) << 2)) * 4);
         }
 #pragma unroll
         for (int it = 0; it < 8; ++it)
@@ -353,32 +351,6 @@ template <int BN, int RE, int W = 8> struct RowCfg {
   static constexpr int THREADS = 64 + 32 * NEPI;
 };
 
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, uint32_t src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(map), "r"(src),
-               "r"(c0), "r"(c1)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void bulk_wait_read() {
-  asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
-}
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]),
-        "r"(r[18]), "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]),
-        "r"(r[27]), "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
-  __nv_bfloat162 t = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&t);
-}
 // thread-row access to a TMA-swizzled slab: 32 rows; fp32 rows are 128 B (SWIZZLE_128B: chunk ^= row & 7),
 // bf16 rows are 64 B (SWIZZLE_64B: chunk ^= (row >> 1) & 3)
 __device__ __forceinline__ uint32_t slab32_addr(uint32_t base, int row, int chunk) {
@@ -462,8 +434,8 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
     auto issue_in = [&](int t, int c, uint32_t gi) {
       uint64_t* nb = my_in_bar + (gi & 1);
       mbar_expect_tx(nb, IN_BYTES);
-      tma_load_2d(&mapIn, nb, egen + (C::IN_BUFS == 2 ? (gi & 1) : 0) * C::IN_STRIDE, (t % p.tiles_n) * BN + c * 32,
-                  (t / p.tiles_n) * BM + quad * 32);
+      tma_load_2d(&mapIn, nb, smem_u32(egen + (C::IN_BUFS == 2 ? (gi & 1) : 0) * C::IN_STRIDE),
+                  (t % p.tiles_n) * BN + c * 32, (t / p.tiles_n) * BM + quad * 32);
     };
     if (HAS_IN && lane == 0) {                        // first input slab
       int t = blockIdx.x, c = half;
@@ -498,15 +470,13 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
           }
           mbar_wait(my_in_bar + (g & 1), (g >> 1) & 1);
         }
-        uint32_t mw[16];                                // RE_MASK: this thread's 32 mask values (bf16 pairs)
+        uint4 mw[4];                                    // RE_MASK: this thread's 32 mask values (bf16 pairs)
         if (RE == RE_MASK) {
           const uint32_t ib = ebase + (C::IN_BUFS == 2 ? (g & 1) : 0) * C::IN_STRIDE;
 #pragma unroll
-          for (int k = 0; k < 4; ++k)
-            asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(mw[4 * k]), "=r"(mw[4 * k + 1]), "=r"(mw[4 * k + 2]),
-                         "=r"(mw[4 * k + 3]) : "r"(slab16_addr(ib, lane, k)));
+          for (int k = 0; k < 4; ++k) mw[k] = lds128(slab16_addr(ib, lane, k));
         }
-        tmem_ld_wait();
+        tmem_ld_wait(r);
         float v[32];
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
@@ -531,7 +501,7 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
         if (RE == RE_MASK) {
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
-            const uint32_t w[4] = {mw[4 * k], mw[4 * k + 1], mw[4 * k + 2], mw[4 * k + 3]};
+            const uint32_t w[4] = {mw[k].x, mw[k].y, mw[k].z, mw[k].w};
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
               // bf16 > 0  <=>  sign bit clear and magnitude non-zero
@@ -556,7 +526,7 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
           const uint32_t ib = ebase + (g & 1) * C::IN_STRIDE;
 #pragma unroll
           for (int k = 0; k < 8; ++k) {
-            const float4 q = lds128(slab32_addr(ib, lane, k));
+            const float4 q = lds128f(slab32_addr(ib, lane, k));
             v[4 * k] += q.x; v[4 * k + 1] += q.y; v[4 * k + 2] += q.z; v[4 * k + 3] += q.w;
           }
         }
@@ -610,8 +580,8 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
           __syncwarp();
 #pragma unroll
           for (int k = 0; k < 4; ++k)
-            sts128(slab16_addr(ob, lane, k), pack_bf16(v[8 * k], v[8 * k + 1]), pack_bf16(v[8 * k + 2], v[8 * k + 3]),
-                   pack_bf16(v[8 * k + 4], v[8 * k + 5]), pack_bf16(v[8 * k + 6], v[8 * k + 7]));
+            sts128(slab16_addr(ob, lane, k), pack2(v[8 * k], v[8 * k + 1]), pack2(v[8 * k + 2], v[8 * k + 3]),
+                   pack2(v[8 * k + 4], v[8 * k + 5]), pack2(v[8 * k + 6], v[8 * k + 7]));
           fence_proxy_async();
           __syncwarp();
           if (lane == 0) {
@@ -630,11 +600,9 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
         auto swap_partial = [&](float mine, int slot) -> float {
           if (lane == 0) bulk_wait_read<0>();
           __syncwarp();
-          asm volatile("st.shared.f32 [%0], %1;" ::"r"(xch_mine + (uint32_t)((slot * 32 + lane) * 4)), "f"(mine) : "memory");
-          asm volatile("bar.sync %0, 64;" ::"r"(1 + quad) : "memory");
-          float other;
-          asm volatile("ld.shared.f32 %0, [%1];" : "=f"(other) : "r"(xch_peer + (uint32_t)((slot * 32 + lane) * 4)) : "memory");
-          return mine + other;
+          sts32(xch_mine + (uint32_t)((slot * 32 + lane) * 4), __float_as_uint(mine));
+          bar_sync(1 + quad, 64);
+          return mine + lds32f(xch_peer + (uint32_t)((slot * 32 + lane) * 4));
         };
         if (NSPLIT == 2) sum = swap_partial(sum, 0);
         const float inv_n = 1.f / (float)p.N;
@@ -644,7 +612,7 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
         for (int ci = half; ci < nchunks; ci += NSPLIT) {
           uint32_t r[32];
           tmem_ld32(taddr + ci * 32, r);
-          tmem_ld_wait();
+          tmem_ld_wait(r);
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
             const float t = __uint_as_float(r[j]) - mean;
@@ -656,13 +624,13 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
         if (rp.rstd && m < p.M && half == 0) rp.rstd[m] = rstd;
         // ---------------- pass C: normalise, scale/shift, write y32 / y16 / xhat ---------------------
         const uint32_t o32 = ebase + 8192, o16 = ebase + 12288, oxh = ebase + 14336;
-        if (NSPLIT == 2) asm volatile("bar.sync %0, 64;" ::"r"(1 + quad) : "memory");   // the peer has read slot 1: staging may be reused
+        if (NSPLIT == 2) bar_sync(1 + quad, 64);   // the peer has read slot 1: staging may be reused
 #pragma unroll 1
         for (int ci = half; ci < nchunks; ci += NSPLIT) {
           const int n = n0 + ci * 32;
           uint32_t r[32];
           tmem_ld32(taddr + ci * 32, r);
-          tmem_ld_wait();
+          tmem_ld_wait(r);
           float xh[32], y[32];
 #pragma unroll
           for (int k = 0; k < 8; ++k) {
@@ -685,12 +653,12 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
                    __float_as_uint(y[4 * k + 2]), __float_as_uint(y[4 * k + 3]));
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
-            sts128(slab16_addr(o16, lane, k), pack_bf16(y[8 * k], y[8 * k + 1]), pack_bf16(y[8 * k + 2], y[8 * k + 3]),
-                   pack_bf16(y[8 * k + 4], y[8 * k + 5]), pack_bf16(y[8 * k + 6], y[8 * k + 7]));
+            sts128(slab16_addr(o16, lane, k), pack2(y[8 * k], y[8 * k + 1]), pack2(y[8 * k + 2], y[8 * k + 3]),
+                   pack2(y[8 * k + 4], y[8 * k + 5]), pack2(y[8 * k + 6], y[8 * k + 7]));
             if (rp.has_xhat)
-              sts128(slab16_addr(oxh, lane, k), pack_bf16(xh[8 * k], xh[8 * k + 1]),
-                     pack_bf16(xh[8 * k + 2], xh[8 * k + 3]), pack_bf16(xh[8 * k + 4], xh[8 * k + 5]),
-                     pack_bf16(xh[8 * k + 6], xh[8 * k + 7]));
+              sts128(slab16_addr(oxh, lane, k), pack2(xh[8 * k], xh[8 * k + 1]),
+                     pack2(xh[8 * k + 2], xh[8 * k + 3]), pack2(xh[8 * k + 4], xh[8 * k + 5]),
+                     pack2(xh[8 * k + 6], xh[8 * k + 7]));
           }
           fence_proxy_async();
           __syncwarp();
@@ -723,45 +691,23 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
 }
 
 // ---- host side ------------------------------------------------------------------------------------
-int get_encode_fn(EncodeTiledFn* out) {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    AMC_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q));
-    AMC_CHECK_ARG(p != nullptr && q == cudaDriverEntryPointSuccess, "cuTensorMapEncodeTiled not available");
-    fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  *out = fn;
-  return 0;
-}
-
 // 2-D tensor [rows, cols] row-major with pitch ld (elements); box = {box_cols, box_rows}; the box's inner
 // extent in bytes equals the swizzle span (128 B, or 64 B for 32-column bf16 epilogue slabs)
 int make_map_ex(CUtensorMap* map, const void* base, int rows, int cols, int ld, int box_cols, int box_rows,
                 bool is_f32, bool swz64) {
-  EncodeTiledFn enc;
-  AMC_TRY(get_encode_fn(&enc));
   const int esz = is_f32 ? 4 : 2;
   AMC_CHECK_ARG((reinterpret_cast<uintptr_t>(base) & 15) == 0, "GEMM tensor must be 16-byte aligned");
   AMC_CHECK_ARG(((size_t)ld * esz) % 16 == 0, "GEMM tensor pitch (%d elements) must be a multiple of 16 bytes", ld);
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * esz};
-  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, is_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
-                   const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   swz64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  AMC_CHECK_ARG(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed (%d) rows=%d cols=%d ld=%d", (int)r, rows, cols,
-                ld);
-  return 0;
+  const cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+  const cuuint64_t strides[1] = {(cuuint64_t)ld * esz};
+  const cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
+  return encode_tiled_map(map, is_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base,
+                          dims, strides, box, swz64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
+                          CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
 }
 int make_map(CUtensorMap* map, const void* base, int rows, int cols, int ld, int box_cols, int box_rows) {
   return make_map_ex(map, base, rows, cols, ld, box_cols, box_rows, false, false);
 }
-
-int num_sms() { return device_sm_count(); }
 
 template <int BN, int MODE_MN, int CS = 0>
 int launch(const GemmArgs& g, cudaStream_t st) {
@@ -785,7 +731,7 @@ int launch(const GemmArgs& g, cudaStream_t st) {
   p.vec_ok = epi_vec_ok<bf16>(g.epi, g.N) ? 1 : 0;
   const long long tiles = (long long)p.tiles_m * p.tiles_n * p.splits;
   AMC_CHECK_ARG(tiles < (1ll << 30), "gemm_bf16: too many tiles");
-  const int grid = (int)std::min<long long>(tiles, num_sms());
+  const int grid = (int)std::min<long long>(tiles, device_sm_count());
   auto kern = gemm_tc_kernel<BN, MODE_MN, CS>;
   AMC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
   kern<<<grid, NTHREADS, C::SMEM_BYTES, st>>>(mapA, mapB, p, g.epi);
@@ -824,7 +770,7 @@ int launch_row(const GemmArgs& g, cudaStream_t st) {
                 "gemm_bf16: fused column sums need a bf16-output epilogue and N <= 2048");
   const long long tiles = (long long)p.tiles_m * p.tiles_n;
   AMC_CHECK_ARG(tiles < (1ll << 30), "gemm_bf16: too many tiles");
-  const int grid = (int)std::min<long long>(tiles, num_sms());
+  const int grid = (int)std::min<long long>(tiles, device_sm_count());
   auto kern = gemm_tc_row_kernel<BN, RE, W>;
   AMC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
   kern<<<grid, C::THREADS, C::SMEM_BYTES, st>>>(mapA, mapB, mapIn, mapO16, mapO32, mapXh, p, rp);
@@ -842,6 +788,32 @@ int launch_row_bn(int bn, const GemmArgs& g, cudaStream_t st) {
 inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 }  // namespace
+
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+int encode_tiled_map(CUtensorMap* map, CUtensorMapDataType dtype, int rank, const void* base, const cuuint64_t* dims,
+                     const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapSwizzle swizzle,
+                     CUtensorMapL2promotion l2) {
+  static const EncodeTiledFn enc = [] {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
+        q != cudaDriverEntryPointSuccess) {
+      (void)cudaGetLastError();
+      p = nullptr;
+    }
+    return reinterpret_cast<EncodeTiledFn>(p);
+  }();
+  AMC_CHECK_ARG(enc != nullptr, "cuTensorMapEncodeTiled not available");
+  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+  const CUresult r = enc(map, dtype, (cuuint32_t)rank, const_cast<void*>(base), dims, strides, box, estr,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  AMC_CHECK_ARG(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed (%d): rank %d, inner dim %llu, box %u x %u", (int)r,
+                rank, (unsigned long long)dims[0], box[0], box[1]);
+  return 0;
+}
 
 int gemm_bf16(const GemmArgs& g, cudaStream_t st) {
   AMC_CHECK_ARG(g.M > 0 && g.N > 0 && g.K > 0, "gemm_bf16: empty problem M=%d N=%d K=%d", g.M, g.N, g.K);
