@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AMC_ABI_VERSION 8
+#define AMC_ABI_VERSION 9
 
 enum { AMC_KIND_RAWIQ = 0, AMC_KIND_VIT = 1 };
 enum { AMC_F32 = 0, AMC_BF16 = 1 };
@@ -234,6 +234,15 @@ int amc_gemm(int dtype, int M, int N, int K, const void* A, int lda, int transA,
 int amc_gemm_ln(int M, int N, int K, const void* A, int lda, const void* B, int ldb, const float* bias,
                 const float* res32, const float* gamma, const float* beta, float eps, void* y16, float* y32,
                 void* xhat, float* rstd, amc_stream_t stream);
+/* bf16 GEMM with the fused LayerNorm-backward epilogue used by the encoder block's backward: the activation gradient
+ * that feeds a post-LN norm, and that norm's backward (amc_layernorm_bwd) on it, in one pass:
+ *   t = A B^T + res32 (the gradient of the norm's output) ; du = rstd * (g - mean(g) - xhat * mean(g*xhat)), g = t*gamma
+ *   over each row (N <= 256, N % 32 == 0); xhat (bf16 [M,N]) and rstd (fp32 [M]) are the forward's.
+ *   du16 (bf16) and du32 (fp32) both receive du; dgamma += sum t*xhat, dbeta += sum t, dbias += sum du over the rows
+ *   (each nullable, accumulated: bias gradient of the layer that produced the norm's input). */
+int amc_gemm_ln_bwd(int M, int N, int K, const void* A, int lda, const void* B, int ldb, const float* res32,
+                    const void* xhat, const float* rstd, const float* gamma, void* du16, float* du32, float* dgamma,
+                    float* dbeta, float* dbias, amc_stream_t stream);
 /* bf16 GEMM whose epilogue applies the ReLU(+dropout) backward mask taken from the stored hidden activations
  * (position_wise_feed_forward.py:14-15 backward): D16 = (A B^T) * (mask > 0 ? mask_scale : 0). */
 int amc_gemm_relu_mask(int M, int N, int K, const void* A, int lda, const void* B, int ldb, const void* mask,

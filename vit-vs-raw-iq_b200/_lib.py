@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libamc_b200.so")
 
-ABI_VERSION = 8
+ABI_VERSION = 9
 KIND_RAWIQ, KIND_VIT = 0, 1
 F32, BF16 = 0, 1
 INPUT_MODEL, INPUT_RAW = 0, 1
@@ -71,6 +71,7 @@ def _load():
         "amc_adv_init": [i64, i64, i32, vp, vp, C.c_uint64, C.c_uint64, vp, vp, vp],
         "amc_gemm": [i32, i32, i32, i32, vp, i32, i32, vp, i32, i32, vp, vp, i32, i32, vp, i32, vp, i32, i32, vp],
         "amc_gemm_ln": [i32, i32, i32, vp, i32, vp, i32, vp, vp, vp, vp, f32, vp, vp, vp, vp, vp],
+        "amc_gemm_ln_bwd": [i32, i32, i32, vp, i32, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp],
         "amc_gemm_relu_mask": [i32, i32, i32, vp, i32, vp, i32, vp, f32, vp, vp],
         "amc_attention_fwd": [i32, i32, i32, i32, i32, vp, vp, vp, vp],
         "amc_attention_bwd": [i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp],

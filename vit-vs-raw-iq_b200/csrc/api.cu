@@ -556,16 +556,33 @@ struct Model {
     return gemm<E>(g, st);
   }
 
-  // backward of post_fwd_part on the same row view: consumes r.dy32, leaves the out-proj input gradient in
-  // r.dO (row pitch r.lddO) and the skip gradient of the layer input in r.du32
+  // With fuse_ln(), LayerNorm backward runs in the epilogue of the dgrad GEMM that produces the gradient of the norm's
+  // output: dgrad FFN1 for norm1, and for norm2 of layer l the dgrad QKV of layer l + 1.  The top layer's norm2 takes its
+  // output gradient from the head (or denc_out) and keeps the separate ln_bwd.
+  bool ln2_bwd_fused(int l) const { return fuse_ln() && l < m.L - 1; }
+  // ... the epilogue: norm (gamma at goff, beta at boff) of layer l with its saved xhat / rstd, dropout `site` on du16,
+  // and dbias (offset dboff) += column sums of du16: the bias gradient of the sub-layer whose output the norm took
+  void ln_bwd_epilogue(GemmArgs& g, int l, const void* xhat, const float* rstd, int64_t goff, int64_t boff, int64_t dboff,
+                       uint32_t site, void* du16, float* du32) {
+    g.epi.ln_bwd = 1;
+    g.epi.ln_xhat = const_cast<void*>(xhat); g.epi.ln_rstd = const_cast<float*>(rstd); g.epi.ln_gamma = PL(l, goff);
+    g.epi.ln_dgamma = GL(l, goff); g.epi.ln_dbeta = GL(l, boff); g.epi.colsum_out = GL(l, dboff);
+    g.epi.drop = drop; g.epi.drop_site = site;
+    g.epi.D16 = du16; g.epi.ldd16 = m.d; g.epi.D32 = du32; g.epi.ldd32 = m.d;
+  }
+
+  // backward of post_fwd_part on the same row view: consumes r.dy32 (or, when the dgrad QKV of layer l + 1 has done
+  // norm2's backward, r.dw16 / r.dw32; only on all rows, the CLS view being the top layer's), leaves the out-proj input gradient in r.dO (row pitch r.lddO) and the skip
+  // gradient of the layer input in r.du32
   int post_bwd_part(int l, const Rows& r) {
     const int d = m.d, F = m.F, Mr = r.n;
     const int64_t dd = (int64_t)d * d;
     GemmArgs g;
     // norm2 backward; dw16 carries dropout2's mask (operand of the FFN2 gradients), dw32 is the skip path
-    AMC_PROF("ln_bwd", 0.0, (double)Mr * d * (8 + 2 * sizeof(E)),
-             ln_bwd<E>(Mr, d, r.dy32, (const E*)r.xhat2, r.rstd2, PL(l, L.g2), (E*)r.dw16, r.dw32, GL(l, L.g2),
-                       GL(l, L.be2), GL(l, L.b2), drop, site_ffn(l), st));
+    if (!ln2_bwd_fused(l))
+      AMC_PROF("ln_bwd", 0.0, (double)Mr * d * (8 + 2 * sizeof(E)),
+               ln_bwd<E>(Mr, d, r.dy32, (const E*)r.xhat2, r.rstd2, PL(l, L.g2), (E*)r.dw16, r.dw32, GL(l, L.g2),
+                         GL(l, L.be2), GL(l, L.b2), drop, site_ffn(l), st));
     AMC_TRY(wgrad_n(Mr, d, F, r.dw16, d, r.hid, F, GL(l, L.w2), nullptr));
     // dgrad FFN2 with the ReLU/dropout mask taken from the stored hidden
     g.M = Mr; g.N = F; g.K = d; g.A = r.dw16; g.lda = d;
@@ -582,12 +599,19 @@ struct Model {
     g.M = Mr; g.N = d; g.K = F; g.A = r.da; g.lda = F;
     dgrad_operand(g, l, L.w1, 4 * dd, F, d);
     g.name = "gemm_dgrad_ffn1";
-    g.epi.res32 = r.dw32; g.epi.ldres = d; g.epi.D32 = r.t32; g.epi.ldd32 = d;
-    AMC_TRY(gemm<E>(g, st));
-    // norm1 backward
-    AMC_PROF("ln_bwd", 0.0, (double)Mr * d * (8 + 2 * sizeof(E)),
-             ln_bwd<E>(Mr, d, r.t32, (const E*)r.xhat1, r.rstd1, PL(l, L.g1), (E*)r.du16, r.du32, GL(l, L.g1),
-                       GL(l, L.be1), GL(l, L.bo), drop, site_attn(l), st));
+    g.epi.res32 = r.dw32; g.epi.ldres = d;
+    if (fuse_ln()) {   // + norm1 backward
+      g.name = "gemm_dgrad_ffn1_lnb";
+      ln_bwd_epilogue(g, l, r.xhat1, r.rstd1, L.g1, L.be1, L.bo, site_attn(l), r.du16, r.du32);
+      AMC_TRY(gemm<E>(g, st));
+    } else {
+      g.epi.D32 = r.t32; g.epi.ldd32 = d;
+      AMC_TRY(gemm<E>(g, st));
+      // norm1 backward
+      AMC_PROF("ln_bwd", 0.0, (double)Mr * d * (8 + 2 * sizeof(E)),
+               ln_bwd<E>(Mr, d, r.t32, (const E*)r.xhat1, r.rstd1, PL(l, L.g1), (E*)r.du16, r.du32, GL(l, L.g1),
+                         GL(l, L.be1), GL(l, L.bo), drop, site_attn(l), st));
+    }
     AMC_TRY(wgrad_n(Mr, d, d, r.du16, d, r.o, r.ldo, GL(l, L.wo), nullptr));
     g = GemmArgs();
     g.M = Mr; g.N = d; g.K = d; g.A = r.du16; g.lda = d;
@@ -622,6 +646,19 @@ struct Model {
     g.M = M; g.N = d; g.K = 3 * d; g.A = w.dqkv; g.lda = 3 * d;
     dgrad_operand(g, l, L.wq, 0, 3 * d, d);
     g.name = "gemm_dgrad_qkv";
+    if (l > 0 && ln2_bwd_fused(l - 1)) {
+      // + norm2 backward of layer l - 1: its dw16 / dw32 are written here
+      if (cls_only) {   // the skip gradient exists on the CLS rows only: spread it over a zeroed full-size residual
+        AMC_CUDA(cudaMemsetAsync(w.du32, 0, (size_t)M * d * 4, st));
+        add_rows_kernel<<<ceil_div(m.B * d, 256), 256, 0, st>>>(m.B, d, w.du32, m.T * d, w.c.du32);
+        AMC_LAUNCH_CHECK();
+      }
+      const LayerBuf& bp = LB(l - 1);
+      g.name = "gemm_dgrad_qkv_lnb";
+      g.epi.res32 = w.du32; g.epi.ldres = d;
+      ln_bwd_epilogue(g, l - 1, bp.xhat2, bp.rstd2, L.g2, L.be2, L.b2, site_ffn(l - 1), w.dw16, w.dw32);
+      return gemm<E>(g, st);
+    }
     g.epi.D32 = w.dy32; g.epi.ldd32 = d;
     if (!cls_only) { g.epi.res32 = w.du32; g.epi.ldres = d; }
     AMC_TRY(gemm<E>(g, st));
@@ -859,6 +896,19 @@ int amc_gemm_ln(int M, int N, int K, const void* A, int lda, const void* B, int 
   g.epi.bias = bias; g.epi.res32 = res32; g.epi.ldres = N; g.epi.ln_gamma = gamma; g.epi.ln_beta = beta;
   g.epi.ln_eps = eps; g.epi.D16 = y16; g.epi.ldd16 = N; g.epi.D32 = y32; g.epi.ldd32 = N; g.epi.ln_xhat = xhat;
   g.epi.ln_rstd = rstd;
+  return gemm_bf16(g, (cudaStream_t)stream);
+}
+
+int amc_gemm_ln_bwd(int M, int N, int K, const void* A, int lda, const void* B, int ldb, const float* res32,
+                    const void* xhat, const float* rstd, const float* gamma, void* du16, float* du32, float* dgamma,
+                    float* dbeta, float* dbias, amc_stream_t stream) {
+  DeviceGuard dev_guard(A);
+  AMC_CHECK_ARG(A && B && res32 && xhat && rstd && gamma && du16 && du32, "NULL argument");
+  GemmArgs g;
+  g.M = M; g.N = N; g.K = K; g.A = A; g.lda = lda; g.B = B; g.ldb = ldb;
+  g.epi.ln_bwd = 1; g.epi.res32 = res32; g.epi.ldres = N; g.epi.ln_xhat = const_cast<void*>(xhat);
+  g.epi.ln_rstd = const_cast<float*>(rstd); g.epi.ln_gamma = gamma; g.epi.D16 = du16; g.epi.ldd16 = N; g.epi.D32 = du32;
+  g.epi.ldd32 = N; g.epi.ln_dgamma = dgamma; g.epi.ln_dbeta = dbeta; g.epi.colsum_out = dbias;
   return gemm_bf16(g, (cudaStream_t)stream);
 }
 

@@ -34,6 +34,12 @@ struct Epi {
   float ln_eps = 0.f;
   void* ln_xhat = nullptr;
   float* ln_rstd = nullptr;
+  // fused LayerNorm backward instead (ln_bwd = 1; bf16 tcgen05 path, N <= 256): t = acc + res32 is the gradient of the
+  // norm's output; reads ln_xhat (pitch N), ln_rstd, ln_gamma -> D32 = du, D16 = du * dropout(drop, drop_site);
+  // ln_dgamma / ln_dbeta += sum t * xhat / sum t, colsum_out += sum D16 (fp32, before rounding); each nullable
+  int ln_bwd = 0;
+  float* ln_dgamma = nullptr;
+  float* ln_dbeta = nullptr;
 };
 
 // ---- fast path: whole float4 in bounds, every pointer vector-aligned; registers only -------------

@@ -299,8 +299,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_tc_kernel(const __grid_const
 //   RE_RES32 : D32 = (acc + bias) [* dropout] + res32                     (dgrad FFN1 / dgrad QKV skips)
 //   RE_LN    : u = (acc + bias)[* dropout] + res32 ; LayerNorm(u) over the row (N <= BN) ->
 //              y16, y32, xhat, rstd.  u is parked in TMEM between the passes (mean, variance, write).
+//   RE_LNB   : t = acc + res32 ; LayerNorm backward of t over the row (N <= BN <= 256) with the forward's xhat / rstd ->
+//              D32 = du, D16 = du [* dropout]; column sums dgamma += t * xhat, dbeta += t, colsum_out += D16 (fp32).
 // =================================================================================================
-enum { RE_BF16 = 0, RE_MASK = 1, RE_RES32 = 2, RE_LN = 3 };
+enum { RE_BF16 = 0, RE_MASK = 1, RE_RES32 = 2, RE_LN = 3, RE_LNB = 4 };
 
 struct RowParams {
   const float* bias;
@@ -311,15 +313,17 @@ struct RowParams {
   const float* gamma;
   const float* beta;
   float ln_eps;
-  float* rstd;
+  float* rstd;         // RE_LN: written; RE_LNB: read
   int has_xhat;
-  float* colsum_out;   // RE_MASK / RE_BF16: += column sums of the values written (bias gradient of the producer layer)
+  float* colsum_out;   // RE_MASK / RE_BF16 / RE_LNB: += column sums of the values written (bias gradient of the producer layer)
+  float* dgamma;       // RE_LNB: += LayerNorm parameter gradients (nullable)
+  float* dbeta;
   int n_cols;          // N (size of the shared-memory column accumulator)
 };
 
 template <int BN, int RE, int W = 8> struct RowCfg {
   // (the two-warps-per-quadrant LayerNorm epilogue pays for its second set of slabs with one operand stage)
-  static constexpr bool LN8 = (RE == RE_LN && W == 8);
+  static constexpr bool LN8 = ((RE == RE_LN || RE == RE_LNB) && W == 8);
   static constexpr int STAGES = BN > 256 ? 2 : (LN8 ? ((BN == 256) ? 2 : (BN == 128 ? 3 : 4)) : ((BN == 256) ? 3 : (BN == 128 ? 4 : 6)));
   static constexpr int STAGE_BYTES = BM * BK * 2 + BN * BK * 2;
   // bf16-output epilogues are instruction-heavy (dropout hash, mask tests, packing): two warps per TMEM
@@ -335,17 +339,23 @@ template <int BN, int RE, int W = 8> struct RowCfg {
   // The LayerNorm epilogue (three passes over the row) takes W = 8 = two warps per quadrant for K <= 256 (out-proj): each
   // warp owns every other 32-column chunk of its rows through all three passes and the two partial row sums / sums of
   // squares are exchanged through the partner's (idle until pass C) staging area around a 64-thread named barrier.
+  // The LayerNorm-backward epilogue (two passes, three column sums, the dropout hash) bounds its GEMMs even at K = 3d / F:
+  // with one warp per quadrant the fused dgrad FFN1 / QKV took as long as the GEMM + ln_bwd pair it replaced.  It runs
+  // W = 8, two warps per quadrant as RE_LN does, with a single-buffered 6 KB input slab (fp32 residual + bf16 xhat) and
+  // single-buffered 4 + 2 KB output staging, 12 KB per warp next to the LN8 operand stages.
   static constexpr bool WIDE = (RE == RE_RES32 || RE == RE_LN);        // fp32 slabs: 4 KB in, 4 + 2 + 2 KB out
-  static constexpr int NEPI = WIDE ? (LN8 ? 8 : 4) : W;
-  static constexpr int EPW = WIDE ? 16384 : ((NEPI == 16) ? 4096 : 8192);   // epilogue bytes per warp
+  static constexpr bool LNB = (RE == RE_LNB);
+  static constexpr int NEPI = LNB ? 8 : (WIDE ? (LN8 ? 8 : 4) : W);
+  static constexpr int EPW = LNB ? 12288 : (WIDE ? 16384 : ((NEPI == 16) ? 4096 : 8192));   // epilogue bytes per warp
   static constexpr int IN_STRIDE = WIDE ? 4096 : 2048;
   static constexpr int IN_BUFS = (!WIDE && NEPI == 16) ? 1 : 2;
   static constexpr int OUT_BUFS = (NEPI == 16 && RE == RE_MASK) ? 1 : 2;
   static constexpr int OUT_OFF = WIDE ? 8192 : ((NEPI == 16) ? (RE == RE_MASK ? 2048 : 0) : 4096);
   static constexpr int EPI_OFF = STAGES * STAGE_BYTES;
   static constexpr int BAR_OFF = EPI_OFF + NEPI * EPW;
-  static constexpr int CS_OFF = BAR_OFF + 512;             // fp32 column accumulator (N <= 2048), bf16-output variants
-  static constexpr int CS_BYTES = WIDE ? 0 : 8192;
+  // fp32 column accumulator: N <= 2048 for the bf16-output variants, [colsum | dgamma | dbeta] x N <= 256 for RE_LNB
+  static constexpr int CS_OFF = BAR_OFF + 512;
+  static constexpr int CS_BYTES = LNB ? 4096 : (WIDE ? 0 : 8192);
   static constexpr int SMEM_BYTES = CS_OFF + CS_BYTES + 1024;
   static constexpr int TMEM_COLS = BN > 256 ? BN : 2 * BN;      // 512-column tiles: single-buffered accumulator
   static constexpr int THREADS = 64 + 32 * NEPI;
@@ -358,6 +368,22 @@ __device__ __forceinline__ uint32_t slab32_addr(uint32_t base, int row, int chun
 }
 __device__ __forceinline__ uint32_t slab16_addr(uint32_t base, int row, int chunk) {
   return base + row * 64 + ((chunk ^ ((row >> 1) & 3)) << 4);
+}
+
+// column sums of a warp's 32 rows x 32 columns (lane = row, t[j] = column j): transpose-reduce butterfly
+// (31 shuffles), lane j returns the sum of column j.  t is consumed.
+__device__ __forceinline__ float warp_colsum32(float (&t)[32], int lane) {
+#pragma unroll
+  for (int sft = 16; sft >= 1; sft >>= 1) {
+    const bool up = (lane & sft) != 0;
+#pragma unroll
+    for (int j = 0; j < sft; ++j) {
+      const float send = up ? t[j] : t[j + sft];
+      const float recv = __shfl_xor_sync(0xffffffffu, send, sft);
+      t[j] = (up ? t[j + sft] : t[j]) + recv;
+    }
+  }
+  return t[0];
 }
 
 template <int BN, int RE, int W = 8>
@@ -395,10 +421,11 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
     fence_barrier_init();
   }
   if (warp == 1) tmem_alloc(tmem_slot, C::TMEM_COLS);
-  float* sacc = reinterpret_cast<float*>(smem + C::CS_OFF);
-  const bool do_cs = C::CS_BYTES > 0 && rp.colsum_out != nullptr;
+  float* sacc = reinterpret_cast<float*>(smem + C::CS_OFF);   // [colsum | dgamma | dbeta] x n_cols
+  const bool do_cs = C::CS_BYTES > 0 && (rp.colsum_out != nullptr || rp.dgamma != nullptr || rp.dbeta != nullptr);
+  const int cs_len = (RE == RE_LNB ? 3 : 1) * rp.n_cols;
   if (do_cs)
-    for (int i = threadIdx.x; i < rp.n_cols; i += blockDim.x) sacc[i] = 0.f;
+    for (int i = threadIdx.x; i < cs_len; i += blockDim.x) sacc[i] = 0.f;
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -408,6 +435,169 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
     if (lane == 0) producer_loop<BN, 0, C::STAGES>(&mapA, &mapB, p, smem, full_bar, empty_bar);
   } else if (warp == 1) {
     if (lane == 0) mma_loop<BN, 0, C::STAGES>(p, smem, full_bar, empty_bar, tfull_bar, tempty_bar, tmem_base);
+  } else if constexpr (RE == RE_LNB) {
+    // ===================== LayerNorm backward: thread = accumulator row, two warps per quadrant =====================
+    //   pass A: t = acc + res32 ; s1 = sum t*gamma, s2 = sum t*gamma*xhat ; dgamma += t*xhat, dbeta += t ; t -> TMEM
+    //   pass B: du = rstd * (t*gamma - s1/N - xhat*s2/N) -> D32 ; du * dropout -> D16, colsum_out
+    // Each warp owns every other 32-column chunk of its quadrant's rows through both passes; the partial s1 / s2 are
+    // swapped with the partner through the output staging (idle between the passes) around a 64-thread named barrier.
+    // t is parked in place of the accumulator, so all 2 x BN TMEM columns are taken; xhat is fetched a second time in
+    // pass B (an L2 hit: pass A read it moments before).  Keeping the xhat rows in shared memory instead would take
+    // 64 KB at N = 256, more than the operand stages can give up.
+    // A warp's slabs for a tile: k < nmine are pass A's (fp32 residual 4 KB + bf16 xhat 2 KB), then pass B's (xhat);
+    // the buffer is single: the next slab is requested as soon as the current one is in registers.
+    constexpr int NSPLIT = C::NEPI / 4;
+    const int ew = warp - 2, quad = warp & 3, half = ew >> 2;
+    const uint32_t ebase = smem_u32(smem + C::EPI_OFF + ew * C::EPW);
+    const uint32_t o32 = ebase + 6144, o16 = ebase + 10240;
+    const uint32_t xch_peer = smem_u32(smem + C::EPI_OFF + (ew ^ 4) * C::EPW) + 10240;
+    uint64_t* my_in_bar = in_bar + ew * 2;
+    const int nc = p.N >> 5;                           // N <= BN: one tile spans the row
+    const int nmine = (nc - half + NSPLIT - 1) / NSPLIT;
+    const bool cs_ln = do_cs && (rp.dgamma != nullptr || rp.dbeta != nullptr);
+    const bool cs_b = do_cs && rp.colsum_out != nullptr;
+    const float inv_n = 1.f / (float)p.N;
+    auto issue = [&](int t, int k, uint32_t gi) {
+      uint64_t* nb = my_in_bar + (gi & 1);
+      const int row = t * BM + quad * 32;
+      if (k < nmine) {
+        const int c = half + k * NSPLIT;
+        mbar_expect_tx(nb, 6144);
+        tma_load_2d(&mapIn, nb, ebase, c * 32, row);
+        tma_load_2d(&mapXh, nb, ebase + 4096, c * 32, row);
+      } else {
+        mbar_expect_tx(nb, 2048);
+        tma_load_2d(&mapXh, nb, ebase + 4096, (half + (k - nmine) * NSPLIT) * 32, row);
+      }
+    };
+    auto issue_next = [&](int t, int k, uint32_t gi) {   // slab after (t, k), once every lane has read the buffer
+      __syncwarp();
+      if (lane != 0) return;
+      if (++k == 2 * nmine) { t += gridDim.x; k = 0; }
+      if (t < total_tiles) issue(t, k, gi);
+    };
+    auto load_xhat = [&](float (&xh)[32]) {
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const uint4 w = lds128(slab16_addr(ebase + 4096, lane, k));
+        xh[8 * k] = bf_lo(w.x); xh[8 * k + 1] = bf_hi(w.x); xh[8 * k + 2] = bf_lo(w.y); xh[8 * k + 3] = bf_hi(w.y);
+        xh[8 * k + 4] = bf_lo(w.z); xh[8 * k + 5] = bf_hi(w.z); xh[8 * k + 6] = bf_lo(w.w); xh[8 * k + 7] = bf_hi(w.w);
+      }
+    };
+    uint32_t g = 0;
+    int as = 0;
+    uint32_t aphase = 0;
+    if (nmine > 0 && lane == 0 && (int)blockIdx.x < total_tiles) issue(blockIdx.x, 0, 0);
+    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
+      const int m_slab = tile * BM + quad * 32, m = m_slab + lane;
+      mbar_wait(tfull_bar + as, aphase);
+      tc_fence_after();
+      const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(as * BN);
+      const float rs = m < p.M ? __ldg(rp.rstd + m) : 0.f;
+      float s1 = 0.f, s2 = 0.f;
+#pragma unroll 1
+      for (int k = 0; k < nmine; ++k, ++g) {           // ---------------- pass A ----------------
+        const int n = (half + k * NSPLIT) * 32;
+        uint32_t r[32];
+        tmem_ld32(taddr + n, r);
+        mbar_wait(my_in_bar + (g & 1), (g >> 1) & 1);
+        float q[32], xh[32];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const float4 v = lds128f(slab32_addr(ebase, lane, j));
+          q[4 * j] = v.x; q[4 * j + 1] = v.y; q[4 * j + 2] = v.z; q[4 * j + 3] = v.w;
+        }
+        load_xhat(xh);
+        issue_next(tile, k, g + 1);
+        tmem_ld_wait(r);
+        float* t = q;                                  // t = acc + res32, in place
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const float4 gm = __ldg(reinterpret_cast<const float4*>(rp.gamma + n) + j);
+          const float gk[4] = {gm.x, gm.y, gm.z, gm.w};
+#pragma unroll
+          for (int i = 0; i < 4; ++i) {
+            t[4 * j + i] += __uint_as_float(r[4 * j + i]);
+            const float gg = t[4 * j + i] * gk[i];
+            s1 += gg;
+            s2 = fmaf(gg, xh[4 * j + i], s2);
+            r[4 * j + i] = __float_as_uint(t[4 * j + i]);
+          }
+        }
+        tmem_st32(taddr + n, r);
+        if (cs_ln) {
+          // rows beyond M are exactly zero here (TMA zero fill of A, the residual and xhat) and add nothing
+#pragma unroll
+          for (int j = 0; j < 32; ++j) xh[j] *= t[j];
+          atomicAdd(sacc + p.N + n + lane, warp_colsum32(xh, lane));
+          atomicAdd(sacc + 2 * p.N + n + lane, warp_colsum32(q, lane));
+        }
+      }
+      tmem_st_wait();
+      if (NSPLIT == 2) {   // partner's partial sums, through its output staging (its last TMA store has read it)
+        if (lane == 0) bulk_wait_read<0>();
+        __syncwarp();
+        sts32(o16 + (uint32_t)(lane * 4), __float_as_uint(s1));
+        sts32(o16 + (uint32_t)((32 + lane) * 4), __float_as_uint(s2));
+        bar_sync(1 + quad, 64);
+        s1 += lds32f(xch_peer + (uint32_t)(lane * 4));
+        s2 += lds32f(xch_peer + (uint32_t)((32 + lane) * 4));
+        bar_sync(1 + quad, 64);                        // the peer has read mine: the staging may be reused
+      }
+      s1 *= inv_n;
+      s2 *= inv_n;
+#pragma unroll 1
+      for (int k = 0; k < nmine; ++k, ++g) {           // ---------------- pass B ----------------
+        const int n = (half + k * NSPLIT) * 32;
+        uint32_t r[32];
+        tmem_ld32(taddr + n, r);
+        mbar_wait(my_in_bar + (g & 1), (g >> 1) & 1);
+        float xh[32];
+        load_xhat(xh);
+        issue_next(tile, nmine + k, g + 1);
+        tmem_ld_wait(r);
+        float du[32];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const float4 gm = __ldg(reinterpret_cast<const float4*>(rp.gamma + n) + j);
+          const float gk[4] = {gm.x, gm.y, gm.z, gm.w};
+#pragma unroll
+          for (int i = 0; i < 4; ++i)
+            du[4 * j + i] = rs * (__uint_as_float(r[4 * j + i]) * gk[i] - s1 - xh[4 * j + i] * s2);
+        }
+        if (lane == 0) bulk_wait_read<0>();             // single-buffered staging: previous stores have read it
+        __syncwarp();
+#pragma unroll
+        for (int j = 0; j < 8; ++j)
+          sts128(slab32_addr(o32, lane, j), __float_as_uint(du[4 * j]), __float_as_uint(du[4 * j + 1]),
+                 __float_as_uint(du[4 * j + 2]), __float_as_uint(du[4 * j + 3]));
+        if (rp.drop.p > 0.f) {                          // the masks of ln_bwd: element index m * N + n
+          const uint64_t e0 = ((uint64_t)m * (uint64_t)p.N + (uint64_t)n) >> 2;
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            const float4 d = dropout_mult4(rp.drop, rp.drop_site, e0 + j);
+            du[4 * j] *= d.x; du[4 * j + 1] *= d.y; du[4 * j + 2] *= d.z; du[4 * j + 3] *= d.w;
+          }
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+          sts128(slab16_addr(o16, lane, j), pack2(du[8 * j], du[8 * j + 1]), pack2(du[8 * j + 2], du[8 * j + 3]),
+                 pack2(du[8 * j + 4], du[8 * j + 5]), pack2(du[8 * j + 6], du[8 * j + 7]));
+        fence_proxy_async();
+        __syncwarp();
+        if (lane == 0) {
+          tma_store_2d(&mapO32, o32, n, m_slab);
+          tma_store_2d(&mapO16, o16, n, m_slab);
+          bulk_commit();
+        }
+        if (cs_b) atomicAdd(sacc + n + lane, warp_colsum32(du, lane));   // rows beyond M: rstd 0, du 0
+      }
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(tempty_bar + as);
+      if (++as == 2) { as = 0; aphase ^= 1; }
+    }
+    if (lane == 0) bulk_wait_all();
   } else {
     // ===================== epilogue: thread = accumulator row =====================
     constexpr bool HAS_IN = (RE != RE_BF16);
@@ -531,22 +721,12 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
           }
         }
         if ((RE == RE_MASK || RE == RE_BF16) && do_cs) {
-          // column sums over the warp's 32 rows: transpose-reduce butterfly (31 shuffles), lane j ends up
-          // with the sum of column n + j; rows beyond M hold zeros (TMA zero fill) and add nothing
+          // column sums over the warp's 32 rows: lane j ends up with the sum of column n + j; rows beyond M hold
+          // zeros (TMA zero fill) and add nothing
           float t[32];
 #pragma unroll
           for (int j = 0; j < 32; ++j) t[j] = (m < p.M) ? v[j] : 0.f;
-#pragma unroll
-          for (int sft = 16; sft >= 1; sft >>= 1) {
-            const bool up = (lane & sft) != 0;
-#pragma unroll
-            for (int j = 0; j < sft; ++j) {
-              const float send = up ? t[j] : t[j + sft];
-              const float recv = __shfl_xor_sync(0xffffffffu, send, sft);
-              t[j] = (up ? t[j + sft] : t[j]) + recv;
-            }
-          }
-          atomicAdd(sacc + n + lane, t[0]);
+          atomicAdd(sacc + n + lane, warp_colsum32(t, lane));
         }
         if (RE == RE_LN) {
           uint32_t w[32];
@@ -680,9 +860,11 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
   tc_fence_before();
   __syncthreads();
   if (do_cs)
-    for (int i = threadIdx.x; i < rp.n_cols; i += blockDim.x) {
+    for (int i = threadIdx.x; i < cs_len; i += blockDim.x) {
+      const int s = i / rp.n_cols;
+      float* dst = s == 0 ? rp.colsum_out : (s == 1 ? rp.dgamma : rp.dbeta);
       const float vsum = sacc[i];
-      if (vsum != 0.f) atomicAdd(rp.colsum_out + i, vsum);
+      if (dst && vsum != 0.f) atomicAdd(dst + (i - s * rp.n_cols), vsum);
     }
   if (warp == 1) {
     tc_fence_after();
@@ -748,10 +930,11 @@ int launch_row(const GemmArgs& g, cudaStream_t st) {
   AMC_TRY(make_map(&mapB, g.B, g.N, g.K, g.ldb, BK, BN > 256 ? 256 : BN));
   mapIn = mapA; mapO16 = mapA; mapO32 = mapA; mapXh = mapA;      // placeholders for unused descriptors
   if (RE == RE_MASK) AMC_TRY(make_map_ex(&mapIn, e.mask_src, g.M, g.N, e.ldmask, 32, 32, false, true));
-  if (RE == RE_RES32 || RE == RE_LN) AMC_TRY(make_map_ex(&mapIn, e.res32, g.M, g.N, e.ldres, 32, 32, true, false));
+  if (RE == RE_RES32 || RE == RE_LN || RE == RE_LNB)
+    AMC_TRY(make_map_ex(&mapIn, e.res32, g.M, g.N, e.ldres, 32, 32, true, false));
   if (e.D16) AMC_TRY(make_map_ex(&mapO16, e.D16, g.M, g.N, e.ldd16, 32, 32, false, true));
   if (e.D32) AMC_TRY(make_map_ex(&mapO32, e.D32, g.M, g.N, e.ldd32, 32, 32, true, false));
-  if (RE == RE_LN && e.ln_xhat) AMC_TRY(make_map_ex(&mapXh, e.ln_xhat, g.M, g.N, g.N, 32, 32, false, true));
+  if ((RE == RE_LN || RE == RE_LNB) && e.ln_xhat) AMC_TRY(make_map_ex(&mapXh, e.ln_xhat, g.M, g.N, g.N, 32, 32, false, true));
   TcParams p;
   p.M = g.M; p.N = g.N; p.K = g.K;
   p.tiles_m = ceil_div(g.M, BM);
@@ -765,6 +948,7 @@ int launch_row(const GemmArgs& g, cudaStream_t st) {
   rp.gamma = e.ln_gamma; rp.beta = e.ln_beta; rp.ln_eps = e.ln_eps; rp.rstd = e.ln_rstd;
   rp.has_xhat = e.ln_xhat ? 1 : 0;
   rp.colsum_out = (C::CS_BYTES > 0 && g.N * 4 <= C::CS_BYTES) ? e.colsum_out : nullptr;
+  rp.dgamma = e.ln_dgamma; rp.dbeta = e.ln_dbeta;
   rp.n_cols = g.N;
   AMC_CHECK_ARG(e.colsum_out == nullptr || rp.colsum_out != nullptr,
                 "gemm_bf16: fused column sums need a bf16-output epilogue and N <= 2048");
@@ -835,6 +1019,13 @@ int gemm_bf16(const GemmArgs& g, cudaStream_t st) {
                       (!e.D16 || (al16(e.D16) && e.ldd16 % 8 == 0)) && (!e.D32 || (al16(e.D32) && e.ldd32 % 4 == 0)) &&
                       (!e.res32 || (al16(e.res32) && e.ldres % 4 == 0)) &&
                       (!e.mask_src || (al16(e.mask_src) && e.ldmask % 8 == 0)) && (!e.bias || al16(e.bias));
+  if (e.ln_bwd) {
+    AMC_CHECK_ARG(row_ok && e.res32 && e.D16 && e.D32 && e.ln_xhat && e.ln_rstd && e.ln_gamma && !e.bias && !e.relu &&
+                      !e.mask_src && g.N <= 256 && al16(e.ln_gamma) && al16(e.ln_xhat),
+                  "gemm_bf16: fused LayerNorm-backward epilogue needs N %% 32 == 0, N <= 256, residual, xhat, rstd, "
+                  "gamma, D16 and D32");
+    return launch_row_bn<RE_LNB, 8>(g.N <= 64 ? 64 : (g.N <= 128 ? 128 : 256), g, st);
+  }
   if (e.ln_gamma) {
     AMC_CHECK_ARG(row_ok && e.res32 && e.D16 && e.D32 && !e.mask_src && !e.relu && g.N <= 512 && al16(e.ln_gamma) &&
                       al16(e.ln_beta) && (!e.ln_xhat || al16(e.ln_xhat)),
