@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AMC_ABI_VERSION 9
+#define AMC_ABI_VERSION 10
 
 enum { AMC_KIND_RAWIQ = 0, AMC_KIND_VIT = 1 };
 enum { AMC_F32 = 0, AMC_BF16 = 1 };
@@ -148,6 +148,18 @@ int amc_model_bwd_ex(const AmcDesc* desc, const float* src, const float* params,
                      float* grads, float* dsrc,
                      int stage_begin, int stage_end, amc_stream_t stream);
 
+/* Attention maps of the whole path: R/models/encoder.py:86-117 / V/models/encoder.py:34-53 with the `score` of every
+ * ScaleDotProductAttention kept (R/models/layers/scale_dot_product_attention.py:26-39).  Dropout off.  desc->training
+ * must be 1 and desc->p_drop 0: the training-mode workspace (amc_model_workspace) keeps every layer's qkv.  Every layer
+ * runs on all token rows and the classifier head does not run.
+ *   layer_mask  bit l -> write layer l's probabilities (bits >= n_layers are an error)
+ *   probs       fp32 [popcount(layer_mask), B, h, T, T] in increasing layer order, or NULL
+ *   rollout     fp32 [B, T], or NULL: attention rollout u^T A_{L-1} ... A_0 with A_l = 0.5 mean_h P_l + 0.5 I and
+ *               u = e_0 (CLS pooling) or 1/T per token (mean pooling)
+ * An empty mask with no rollout is an error. */
+int amc_model_attention(const AmcDesc* desc, const float* src, const float* params, const float* pos,
+                        void* workspace, uint32_t layer_mask, float* probs, float* rollout, amc_stream_t stream);
+
 /* nn.CrossEntropyLoss(label_smoothing) + argmax statistics (R/training/train.py:260,274-277,504).
  *   stats[0] += sum of per-frame losses * loss_scale, stats[1] += #correct (fp32 accumulators)
  *   dlogits = (softmax - smoothed one-hot) * grad_scale   (grad_scale = 1/global_batch)
@@ -260,6 +272,15 @@ int amc_attention_fwd(int dtype, int B, int T, int h, int dh, const void* qkv, v
                       amc_stream_t stream);
 int amc_attention_bwd(int dtype, int B, int T, int h, int dh, const void* qkv, const void* out, const float* lse,
                       const void* dout, void* dqkv, float* dbias, amc_stream_t stream);
+/* The attention probabilities of the above, which the fused kernels never write: probs[b, hh, i, j] =
+ * softmax_j(q_i . k_j / sqrt(dh)), fp32 [B, h, T, T] (scale_dot_product_attention.py:26-39, the returned `score`).
+ * Every (T, dh) amc_attention_fwd takes; the row statistics are recomputed from q and k (no lse needed). */
+int amc_attention_probs(int dtype, int B, int T, int h, int dh, const void* qkv, float* probs, amc_stream_t stream);
+/* One attention-rollout step without writing P (Abnar & Zuidema 2020, the residual-averaged form):
+ *   v_out[b, j] = 0.5 v_in[b, j] + (0.5 / h) sum_hh sum_i v_in[b, i] P[b, hh, i, j]
+ * v_in, v_out fp32 [B, T] (distinct buffers).  Rows with v_in = 0 cost nothing; deterministic (no atomics). */
+int amc_attention_rollout_step(int dtype, int B, int T, int h, int dh, const void* qkv, const float* v_in, float* v_out,
+                               amc_stream_t stream);
 
 /* The same attention restricted to query row 0 of every frame, bf16, head dim 16 / 32 / 64: what the TOP encoder layer
  * of a CLS-pooled model needs, since only `x[:, 0]` feeds the classifier head (R/models/transformer_rawIQ.py:88-90,

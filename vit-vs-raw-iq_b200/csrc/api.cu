@@ -318,10 +318,11 @@ struct Model {
   bool fuse_ln() const { return sizeof(E) == 2 && m.d % 32 == 0 && m.d <= 256; }
   int xi(int l) const { return D.training ? l : (l & 1); }
 
-  int pack_weights() {
+  // bf16 copy of the blob; with `dgrad_operands` also the transposed weights the backward's dgrad GEMMs read
+  int pack_weights(bool dgrad_operands) {
     if (sizeof(E) != 2) return 0;
     AMC_PROF("pack_weights", 0.0, (double)L.total * 6, cast_blob(L.total, params, w.w16, st));
-    if (!D.training) return 0;
+    if (!dgrad_operands) return 0;
     const int64_t d = m.d, F = m.F;
     TransposeBatch tb;
     tb.n = 0;
@@ -422,14 +423,19 @@ struct Model {
   // (T <= 16 stays on the warp-per-(frame, head) tensor-core kernel, which is already at its HBM floor there)
   bool cls_attn() const { return sizeof(E) == 2 && m.T > 16 && attn_cls_supported(m.T, m.h, m.dh) && (m.d % 8) == 0; }
 
+  int qkv_fwd(int l) {
+    const int d = m.d;
+    GemmArgs g;
+    g.M = (int)m.M; g.N = 3 * d; g.K = d; g.A = w.x16[xi(l)]; g.lda = d; g.B = WL(l, L.wq); g.ldb = d;
+    g.name = "gemm_qkv";
+    g.epi.bias = PL(l, L.bq); g.epi.D16 = LB(l).qkv; g.epi.ldd16 = 3 * d;
+    return gemm<E>(g, st);
+  }
+
   int attn_fwd_part(int l, bool cls_only = false) {
     const int M = (int)m.M, d = m.d;
     const LayerBuf& b = LB(l);
-    GemmArgs g;
-    g.M = M; g.N = 3 * d; g.K = d; g.A = w.x16[xi(l)]; g.lda = d; g.B = WL(l, L.wq); g.ldb = d;
-    g.name = "gemm_qkv";
-    g.epi.bias = PL(l, L.bq); g.epi.D16 = b.qkv; g.epi.ldd16 = 3 * d;
-    AMC_TRY(gemm<E>(g, st));
+    AMC_TRY(qkv_fwd(l));
     if (cls_only && cls_attn()) {
       ProfScope ps("attn_cls_fwd", st, 4.0 * m.M * d, (double)M * 2 * d * sizeof(E));
       AMC_TRY(attn_cls_fwd(m.B, m.T, m.h, m.dh, (const bf16*)b.qkv, (bf16*)b.o, st));
@@ -497,7 +503,7 @@ struct Model {
 
   int forward(const float* src, const float* pos, float* logits, float* enc_out) {
     if (m.B == 0) return 0;
-    AMC_TRY(pack_weights());
+    AMC_TRY(pack_weights(D.training));
     AMC_TRY(frontend(src, pos));
     // Only the CLS rows of the top layer reach the head (transformer_rawIQ.py:88-90, amc_transformer.py:29): when
     // just the logits are wanted, the top layer's out-proj / FFN / LayerNorms run on those B rows alone.
@@ -511,6 +517,43 @@ struct Model {
       AMC_PROF("head", 0.0, 0.0, head_fwd(m.B, headT, m.d, m.C, m.has_cls, D.head_ln, D.head_ln_eps, xL,
                        D.head_ln ? P(L.head_ln_w) : nullptr, D.head_ln ? P(L.head_ln_b) : nullptr, P(L.head_w),
                        P(L.head_b), logits, w.hl, w.hxhat, w.hrstd, st));
+    return 0;
+  }
+
+  // Attention maps (amc_model_attention): every layer below the top on all rows, and of the top layer only its QKV
+  // projection on all rows (no CLS-row top layer: its maps need every row; nothing reads its attention output, FFN or
+  // norms), then the probabilities of the masked layers and the rollout from layer L-1 down to 0.  No backward follows,
+  // so the transposed dgrad weights are not packed.  The training-mode carve keeps every
+  // layer's qkv; the rollout ping-pongs between `rollout` and w.u32 ([M, d] fp32, dead once the forward is done), started
+  // so that the last step lands in `rollout`.
+  int attention(const float* src, const float* pos, uint32_t mask, float* probs, float* rollout) {
+    AMC_CHECK_ARG(D.training == 1 && D.p_drop == 0.f, "amc_model_attention needs desc.training=1 and desc.p_drop=0");
+    AMC_CHECK_ARG(mask != 0 || rollout, "amc_model_attention: empty layer_mask and no rollout");
+    AMC_CHECK_ARG(m.L >= 32 || (mask >> m.L) == 0, "amc_model_attention: layer_mask 0x%x names a layer >= n_layers (%d)",
+                  mask, m.L);
+    AMC_CHECK_ARG(mask == 0 || probs, "amc_model_attention: probs is NULL");
+    if (m.B == 0) return 0;
+    AMC_TRY(pack_weights(false));
+    AMC_TRY(frontend(src, pos));
+    for (int l = 0; l + 1 < m.L; ++l) AMC_TRY(layer_fwd(l, false));
+    if (m.L >= 1) AMC_TRY(qkv_fwd(m.L - 1));
+    const size_t per = (size_t)m.B * m.h * m.T * m.T;
+    const double s_flops = 2.0 * m.M * m.T * m.d, qk_bytes = (double)m.M * 2 * m.d * sizeof(E);
+    float* out = probs;
+    for (int l = 0; l < m.L && l < 32; ++l) {
+      if (!((mask >> l) & 1u)) continue;
+      AMC_PROF("attn_probs", s_flops, qk_bytes + 4.0 * per,
+               attention_probs<E>(m.B, m.T, m.h, m.dh, (const E*)LB(l).qkv, out, st));
+      out += per;
+    }
+    if (rollout) {
+      float* v[2] = {rollout, w.u32};
+      int cur = m.L & 1;
+      AMC_PROF("attn_rollout", 0.0, (double)m.M * 4, rollout_init(m.B, m.T, m.has_cls, v[cur], st));
+      for (int l = m.L - 1; l >= 0; --l, cur ^= 1)
+        AMC_PROF("attn_rollout", 2.0 * s_flops, qk_bytes + (double)m.M * 8,
+                 attention_rollout_step<E>(m.B, m.T, m.h, m.dh, (const E*)LB(l).qkv, v[cur], v[cur ^ 1], st));
+    }
     return 0;
   }
 
@@ -815,6 +858,22 @@ int amc_model_bwd_ex(const AmcDesc* desc, const float* src, const float* params,
   return mdl.backward(dlogits, denc_out, grads, dsrc, stage_begin, stage_end);
 }
 
+int amc_model_attention(const AmcDesc* desc, const float* src, const float* params, const float* pos, void* workspace,
+                        uint32_t layer_mask, float* probs, float* rollout, amc_stream_t stream) {
+  DeviceGuard dev_guard(params);
+  AMC_CHECK_ARG(desc && params && pos, "NULL argument");
+  AMC_CHECK_ARG(src || desc->B == 0, "src is NULL");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (desc->dtype == AMC_BF16) {
+    Model<bf16> mdl(*desc, params, st);
+    AMC_TRY(mdl.init(workspace));
+    return mdl.attention(src, pos, layer_mask, probs, rollout);
+  }
+  Model<float> mdl(*desc, params, st);
+  AMC_TRY(mdl.init(workspace));
+  return mdl.attention(src, pos, layer_mask, probs, rollout);
+}
+
 int amc_model_bwd(const AmcDesc* desc, const float* src, const float* params, void* workspace, const float* dlogits,
                   const float* denc_out, float* grads, int stage_begin, int stage_end, amc_stream_t stream) {
   AMC_CHECK_ARG(grads, "NULL argument");
@@ -929,6 +988,23 @@ int amc_attention_fwd(int dtype, int B, int T, int h, int dh, const void* qkv, v
   if (dtype == AMC_BF16)
     return attention_fwd<bf16>(B, T, h, dh, (const bf16*)qkv, (bf16*)out, lse, (cudaStream_t)stream);
   return attention_fwd<float>(B, T, h, dh, (const float*)qkv, (float*)out, lse, (cudaStream_t)stream);
+}
+int amc_attention_probs(int dtype, int B, int T, int h, int dh, const void* qkv, float* probs, amc_stream_t stream) {
+  DeviceGuard dev_guard(qkv);
+  AMC_CHECK_ARG(qkv && probs, "NULL argument");
+  if (dtype == AMC_BF16) return attention_probs<bf16>(B, T, h, dh, (const bf16*)qkv, probs, (cudaStream_t)stream);
+  AMC_CHECK_ARG(dtype == AMC_F32, "unknown dtype %d", dtype);
+  return attention_probs<float>(B, T, h, dh, (const float*)qkv, probs, (cudaStream_t)stream);
+}
+int amc_attention_rollout_step(int dtype, int B, int T, int h, int dh, const void* qkv, const float* v_in, float* v_out,
+                               amc_stream_t stream) {
+  DeviceGuard dev_guard(qkv);
+  AMC_CHECK_ARG(qkv && v_in && v_out, "NULL argument");
+  AMC_CHECK_ARG(v_in != v_out, "attention_rollout_step: v_in and v_out must be distinct buffers");
+  if (dtype == AMC_BF16)
+    return attention_rollout_step<bf16>(B, T, h, dh, (const bf16*)qkv, v_in, v_out, (cudaStream_t)stream);
+  AMC_CHECK_ARG(dtype == AMC_F32, "unknown dtype %d", dtype);
+  return attention_rollout_step<float>(B, T, h, dh, (const float*)qkv, v_in, v_out, (cudaStream_t)stream);
 }
 int amc_attention_cls_fwd(int B, int T, int h, int dh, const void* qkv, void* out, amc_stream_t stream) {
   DeviceGuard dev_guard(qkv);

@@ -41,4 +41,13 @@ int attn_long_bwd(int B, int T, int h, int dh, const E* qkv, const E* out, const
 bool attn_cls_supported(int T, int h, int dh);
 int attn_cls_fwd(int B, int T, int h, int dh, const bf16* qkv, bf16* out, cudaStream_t st);
 int attn_cls_bwd(int B, int T, int h, int dh, const bf16* qkv, const bf16* dO, bf16* dqkv, float* dbias, cudaStream_t st);
+
+// attn_maps.cu: attention probabilities fp32 [B, h, T, T] and one rollout step v_out = v_in^T (0.5 mean_h P + 0.5 I),
+// v fp32 [B, T], for every (T, dh) attention_fwd takes; neither needs the forward's lse
+template <typename E>
+int attention_probs(int B, int T, int h, int dh, const E* qkv, float* probs, cudaStream_t st);
+template <typename E>
+int attention_rollout_step(int B, int T, int h, int dh, const E* qkv, const float* v_in, float* v_out, cudaStream_t st);
+// v = e_0 per frame (CLS pooling) or 1/T (mean pooling)
+int rollout_init(int B, int T, int has_cls, float* v, cudaStream_t st);
 }  // namespace amc

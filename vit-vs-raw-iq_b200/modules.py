@@ -15,9 +15,11 @@ lets w_q / w_k / w_v stay three ``state_dict`` tensors while the kernel reads on
 from __future__ import annotations
 
 import ctypes as C
+import operator
 import os
 from typing import List, Optional, Tuple
 
+import numpy as np
 import torch
 from torch import nn
 
@@ -364,6 +366,74 @@ class _AMCBase(nn.Module):
         if not self._core.is_flat():
             self._core.flatten()
         return self._core.flat
+
+    @torch.no_grad()
+    def _attention(self, src, mask: int, want_rollout: bool):
+        core = self._core
+        # training=1 keeps every layer's qkv in the workspace; module_training=False turns dropout off
+        desc = core.make_desc(src, training=True, module_training=False)
+        dev = src.device
+        T, h = core.layout.T, core.fields["h"]
+        ws = torch.empty(_lib.workspace_bytes(desc), dtype=torch.uint8, device=dev)
+        probs = torch.empty((bin(mask).count("1"), desc.B, h, T, T), dtype=torch.float32, device=dev) if mask else None
+        roll = torch.empty((desc.B, T), dtype=torch.float32, device=dev) if want_rollout else None
+        _lib.check(_lib.lib.amc_model_attention(C.byref(desc), src.data_ptr(), core.flat.data_ptr(),
+                                                core.pos_buffer().data_ptr(), ws.data_ptr(), mask, _lib.ptr(probs),
+                                                _lib.ptr(roll), torch.cuda.current_stream(dev).cuda_stream),
+                   "amc_model_attention")
+        return probs, roll
+
+    def attention_maps(self, src, layers=None) -> List[torch.Tensor]:
+        """The attention probabilities softmax(q k^T / sqrt(d_head)) of the requested encoder layers: the ``score`` that
+        the reference's ``ScaleDotProductAttention`` returns (R/models/layers/scale_dot_product_attention.py:26-39).
+
+        ``src`` is what ``forward`` takes (either input layout, see ``set_raw_input``).  ``layers`` is a sequence of
+        layer indices in ``[0, n_layers)`` (any integer type), or ``None`` for all of them.  Returns one fp32
+        tensor ``[B, n_head, T, T]`` per requested layer, in the order requested (a repeated layer is a separate copy); T counts the CLS token when the model has one.
+
+        Runs under ``torch.no_grad()`` with dropout off whatever ``self.training`` is, in the model's compute dtype.
+        The maps take ``4 B h T^2`` bytes per layer (3.3 GB for all 6 layers at B = 1024, T = 129, h = 8)."""
+        n = self._core.n_layers
+        idx = []
+        for l in (range(n) if layers is None else layers):
+            try:
+                i = operator.index(l)             # any integer type (int, numpy / torch integer scalars), not bool
+            except TypeError:
+                i = None
+            if isinstance(l, (bool, np.bool_)) or i is None or not 0 <= i < min(n, 32):
+                raise ValueError(f"layers must hold encoder layer indices in [0, {min(n, 32)}), got {l!r}")
+            idx.append(i)
+        if not idx:
+            raise ValueError("layers is empty")
+        uniq = sorted(set(idx))
+        probs, _ = self._attention(src, sum(1 << l for l in uniq), False)
+        # a layer asked for twice comes back as two tensors that do not share storage
+        seen = set()
+        out = []
+        for l in idx:
+            t = probs[uniq.index(l)]
+            out.append(t.clone() if l in seen else t)
+            seen.add(l)
+        return out
+
+    def attention_rollout(self, src) -> torch.Tensor:
+        """Attention rollout (Abnar & Zuidema, 2020) of the whole encoder: ``u^T A_{L-1} ... A_0`` with
+        ``A_l = 0.5 * mean_heads(P_l) + 0.5 * I`` (the residual path counted as half of each layer), and ``u`` the head's
+        read-out of the top layer: the CLS row (``e_0``) or, for mean pooling, ``1/T`` on every token.  Returns fp32
+        ``[B, T]``; every row is non-negative and sums to 1.  Computed on the device without materialising any ``P``.
+
+        Columns (S = segment_size, p = patch_size):
+          * column 0 is the CLS token (when the model has one);
+          * raw-IQ ``embedding_type='segment'``: column t >= 1 covers samples ``[(t-1)*S, t*S)`` of both I and Q;
+          * raw-IQ ``embedding_type='conv1d'``: column t >= 1 is sample t - 1;
+          * ViT: column t >= 1 is patch ``divmod(t-1, 64 // p)`` (patch row, patch column) of the ``[1, 32, 64]`` image,
+            whose rows 0-15 hold I and rows 16-31 hold Q;
+          * without a CLS token (mean pooling): column t is token t (the same segment / sample without the shift).
+
+        ``src`` is what ``forward`` takes (either input layout).  Runs under ``torch.no_grad()`` with dropout off
+        whatever ``self.training`` is, in the model's compute dtype."""
+        _, roll = self._attention(src, 0, True)
+        return roll
 
     def _run(self, src, want_logits):
         # grad mode is switched off inside Function.forward, so decide here whether to keep activations
