@@ -25,6 +25,34 @@ U = 2.0 ** -24          # unit roundoff of fp32
 C_ACC = 4.0             # slack on the classical gamma_n = n*u bound (tensor-core adders, atomics, fused adds)
 
 
+def check(what, got, ref, bound, quiet=False):
+    """|got - ref| <= bound element by element (a zero bound demands exact equality).  numpy arrays or torch tensors;
+    tensors are compared in float64 on the device of ``ref``.  Prints (unless ``quiet``) and returns the worst
+    err/bound over the elements with a positive bound."""
+    import torch
+
+    def f64(x, device=None):        # numpy arrays and Python scalars go through float64 without an fp32 rounding
+        if isinstance(x, torch.Tensor):
+            return x.to(device or x.device, torch.float64)
+        return torch.from_numpy(np.array(x, dtype=np.float64)).to(device or "cpu")
+
+    ref = f64(ref)
+    got = f64(got, ref.device)
+    bound = f64(bound, ref.device).expand(ref.shape)
+    assert got.shape == ref.shape, (what, tuple(got.shape), tuple(ref.shape))
+    err = (got - ref).abs()
+    bad = ~(err <= bound)
+    pos = bound > 0
+    worst = float((err[pos] / bound[pos]).max()) if bool(pos.any()) else 0.0
+    if not quiet:
+        print(f"  {what}: worst err/bound {worst:.3g}")
+    if bool(bad.any()):
+        i = np.unravel_index(int(bad.flatten().nonzero()[0, 0]), tuple(ref.shape))
+        raise AssertionError(f"{what}: {int(bad.sum())} of {ref.numel()} elements out of bound; first at {i}: "
+                             f"got {float(got[i])!r} ref {float(ref[i])!r} bound {float(bound[i])!r}")
+    return worst
+
+
 def bf16_rne(x):
     """float32 -> nearest bfloat16 (ties to even), computed on the float32 bit pattern; returned as float32."""
     a = np.ascontiguousarray(x, dtype=np.float32)

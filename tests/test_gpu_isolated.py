@@ -32,24 +32,6 @@ def cuda(a, dtype=torch.float32):
     return torch.from_numpy(np.ascontiguousarray(a)).to(DEV, dtype)
 
 
-def check(what, got, ref, bound):
-    """|got - ref| <= bound element by element (a zero bound demands exact equality)."""
-    got = np.asarray(got, dtype=np.float64)
-    ref = np.asarray(ref, dtype=np.float64)
-    bound = np.broadcast_to(np.asarray(bound, dtype=np.float64), ref.shape)
-    assert got.shape == ref.shape, (what, got.shape, ref.shape)
-    err = np.abs(got - ref)
-    bad = ~(err <= bound)
-    pos = bound > 0
-    worst = float((err[pos] / bound[pos]).max()) if pos.any() else 0.0
-    print(f"  {what}: worst err/bound {worst:.3g}")
-    if bad.any():
-        i = np.unravel_index(np.argmax(bad), ref.shape)
-        raise AssertionError(f"{what}: {int(bad.sum())} of {ref.size} elements out of bound; first at {i}: "
-                             f"got {got[i]!r} ref {ref[i]!r} bound {bound[i]!r}")
-    return worst
-
-
 # ---------------------------------------------------------------------------------------------------------------------
 # 0-layer models through the C ABI
 # ---------------------------------------------------------------------------------------------------------------------
@@ -169,9 +151,9 @@ def check_frontend_bwd(m, got_blob, dsrc, ref, extra=None):
         if ref[name] is None:
             continue
         b = ref[name + "_bound"] + (extra[name] if extra is not None else 0.0)
-        check(name, m.grad(got_blob, name), ref[name], b)
+        R.check(name, m.grad(got_blob, name), ref[name], b)
     if dsrc is not None:
-        check("dsrc", dsrc, ref["dsrc"], ref["dsrc_bound"])
+        R.check("dsrc", dsrc, ref["dsrc"], ref["dsrc_bound"])
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -214,7 +196,7 @@ def test_frontend_forward_and_backward(case, layout):
     if path == FUSED:
         assert "patchify" not in classes
     ref, A, bound = m.ref()
-    check("x0", x0, ref, bound)
+    R.check("x0", x0, ref, bound)
     G = np.random.default_rng(5).standard_normal(x0.shape).astype(np.float32)
     blob, dsrc = m.backward(denc=G)
     rb = R.frontend_bwd_ref(G, A, m.p, m.cfg, layout, STATS, m.bf16)
@@ -239,7 +221,7 @@ def test_pe_dropout_mask_scale_and_regeneration(dtype, geo, p):
     s = R.keep_scale(p)
     kept = x0 != 0
     # a kept element is the reference times the fp32 scale: one more rounding
-    check("x0 kept", np.where(kept, x0, ref * s), ref * s, (bound + 2 * U * np.abs(ref)) * s)
+    R.check("x0 kept", np.where(kept, x0, ref * s), ref * s, (bound + 2 * U * np.abs(ref)) * s)
     pe = R.p_effective(p)
     frac = kept.mean()
     sigma = np.sqrt(pe * (1 - pe) / kept.size)
@@ -288,15 +270,15 @@ def test_head_forward_and_backward(case):
     x0, logits, classes = m.forward()
     assert "head" in classes
     ref_logits, cache, lb = R.head_ref(x0, m.p, m.cfg, bool(head_ln))
-    check("logits", logits, ref_logits, lb)
+    R.check("logits", logits, ref_logits, lb)
     dl = np.random.default_rng(9).standard_normal((B, Cn)).astype(np.float32)
     blob, _ = m.backward(dlogits=dl)
     hb = R.head_bwd_ref(dl, cache)
-    check("head_w", m.grad(blob, "head_w"), hb["head_w"], hb["head_w_bound"])
-    check("head_b", m.grad(blob, "head_b"), hb["head_b"], hb["head_b_bound"])
+    R.check("head_w", m.grad(blob, "head_w"), hb["head_w"], hb["head_w_bound"])
+    R.check("head_b", m.grad(blob, "head_b"), hb["head_b"], hb["head_b_bound"])
     if head_ln:
-        check("mlp_head.0.weight", m.grad(blob, "ln_w"), hb["ln_w"], hb["ln_w_bound"])
-        check("mlp_head.0.bias", m.grad(blob, "ln_b"), hb["ln_b"], hb["ln_b_bound"])
+        R.check("mlp_head.0.weight", m.grad(blob, "ln_w"), hb["ln_w"], hb["ln_w_bound"])
+        R.check("mlp_head.0.bias", m.grad(blob, "ln_b"), hb["ln_b"], hb["ln_b_bound"])
     # dx0 reaches the embedding gradients (fp32: no rounding of demb); its bound propagates linearly
     _, A, _ = m.ref()
     rb = R.frontend_bwd_ref(hb["dx0"], A, m.p, m.cfg)
@@ -348,15 +330,15 @@ def test_ce_loss(ls, Cn, B):
     gs, lsc = 1.0 / 3.0, 0.25
     loss, dl, e_loss, e_dl = ce_bounds(z, labels, ls, gs)
     got_dl, st = ce_call(z, labels, ls, gs, lsc)
-    check("dlogits", got_dl, dl * gs, e_dl)
+    R.check("dlogits", got_dl, dl * gs, e_dl)
     # stats[0] += sum_b loss_b * loss_scale: B terms through warp sums and one fp32 atomic per warp
-    check("stats[0]", st[0], loss.sum() * lsc, lsc * (e_loss.sum() + R.C_ACC * (B + 1) * U * np.abs(loss).sum()))
+    R.check("stats[0]", st[0], loss.sum() * lsc, lsc * (e_loss.sum() + R.C_ACC * (B + 1) * U * np.abs(loss).sum()))
     assert st[1] == (R.argmax_ref(z) == labels).sum()
     # NULL outputs: each of the two may be left out
     got_dl2, _ = ce_call(z, labels, ls, gs, lsc, want_stats=False)
     assert np.array_equal(got_dl2, got_dl)
     _, st2 = ce_call(z, labels, ls, gs, lsc, want_dl=False)
-    check("stats[0] without dlogits", st2[0], loss.sum() * lsc,
+    R.check("stats[0] without dlogits", st2[0], loss.sum() * lsc,
           lsc * (e_loss.sum() + R.C_ACC * (B + 1) * U * np.abs(loss).sum()))
     assert st2[1] == st[1]
 
@@ -373,7 +355,7 @@ def test_ce_loss_out_of_range_label_poisons_only_the_loss():
     assert np.isnan(st[0])
     ok = (labels >= 0) & (labels < Cn)
     assert st[1] == ((R.argmax_ref(z) == labels) & ok).sum()
-    check("dlogits (bad rows: all-smoothing target)", got_dl, dl, e_dl)
+    R.check("dlogits (bad rows: all-smoothing target)", got_dl, dl, e_dl)
 
 
 @pytest.mark.parametrize("B", [1, 127, 129, 1000])
@@ -422,11 +404,11 @@ def check_adam(tag, got, state, step, wd, max_norm, gs, ws):
     rp, rm, rv, norm = R.adamw_ref(p, g, m, v, step, HP["lr"], HP["beta1"], HP["beta2"], HP["eps"], wd, max_norm, gs)
     ep, em, ev, e_norm = R.adamw_bound(p, g, m, v, step, HP["lr"], HP["beta1"], HP["beta2"], HP["eps"], wd, max_norm, gs,
                                        n_chain(n))
-    check(f"{tag} exp_avg", got[2], rm, em)
-    check(f"{tag} exp_avg_sq", got[3], rv, ev)
-    check(f"{tag} param", got[0], rp, ep)
+    R.check(f"{tag} exp_avg", got[2], rm, em)
+    R.check(f"{tag} exp_avg_sq", got[3], rv, ev)
+    R.check(f"{tag} param", got[0], rp, ep)
     if max_norm > 0:
-        check(f"{tag} norm_ws[1]", ws[1], norm, norm * e_norm)
+        R.check(f"{tag} norm_ws[1]", ws[1], norm, norm * e_norm)
     else:                               # clipping disabled: the scratch is neither read nor written
         assert np.isnan(ws).all()
 
@@ -516,10 +498,10 @@ def test_iq_stats_sums(shape, mean, std):
     ref, bound = R.iq_stats_ref(x)
     rc, acc = iq_call(x)
     assert rc == 0
-    check("sums", acc.cpu().numpy(), ref, bound)
+    R.check("sums", acc.cpu().numpy(), ref, bound)
     rc, acc = iq_call(x, acc)                    # a second call accumulates
     assert rc == 0
-    check("sums after two calls", acc.cpu().numpy(), 2 * ref, 2 * bound + 2 * U * U * np.abs(ref))
+    R.check("sums after two calls", acc.cpu().numpy(), 2 * ref, 2 * bound + 2 * U * U * np.abs(ref))
     if mean == 1e3:                              # the unbiased std survives the cancellation
         s = acc.cpu().numpy() / 2
         n = x.size // 2
@@ -532,7 +514,7 @@ def test_iq_stats_alignment():
     ref, bound = R.iq_stats_ref(x)
     rc, acc = iq_call(x, offset_floats=2)        # 8-byte but not 16-byte aligned
     assert rc == 0
-    check("sums (8-byte aligned)", acc.cpu().numpy(), ref, bound)
+    R.check("sums (8-byte aligned)", acc.cpu().numpy(), ref, bound)
     rc, _ = iq_call(x, offset_floats=1)          # 4-byte aligned: refused
     assert rc < 0 and b"aligned" in _lib.lib.amc_last_error()
 
@@ -556,7 +538,7 @@ def test_gemm_generic_epilogue(M, N, K, lda, ldd16, ldd32):
     ref = a @ Bm.T.astype(np.float64) + bias
     bound = R.C_ACC * (K + 1) * U * (np.abs(a) @ np.abs(Bm.T.astype(np.float64)) + np.abs(bias))
     d32 = D32.cpu().numpy()
-    check("D32", d32[:, :N], ref, bound)
+    R.check("D32", d32[:, :N], ref, bound)
     assert (d32[:, N:] == 7.0).all()                      # the row padding is not written
     if D16 is not None:
         d16 = D16.float().cpu().numpy()

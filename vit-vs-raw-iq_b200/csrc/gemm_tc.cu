@@ -471,6 +471,10 @@ gemm_tc_row_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
       }
     };
     auto issue_next = [&](int t, int k, uint32_t gi) {   // slab after (t, k), once every lane has read the buffer
+      // The TMA write (async proxy) must not overtake this lane's shared loads of the slab (generic proxy): they are
+      // issued just above and their values are not consumed yet.  Without the fence, a small L2-hit xhat load could
+      // land first and pass B would read the next chunk's xhat (wrong du in one 16-byte chunk of two adjacent rows).
+      fence_proxy_async();
       __syncwarp();
       if (lane != 0) return;
       if (++k == 2 * nmine) { t += gridDim.x; k = 0; }
