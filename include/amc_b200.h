@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AMC_ABI_VERSION 10
+#define AMC_ABI_VERSION 11
 
 enum { AMC_KIND_RAWIQ = 0, AMC_KIND_VIT = 1 };
 enum { AMC_F32 = 0, AMC_BF16 = 1 };
@@ -160,6 +160,24 @@ int amc_model_bwd_ex(const AmcDesc* desc, const float* src, const float* params,
 int amc_model_attention(const AmcDesc* desc, const float* src, const float* params, const float* pos,
                         void* workspace, uint32_t layer_mask, float* probs, float* rollout, amc_stream_t stream);
 
+/* Class-specific attention relevance, the gradient-weighted rollout of Chefer, Gur & Wolf, "Generic Attention-model
+ * Explainability" (ICCV 2021), for the model of R/models/transformer_rawIQ.py:72-98 / V/models/amc_transformer.py:26-31
+ * with dropout off.  desc->training must be 1 and desc->p_drop 0; the workspace is the training-mode one
+ * (amc_model_workspace), which is all the call needs besides its outputs.
+ *   target     device int64 [B], or NULL: t_b = the first maximum of logits[b] (amc_argmax's rule, same forward)
+ *   logits     fp32 [B, C] out: the forward's logits (the top layer of a CLS model runs on its CLS rows, as in
+ *              amc_model_fwd)
+ *   relevance  fp32 [B, T] out: r = u^T (I + A_{L-1}) ... (I + A_0) with
+ *                A_l = mean_h relu(dy_t/dP_l,h * P_l,h),  dy_t/dP_l,h = dO_l,h V_l,h^T,
+ *              y_t the logit of class t_b (not the loss, not the softmax), dO_l the gradient of y_t w.r.t. the
+ *              head-concatenated attention output of layer l (before w_concat), and u = e_0 (CLS pooling) or 1/T on
+ *              every token (mean pooling).  Every entry is >= 0 and r >= u, so r[:, 0] >= 1 for CLS models; rows are
+ *              not normalised.  Columns as for amc_model_attention's rollout.
+ * A target outside [0, C) makes that frame's relevance row NaN (the amc_ce_loss convention).  The backward is the
+ * frozen one of amc_model_bwd_ex with grads = NULL and no dsrc; it stops after layer 0's out-projection gradient. */
+int amc_model_relevance(const AmcDesc* desc, const float* src, const float* params, const float* pos, void* workspace,
+                        const int64_t* target, float* logits, float* relevance, amc_stream_t stream);
+
 /* nn.CrossEntropyLoss(label_smoothing) + argmax statistics (R/training/train.py:260,274-277,504).
  *   stats[0] += sum of per-frame losses * loss_scale, stats[1] += #correct (fp32 accumulators)
  *   dlogits = (softmax - smoothed one-hot) * grad_scale   (grad_scale = 1/global_batch)
@@ -281,6 +299,14 @@ int amc_attention_probs(int dtype, int B, int T, int h, int dh, const void* qkv,
  * v_in, v_out fp32 [B, T] (distinct buffers).  Rows with v_in = 0 cost nothing; deterministic (no atomics). */
 int amc_attention_rollout_step(int dtype, int B, int T, int h, int dh, const void* qkv, const float* v_in, float* v_out,
                                amc_stream_t stream);
+/* One class-specific relevance step (amc_model_relevance) without writing P or dP:
+ *   v_out[b, j] = v_in[b, j] + (1 / h) sum_hh sum_i v_in[b, i] relu(dP[b, hh, i, j] P[b, hh, i, j]),
+ *   dP[b, hh] = dO_hh V_hh^T
+ * dout is [B*T, d] in dtype, heads concatenated like `out` of amc_attention_fwd: the gradient of the attention output
+ * (multi_head_attention.py:41-47, before w_concat).  Rows i with v_in[b, i] = 0 are never read, so they may hold
+ * anything, NaN included.  v_in, v_out fp32 [B, T], distinct buffers; deterministic (no atomics). */
+int amc_attention_relevance_step(int dtype, int B, int T, int h, int dh, const void* qkv, const void* dout,
+                                 const float* v_in, float* v_out, amc_stream_t stream);
 
 /* The same attention restricted to query row 0 of every frame, bf16, head dim 16 / 32 / 64: what the TOP encoder layer
  * of a CLS-pooled model needs, since only `x[:, 0]` feeds the classifier head (R/models/transformer_rawIQ.py:88-90,

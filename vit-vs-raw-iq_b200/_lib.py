@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libamc_b200.so")
 
-ABI_VERSION = 10
+ABI_VERSION = 11
 KIND_RAWIQ, KIND_VIT = 0, 1
 F32, BF16 = 0, 1
 INPUT_MODEL, INPUT_RAW = 0, 1
@@ -62,6 +62,7 @@ def _load():
         "amc_model_bwd": [C.POINTER(AmcDesc), vp, vp, vp, vp, vp, vp, i32, i32, vp],
         "amc_model_bwd_ex": [C.POINTER(AmcDesc), vp, vp, vp, vp, vp, vp, vp, i32, i32, vp],
         "amc_model_attention": [C.POINTER(AmcDesc), vp, vp, vp, vp, C.c_uint32, vp, vp, vp],
+        "amc_model_relevance": [C.POINTER(AmcDesc), vp, vp, vp, vp, vp, vp, vp, vp],
         "amc_ce_loss": [i32, i32, vp, vp, f32, f32, f32, vp, vp, vp],
         "amc_argmax": [i32, i32, vp, vp, vp],
         "amc_zero": [vp, C.c_size_t, vp],
@@ -78,6 +79,7 @@ def _load():
         "amc_attention_bwd": [i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp],
         "amc_attention_probs": [i32, i32, i32, i32, i32, vp, vp, vp],
         "amc_attention_rollout_step": [i32, i32, i32, i32, i32, vp, vp, vp, vp],
+        "amc_attention_relevance_step": [i32, i32, i32, i32, i32, vp, vp, vp, vp, vp],
         "amc_attention_cls_fwd": [i32, i32, i32, i32, vp, vp, vp],
         "amc_attention_cls_bwd": [i32, i32, i32, i32, vp, vp, vp, vp, vp],
         "amc_layernorm_fwd": [i32, i32, i32, vp, vp, vp, f32, vp, vp, vp, vp, vp],

@@ -557,6 +557,39 @@ struct Model {
     return 0;
   }
 
+  // Class-specific relevance (amc_model_relevance): the forward of forward() with logits, the one-hot dlogits of the
+  // target (or argmax) class, then the frozen backward (grads = NULL) from the head down, with one relevance step on each
+  // layer's attention-output gradient dO_l as layer_bwd_out leaves it.  Layer 0's attention backward, dgrad QKV and the
+  // front end would only feed layers below it, so they do not run.  The vector ping-pongs between `relevance` and w.u32,
+  // and the one-hot dlogits sit in w.u32 behind it: w.u32 ([M, d] fp32) is forward scratch that no backward kernel
+  // writes (post_bwd_part, layer_bwd_attn and the head backward use dy32 / dw32 / t32 / du32 and their CLS-view copies).
+  int relevance(const float* src, const float* pos, const int64_t* target, float* logits, float* relevance) {
+    AMC_CHECK_ARG(D.training == 1 && D.p_drop == 0.f, "amc_model_relevance needs desc.training=1 and desc.p_drop=0");
+    AMC_CHECK_ARG(logits && relevance, "amc_model_relevance: logits or relevance is NULL");
+    AMC_CHECK_ARG(m.L >= 1, "amc_model_relevance: the model has no encoder layer");
+    if (m.B == 0) return 0;
+    const size_t vn = align_up((size_t)m.M, 64);
+    AMC_CHECK_ARG(vn + (size_t)m.B * m.C <= m.M * (size_t)m.d, "amc_model_relevance: scratch too small");
+    AMC_TRY(forward(src, pos, logits, nullptr));
+    float* dlogits = w.u32 + vn;
+    AMC_PROF("relevance", 0.0, 0.0, relevance_seed(m.B, m.C, logits, target, dlogits, st));
+    AMC_TRY(backward(dlogits, nullptr, nullptr, nullptr, 0, 1));   // head
+    const bool cls_top = m.has_cls;                                 // forward() ran with logits: mirrors its choice
+    float* v[2] = {relevance, w.u32};
+    int cur = m.L & 1;
+    AMC_PROF("relevance", 0.0, (double)m.M * 4, rollout_init(m.B, m.T, m.has_cls, v[cur], st));
+    const double s_flops = 2.0 * m.M * m.T * m.d, qkv_bytes = (double)m.M * 3 * m.d * sizeof(E);
+    for (int l = m.L - 1; l >= 0; --l, cur ^= 1) {
+      const bool cls_only = cls_top && l == m.L - 1;
+      AMC_TRY(layer_bwd_out(l, cls_only));
+      AMC_PROF("relevance", 3.0 * s_flops, qkv_bytes + (double)m.M * m.d * sizeof(E) + (double)m.M * 8,
+               attention_relevance_step<E>(m.B, m.T, m.h, m.dh, (const E*)LB(l).qkv, (const E*)w.dO, v[cur],
+                                           v[cur ^ 1], st));
+      if (l > 0) AMC_TRY(layer_bwd_attn(l, cls_only));
+    }
+    return 0;
+  }
+
   // ---- backward ---------------------------------------------------------------------------
   // weight-gradient GEMM: dW[No, Ki] += dY[M, No]^T X[M, Ki]
   // ... and db[No] += column sums of dY: inside the same kernel on the bf16 path, a colsum launch in fp32
@@ -666,16 +699,23 @@ struct Model {
   }
 
   int layer_bwd(int l, bool cls_only) {
+    AMC_TRY(layer_bwd_out(l, cls_only));
+    return layer_bwd_attn(l, cls_only);
+  }
+  // the first half of layer_bwd: leaves the attention-output gradient in w.dO
+  int layer_bwd_out(int l, bool cls_only) {
+    if (cls_only) {
+      // every non-CLS row of the attention-output gradient is exactly zero (the CLS-row kernel never reads them)
+      if (!cls_attn()) AMC_CUDA(cudaMemsetAsync(w.dO, 0, (size_t)m.M * m.d * sizeof(E), st));
+      return post_bwd_part(l, cls_rows_view(l));
+    }
+    return post_bwd_part(l, all_rows(l));
+  }
+  // the second half: attention backward, dgrad QKV and the skip path into the gradient of the layer input
+  int layer_bwd_attn(int l, bool cls_only) {
     const int M = (int)m.M, d = m.d;
     const LayerBuf& b = LB(l);
     const bool cls_kernel = cls_only && cls_attn();
-    if (cls_only) {
-      // every non-CLS row of the attention-output gradient is exactly zero (the CLS-row kernel never reads them)
-      if (!cls_kernel) AMC_CUDA(cudaMemsetAsync(w.dO, 0, (size_t)M * d * sizeof(E), st));
-      AMC_TRY(post_bwd_part(l, cls_rows_view(l)));
-    } else {
-      AMC_TRY(post_bwd_part(l, all_rows(l)));
-    }
     if (cls_kernel) {
       ProfScope ps("attn_cls_bwd", st, 10.0 * m.M * d, (double)M * 5 * d * sizeof(E));
       AMC_TRY(attn_cls_bwd(m.B, m.T, m.h, m.dh, (const bf16*)b.qkv, (const bf16*)w.dO, (bf16*)w.dqkv, GL(l, L.bq), st));
@@ -874,6 +914,22 @@ int amc_model_attention(const AmcDesc* desc, const float* src, const float* para
   return mdl.attention(src, pos, layer_mask, probs, rollout);
 }
 
+int amc_model_relevance(const AmcDesc* desc, const float* src, const float* params, const float* pos, void* workspace,
+                        const int64_t* target, float* logits, float* relevance, amc_stream_t stream) {
+  DeviceGuard dev_guard(params);
+  AMC_CHECK_ARG(desc && params && pos, "NULL argument");
+  AMC_CHECK_ARG(src || desc->B == 0, "src is NULL");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (desc->dtype == AMC_BF16) {
+    Model<bf16> mdl(*desc, params, st);
+    AMC_TRY(mdl.init(workspace));
+    return mdl.relevance(src, pos, target, logits, relevance);
+  }
+  Model<float> mdl(*desc, params, st);
+  AMC_TRY(mdl.init(workspace));
+  return mdl.relevance(src, pos, target, logits, relevance);
+}
+
 int amc_model_bwd(const AmcDesc* desc, const float* src, const float* params, void* workspace, const float* dlogits,
                   const float* denc_out, float* grads, int stage_begin, int stage_end, amc_stream_t stream) {
   AMC_CHECK_ARG(grads, "NULL argument");
@@ -1005,6 +1061,18 @@ int amc_attention_rollout_step(int dtype, int B, int T, int h, int dh, const voi
     return attention_rollout_step<bf16>(B, T, h, dh, (const bf16*)qkv, v_in, v_out, (cudaStream_t)stream);
   AMC_CHECK_ARG(dtype == AMC_F32, "unknown dtype %d", dtype);
   return attention_rollout_step<float>(B, T, h, dh, (const float*)qkv, v_in, v_out, (cudaStream_t)stream);
+}
+int amc_attention_relevance_step(int dtype, int B, int T, int h, int dh, const void* qkv, const void* dout,
+                                 const float* v_in, float* v_out, amc_stream_t stream) {
+  DeviceGuard dev_guard(qkv);
+  AMC_CHECK_ARG(qkv && dout && v_in && v_out, "NULL argument");
+  AMC_CHECK_ARG(v_in != v_out, "attention_relevance_step: v_in and v_out must be distinct buffers");
+  if (dtype == AMC_BF16)
+    return attention_relevance_step<bf16>(B, T, h, dh, (const bf16*)qkv, (const bf16*)dout, v_in, v_out,
+                                          (cudaStream_t)stream);
+  AMC_CHECK_ARG(dtype == AMC_F32, "unknown dtype %d", dtype);
+  return attention_relevance_step<float>(B, T, h, dh, (const float*)qkv, (const float*)dout, v_in, v_out,
+                                         (cudaStream_t)stream);
 }
 int amc_attention_cls_fwd(int B, int T, int h, int dh, const void* qkv, void* out, amc_stream_t stream) {
   DeviceGuard dev_guard(qkv);

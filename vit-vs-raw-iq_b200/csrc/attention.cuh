@@ -48,6 +48,14 @@ template <typename E>
 int attention_probs(int B, int T, int h, int dh, const E* qkv, float* probs, cudaStream_t st);
 template <typename E>
 int attention_rollout_step(int B, int T, int h, int dh, const E* qkv, const float* v_in, float* v_out, cudaStream_t st);
+// one class-specific relevance step v_out = v_in + (1/h) sum_h v_in^T relu((dO V^T) * P_h); dO [B*T, d] is the gradient of
+// the head-concatenated attention output, and its rows whose v_in is 0 are never read
+template <typename E>
+int attention_relevance_step(int B, int T, int h, int dh, const E* qkv, const E* dout, const float* v_in, float* v_out,
+                             cudaStream_t st);
 // v = e_0 per frame (CLS pooling) or 1/T (mean pooling)
 int rollout_init(int B, int T, int has_cls, float* v, cudaStream_t st);
+// dlogits fp32 [B, C] = one_hot(target[b]), or of the first maximum of logits[b] with target NULL; NaN rows for targets
+// outside [0, C)
+int relevance_seed(int B, int C, const float* logits, const int64_t* target, float* dlogits, cudaStream_t st);
 }  // namespace amc

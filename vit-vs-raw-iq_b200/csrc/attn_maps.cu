@@ -16,6 +16,11 @@
 //                        column sums into its own shared-memory row; the CTA (up to 16 warps) then sums the warps in a
 //                        fixed order: no atomics, bit-reproducible.  Tiles whose 16 v_in entries are all zero are
 //                        skipped, so the top layer of a CLS model (v_in = e_0) costs one tile per head.
+//                        With REL, one step of class-specific relevance (Chefer, Gur & Wolf, ICCV 2021):
+//                        v_out = v_in + (1 / h) sum_hh v_in^T relu(dP_hh * P_hh), dP = dO V^T the gradient of the target
+//                        score w.r.t. P.  The tile's dO rows sit next to its Q rows and each V chunk next to its K
+//                        chunk; pass 2 forms dP with the same chunk product as S.  dO rows whose v_in is 0 are zero-filled
+//                        on load, never read: under the CLS-row top layer only row 0 of each frame's dO is written.
 #include "attention.cuh"
 #include "ptx.cuh"
 
@@ -36,23 +41,23 @@ template <typename E, int KD> struct Geo {
   static constexpr size_t k_bytes = (size_t)KC * LDE * sizeof(E);
 };
 
-// dst[r][c] = src[r * ld + c] for r < nvalid, c < dh, zero elsewhere (r < nrows, c < DHP)
+// dst[r][c] = src[r * ld + c] for r < nvalid, c < dh and bit r % 32 of `live` set, zero elsewhere (r < nrows, c < DHP)
 template <typename E, int KD>
 __device__ __forceinline__ void load_rows(E* dst, const E* __restrict__ src, int ld, int nvalid, int nrows, int dh,
-                                          bool vec, int lane) {
+                                          bool vec, int lane, uint32_t live = 0xffffffffu) {
   using G = Geo<E, KD>;
   if (vec) {
     constexpr int CPR = G::DHP / G::VEC;
     for (int i = lane; i < nrows * CPR; i += 32) {
       const int r = i / CPR, c = (i - r * CPR) * G::VEC;
       uint4 v = make_uint4(0u, 0u, 0u, 0u);
-      if (r < nvalid && c < dh) v = __ldg(reinterpret_cast<const uint4*>(src + (size_t)r * ld + c));
+      if (r < nvalid && c < dh && ((live >> (r & 31)) & 1u)) v = __ldg(reinterpret_cast<const uint4*>(src + (size_t)r * ld + c));
       *reinterpret_cast<uint4*>(dst + r * G::LDE + c) = v;
     }
   } else {
     for (int i = lane; i < nrows * G::DHP; i += 32) {
       const int r = i / G::DHP, c = i - r * G::DHP;
-      dst[r * G::LDE + c] = (r < nvalid && c < dh) ? src[(size_t)r * ld + c] : from_f<E>(0.f);
+      dst[r * G::LDE + c] = (r < nvalid && c < dh && ((live >> (r & 31)) & 1u)) ? src[(size_t)r * ld + c] : from_f<E>(0.f);
     }
   }
 }
@@ -269,16 +274,19 @@ __global__ void __launch_bounds__(128) attn_probs_kernel(int T, int h, int dh, i
   }
 }
 
-template <typename E, int KD>
+// per warp: Q rows | K chunk | fp32 column sums [T] | (REL: dO rows | V chunk)
+__host__ __device__ inline size_t rollout_acc_bytes(int T) { return (size_t)(T + 3) / 4 * 4 * 4; }
+template <typename E, int KD, bool REL>
 inline size_t rollout_warp_bytes(int T) {
   using G = Geo<E, KD>;
-  return G::q_bytes + G::k_bytes + (size_t)(T + 3) / 4 * 4 * 4;
+  return (REL ? 2 : 1) * (G::q_bytes + G::k_bytes) + rollout_acc_bytes(T);
 }
 
-template <typename E, int KD>
+template <typename E, int KD, bool REL>
 __global__ void __launch_bounds__(512) attn_rollout_kernel(int T, int h, int dh, const E* __restrict__ qkv,
                                                            const float* __restrict__ v_in, float* __restrict__ v_out,
-                                                           float sl2, size_t warp_bytes, int vec) {
+                                                           float sl2, size_t warp_bytes, int vec,
+                                                           const E* __restrict__ dout) {
   using G = Geo<E, KD>;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int nw = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -286,6 +294,8 @@ __global__ void __launch_bounds__(512) attn_rollout_kernel(int T, int h, int dh,
   E* Qs = reinterpret_cast<E*>(wsm);
   E* Ks = reinterpret_cast<E*>(wsm + G::q_bytes);
   float* colacc = reinterpret_cast<float*>(wsm + G::q_bytes + G::k_bytes);
+  E* dOs = reinterpret_cast<E*>(wsm + G::q_bytes + G::k_bytes + rollout_acc_bytes(T));
+  E* Vs = dOs + 16 * G::LDE;
   const int b = blockIdx.x, d = h * dh, ld = 3 * d;
   const float* vb = v_in + (size_t)b * T;
   for (int j = lane; j < T; j += 32) colacc[j] = 0.f;
@@ -299,6 +309,10 @@ __global__ void __launch_bounds__(512) attn_rollout_kernel(int T, int h, int dh,
     const E* kbase = qkv + (size_t)b * T * ld + d + (size_t)hh * dh;
     __syncwarp();
     load_rows<E, KD>(Qs, qkv + ((size_t)b * T + i0) * ld + (size_t)hh * dh, ld, nrow, 16, dh, vec != 0, lane);
+    if constexpr (REL) {
+      const uint32_t live = __ballot_sync(0xffffffffu, lane < 16 && vr != 0.f);
+      load_rows<E, KD>(dOs, dout + ((size_t)b * T + i0) * d + (size_t)hh * dh, d, nrow, 16, dh, vec != 0, lane, live);
+    }
     __syncwarp();
     uint32_t aq[KD][4];
     load_qfrag<E, KD>(Qs, aq, lane);
@@ -308,15 +322,42 @@ __global__ void __launch_bounds__(512) attn_rollout_kernel(int T, int h, int dh,
     for (int k0 = 0; k0 < T; k0 += KC) {
       __syncwarp();
       load_rows<E, KD>(Ks, kbase + (size_t)k0 * ld, ld, min(KC, T - k0), KC, dh, vec != 0, lane);
+      if constexpr (REL) load_rows<E, KD>(Vs, kbase + d + (size_t)k0 * ld, ld, min(KC, T - k0), KC, dh, vec != 0, lane);
       __syncwarp();
-      float c[8][4];
-      chunk_scores<E, KD>(Qs, Ks, aq, c, lane);
-      scale_mask(c, k0, T, sl2, lane);
       float s[8][2];
+      if constexpr (REL) {
+        // dP first; the dO and Q fragments (bf16) are reloaded from shared memory per chunk, so that no fragment stays
+        // live across chunks and every instantiation fits the 128 registers of a 512-thread CTA without spilling
+        float dp[8][4];
+        {
+          uint32_t ado[KD][4];
+          load_qfrag<E, KD>(dOs, ado, lane);
+          chunk_scores<E, KD>(dOs, Vs, ado, dp, lane);   // unscaled; keys >= T meet zero-filled V rows: dP = 0
+        }
+        float c[8][4];
+        {
+          uint32_t aqc[KD][4];
+          load_qfrag<E, KD>(Qs, aqc, lane);
+          chunk_scores<E, KD>(Qs, Ks, aqc, c, lane);
+        }
+        scale_mask(c, k0, T, sl2, lane);
+        // relu that keeps NaN (fmaxf would drop it): a NaN dO row, which an invalid target's NaN dlogits row produces,
+        // must reach v_out.  Rows with v_in = 0 were zero-filled and keys >= T give 0 * 0, so neither makes a NaN.
+        auto relu = [](float x) { return x < 0.f ? 0.f : x; };
 #pragma unroll
-      for (int n = 0; n < 8; ++n) {
-        s[n][0] = fmaf(w0, ex2(c[n][0] - m0), w1 * ex2(c[n][2] - m1));
-        s[n][1] = fmaf(w0, ex2(c[n][1] - m0), w1 * ex2(c[n][3] - m1));
+        for (int n = 0; n < 8; ++n) {
+          s[n][0] = fmaf(w0, relu(dp[n][0] * ex2(c[n][0] - m0)), w1 * relu(dp[n][2] * ex2(c[n][2] - m1)));
+          s[n][1] = fmaf(w0, relu(dp[n][1] * ex2(c[n][1] - m0)), w1 * relu(dp[n][3] * ex2(c[n][3] - m1)));
+        }
+      } else {
+        float c[8][4];
+        chunk_scores<E, KD>(Qs, Ks, aq, c, lane);
+        scale_mask(c, k0, T, sl2, lane);
+#pragma unroll
+        for (int n = 0; n < 8; ++n) {
+          s[n][0] = fmaf(w0, ex2(c[n][0] - m0), w1 * ex2(c[n][2] - m1));
+          s[n][1] = fmaf(w0, ex2(c[n][1] - m0), w1 * ex2(c[n][3] - m1));
+        }
       }
       // sum over the 8 row pairs (lanes with equal lane % 4), in a fixed order
 #pragma unroll
@@ -338,11 +379,11 @@ __global__ void __launch_bounds__(512) attn_rollout_kernel(int T, int h, int dh,
     }
   }
   __syncthreads();
-  const float hs = 0.5f / (float)h;
+  const float hs = (REL ? 1.f : 0.5f) / (float)h;
   for (int j = threadIdx.x; j < T; j += blockDim.x) {
     float a = 0.f;
     for (int w = 0; w < nw; ++w) a += reinterpret_cast<const float*>(smem_raw + (size_t)w * warp_bytes + G::q_bytes + G::k_bytes)[j];
-    v_out[(size_t)b * T + j] = fmaf(0.5f, vb[j], hs * a);
+    v_out[(size_t)b * T + j] = REL ? fmaf(hs, a, vb[j]) : fmaf(0.5f, vb[j], hs * a);
   }
 }
 
@@ -352,6 +393,17 @@ __global__ void rollout_init_kernel(int B, int T, int has_cls, float* __restrict
   if (i >= (int64_t)B * T) return;
   const int t = (int)(i % T);
   v[i] = has_cls ? (t == 0 ? 1.f : 0.f) : 1.f / (float)T;
+}
+
+// dlogits[b] = one_hot(t_b): t_b = target[b], or with target NULL the first maximum of logits[b] (amc_argmax's rule);
+// a target outside [0, C) gives a NaN row.  One thread per frame.
+__global__ void relevance_seed_kernel(int B, int C, const float* __restrict__ logits, const int64_t* __restrict__ target,
+                                      float* __restrict__ dlogits) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const int64_t t = target ? target[b] : row_argmax(logits + (size_t)b * C, C);
+  const bool ok = t >= 0 && t < C;
+  for (int c = 0; c < C; ++c) dlogits[(size_t)b * C + c] = ok ? (c == t ? 1.f : 0.f) : __int_as_float(0x7fffffff);
 }
 
 // warps per CTA (at most `cap`) whose shared memory fits the plan, or 0
@@ -378,9 +430,11 @@ int probs_launch(int B, int T, int h, int dh, const E* qkv, float* probs, cudaSt
   return 0;
 }
 
-template <typename E, int KD>
-int rollout_launch(int B, int T, int h, int dh, const E* qkv, const float* v_in, float* v_out, cudaStream_t st) {
-  const size_t wb = rollout_warp_bytes<E, KD>(T);
+template <typename E, int KD, bool REL = false>
+int rollout_launch(int B, int T, int h, int dh, const E* qkv, const float* v_in, float* v_out, cudaStream_t st,
+                   const E* dout = nullptr) {
+  const char* what = REL ? "attention_relevance_step" : "attention_rollout_step";
+  const size_t wb = rollout_warp_bytes<E, KD, REL>(T);
   // One CTA per frame of h * ceil(T / 16) tiles.  4 warps while the batch gives every SM two CTAs or more; 16 when it does
   // not, so that a small batch of long frames (conv1d: 128 frames, 520 tiles each) still fills the SMs (2.19 against
   // 6.28 ms per step).  With enough frames 16 warps lose 2-10 % to the longer cross-warp sum (DESIGN §5.8).  Never more
@@ -388,13 +442,19 @@ int rollout_launch(int B, int T, int h, int dh, const E* qkv, const float* v_in,
   const int tiles = h * ((T + 15) / 16);
   const int cap = B >= 2 * device_sm_count() ? 4 : 16;
   const int nw = std::min(warps_for(wb, cap), std::max(1, (tiles + 1) / 2));
-  AMC_CHECK_ARG(nw >= 1, "attention_rollout_step: T=%d dh=%d needs %zu bytes of shared memory per warp", T, dh, wb);
-  AMC_CUDA(cudaFuncSetAttribute(attn_rollout_kernel<E, KD>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_CAP));
-  attn_rollout_kernel<E, KD><<<B, nw * 32, nw * wb, st>>>(T, h, dh, qkv, v_in, v_out,
-                                                          1.4426950408889634f / sqrtf((float)dh), wb,
-                                                          vec_ok(qkv, h, dh, sizeof(E)) ? 1 : 0);
+  AMC_CHECK_ARG(nw >= 1, "%s: T=%d dh=%d needs %zu bytes of shared memory per warp", what, T, dh, wb);
+  AMC_CUDA(cudaFuncSetAttribute(attn_rollout_kernel<E, KD, REL>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_CAP));
+  const bool vec = vec_ok(qkv, h, dh, sizeof(E)) && (reinterpret_cast<uintptr_t>(dout) & 15) == 0;
+  attn_rollout_kernel<E, KD, REL><<<B, nw * 32, nw * wb, st>>>(T, h, dh, qkv, v_in, v_out,
+                                                               1.4426950408889634f / sqrtf((float)dh), wb, vec ? 1 : 0,
+                                                               dout);
   AMC_LAUNCH_CHECK();
   return 0;
+}
+template <typename E, int KD>
+int relevance_launch(int B, int T, int h, int dh, const E* qkv, const E* dout, const float* v_in, float* v_out,
+                     cudaStream_t st) {
+  return rollout_launch<E, KD, true>(B, T, h, dh, qkv, v_in, v_out, st, dout);
 }
 
 int check_shape(const char* what, int B, int T, int h, int dh) {
@@ -436,10 +496,29 @@ int attention_rollout_step(int B, int T, int h, int dh, const E* qkv, const floa
 template int attention_rollout_step<float>(int, int, int, int, const float*, const float*, float*, cudaStream_t);
 template int attention_rollout_step<bf16>(int, int, int, int, const bf16*, const float*, float*, cudaStream_t);
 
+template <typename E>
+int attention_relevance_step(int B, int T, int h, int dh, const E* qkv, const E* dout, const float* v_in, float* v_out,
+                             cudaStream_t st) {
+  AMC_TRY(check_shape("attention_relevance_step", B, T, h, dh));
+  if (B == 0) return 0;
+  AMC_MAPS_DISPATCH(relevance_launch, B, T, h, dh, qkv, dout, v_in, v_out, st)
+}
+template int attention_relevance_step<float>(int, int, int, int, const float*, const float*, const float*, float*,
+                                             cudaStream_t);
+template int attention_relevance_step<bf16>(int, int, int, int, const bf16*, const bf16*, const float*, float*,
+                                            cudaStream_t);
+
 int rollout_init(int B, int T, int has_cls, float* v, cudaStream_t st) {
   const int64_t n = (int64_t)B * T;
   if (n == 0) return 0;
   rollout_init_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(B, T, has_cls, v);
+  AMC_LAUNCH_CHECK();
+  return 0;
+}
+
+int relevance_seed(int B, int C, const float* logits, const int64_t* target, float* dlogits, cudaStream_t st) {
+  if (B == 0) return 0;
+  relevance_seed_kernel<<<(B + 127) / 128, 128, 0, st>>>(B, C, logits, target, dlogits);
   AMC_LAUNCH_CHECK();
   return 0;
 }

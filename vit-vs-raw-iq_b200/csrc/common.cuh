@@ -191,4 +191,16 @@ inline int device_sm_count() {
 inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// index of the first maximum of r[0..C) (torch.max(1) / argmax semantics of R/training/utils.py:311-317; a row with a NaN
+// gives the index of its first NaN, as torch does): amc_argmax and the relevance seed share it
+__device__ __forceinline__ int row_argmax(const float* r, int C) {
+  float best = r[0];
+  int bi = 0;
+  for (int c = 1; c < C; ++c) {
+    const float v = r[c];
+    if (best == best && (v > best || v != v)) { best = v; bi = c; }
+  }
+  return bi;
+}
+
 }  // namespace amc

@@ -978,19 +978,11 @@ int ce_loss(int B, int C, const float* logits, const int64_t* labels, float ls, 
   return 0;
 }
 
-// first index of the row maximum (torch.max(1) / argmax semantics of R/training/utils.py:311-317; NaN rows give the index
-// of the first NaN, as torch does); one thread per frame -- C is 11 or 19
+// first index of the row maximum (row_argmax); one thread per frame -- C is 11 or 19
 __global__ void argmax_kernel(int B, int C, const float* __restrict__ logits, int64_t* __restrict__ out) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
-  const float* r = logits + (size_t)b * C;
-  float best = r[0];
-  int bi = 0;
-  for (int c = 1; c < C; ++c) {
-    const float v = r[c];
-    if (best == best && (v > best || v != v)) { best = v; bi = c; }
-  }
-  out[b] = bi;
+  out[b] = row_argmax(logits + (size_t)b * C, C);
 }
 int argmax_rows(int B, int C, const float* logits, int64_t* out, cudaStream_t st) {
   if (B == 0) return 0;

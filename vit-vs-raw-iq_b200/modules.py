@@ -435,6 +435,54 @@ class _AMCBase(nn.Module):
         _, roll = self._attention(src, 0, True)
         return roll
 
+    @torch.no_grad()
+    def attention_relevance(self, src, target=None) -> torch.Tensor:
+        """Class-specific attention relevance: the gradient-weighted rollout of Chefer, Gur & Wolf, "Generic
+        Attention-model Explainability" (ICCV 2021).  Where ``attention_rollout`` gives one map per frame, this answers
+        "which tokens made the model score class t?".
+
+        ``r = u^T (I + A_{L-1}) ... (I + A_0)`` with ``A_l = mean_heads(relu(dy_t/dP_l * P_l))``: ``P_l`` the attention
+        probabilities of layer l, ``y_t`` the logit of the target class (not the loss and not the softmax), and ``u`` the
+        head's read-out of the top layer, ``e_0`` for a CLS model or ``1/T`` on every token for mean pooling.  The
+        gradient comes from a frozen backward on the device; no ``[B, h, T, T]`` tensor is materialised.
+
+        ``target`` is ``None`` (each frame's predicted class, the first maximum of its logits) or a contiguous int64
+        CUDA tensor ``[B]`` on the model's device with values in ``[0, num_classes)``; anything else raises
+        ``ValueError``.  Returns fp32 ``[B, T]``; columns as in ``attention_rollout`` (column 0 is the CLS token when the
+        model has one).  Every entry is non-negative and ``r >= u`` elementwise, so ``r[:, 0] >= 1`` for CLS models.
+        Rows are not normalised: divide by the row sum, or subtract ``u``, to compare frames.
+
+        ``src`` is what ``forward`` takes (either input layout).  Runs under ``torch.no_grad()`` with dropout off whatever
+        ``self.training`` is, in the model's compute dtype; parameters, their ``.grad`` and ``training`` are left as they
+        are.  Memory: the training-mode workspace of the batch plus ``[B, T]`` and ``[B, num_classes]`` fp32."""
+        core = self._core
+        B = int(src.shape[0]) if src.dim() >= 1 else -1
+        if target is not None:
+            if not isinstance(target, torch.Tensor):
+                raise ValueError(f"target must be None or an int64 CUDA tensor [B], got {type(target).__name__}")
+            if target.dtype != torch.int64 or target.dim() != 1 or target.shape[0] != B or not target.is_contiguous():
+                raise ValueError(f"target must be a contiguous int64 tensor of shape [{B}], got {target.dtype} "
+                                 f"{tuple(target.shape)}")
+            if target.device != core.params[0].device:
+                raise ValueError(f"target is on {target.device}, the model on {core.params[0].device}")
+            if B > 0:
+                lo, hi = torch.aminmax(target)
+                lo, hi = int(lo), int(hi)
+                if lo < 0 or hi >= core.C:
+                    raise ValueError(f"target values must lie in [0, {core.C}), got [{lo}, {hi}]")
+        # training=1 keeps every layer's activations for the backward; module_training=False turns dropout off
+        desc = core.make_desc(src, training=True, module_training=False)
+        dev = src.device
+        ws = torch.empty(_lib.workspace_bytes(desc), dtype=torch.uint8, device=dev)
+        logits = torch.empty((desc.B, core.C), dtype=torch.float32, device=dev)
+        rel = torch.empty((desc.B, core.layout.T), dtype=torch.float32, device=dev)
+        _lib.check(_lib.lib.amc_model_relevance(C.byref(desc), src.data_ptr(), core.flat.data_ptr(),
+                                                core.pos_buffer().data_ptr(), ws.data_ptr(), _lib.ptr(target),
+                                                logits.data_ptr(), rel.data_ptr(),
+                                                torch.cuda.current_stream(dev).cuda_stream),
+                   "amc_model_relevance")
+        return rel
+
     def _run(self, src, want_logits):
         # grad mode is switched off inside Function.forward, so decide here whether to keep activations
         need_grad = torch.is_grad_enabled() and (src.requires_grad or any(p.requires_grad for p in self._core.params))
