@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AMC_ABI_VERSION 11
+#define AMC_ABI_VERSION 12
 
 enum { AMC_KIND_RAWIQ = 0, AMC_KIND_VIT = 1 };
 enum { AMC_F32 = 0, AMC_BF16 = 1 };
@@ -177,6 +177,36 @@ int amc_model_attention(const AmcDesc* desc, const float* src, const float* para
  * frozen one of amc_model_bwd_ex with grads = NULL and no dsrc; it stops after layer 0's out-projection gradient. */
 int amc_model_relevance(const AmcDesc* desc, const float* src, const float* params, const float* pos, void* workspace,
                         const int64_t* target, float* logits, float* relevance, amc_stream_t stream);
+
+/* Integrated Gradients (Sundararajan, Taly & Yan, "Axiomatic Attribution for Deep Networks", ICML 2017) of the model of
+ * R/models/transformer_rawIQ.py:72-98 / V/models/amc_transformer.py:26-31 with dropout off, w.r.t. the input frames:
+ *   attr = (src - baseline) * sum_k weight[k] * dy_t/dsrc (baseline + alpha[k] (src - baseline)),  k = 0 .. steps-1
+ * y_t the logit of class t_b (not the loss, not the softmax); with Gauss-Legendre nodes and weights on [0, 1] the sum is
+ * the quadrature of the path integral, and sum(attr[b]) -> y_t(src_b) - y_t(baseline_b) (completeness).
+ * desc->training must be 1 and desc->p_drop 0.  The workspace is amc_model_ig_workspace(desc, chunk) bytes.
+ *   src, baseline  device fp32, both in the layout desc->input_layout defines ([B,L,2] dataset frames: the attribution
+ *                  is w.r.t. the un-normalised samples, as dsrc of amc_model_bwd_ex)
+ *   target         device int64 [B], or NULL: t_b = the first maximum of logits[0, b] (amc_argmax's rule)
+ *   alpha, weight  device fp32 [steps]: the path points and their quadrature weights
+ *   chunk          path points per device pass: each pass runs the layers forward and the frozen backward on chunk * B
+ *                  frames (the last pass on what is left)
+ *   logits         fp32 [2, B, C] out: the logits of src, then of baseline (one forward of both, the top layer of a CLS
+ *                  model on its CLS rows as in amc_model_fwd)
+ *   attr           fp32 out, the shape and layout of src; overwritten; samples no patch covers get 0
+ * How: the front end runs once on [src; baseline]; a path point's embedding rows are blended from the two (the front
+ * end is affine in src); the seed weight[k] * e_t enters the frozen backward of amc_model_bwd_ex (grads = NULL), which
+ * stops at the embedding rows; their gradients are summed over the points in fp32 in a fixed order (no atomics: repeated
+ * calls are bit-identical), and the embedding dgrad and the scatter into the input layout, multiplied by
+ * src - baseline, run once.  A target outside [0, C) makes that frame's rows of attr NaN (the amc_ce_loss convention;
+ * samples no patch covers stay 0) and leaves the other frames as they are. */
+int amc_model_integrated_gradients(const AmcDesc* desc, const float* src, const float* baseline, const float* params,
+                                   const float* pos, void* workspace, const int64_t* target, int steps,
+                                   const float* alpha, const float* weight, int chunk, float* logits, float* attr,
+                                   amc_stream_t stream);
+/* Workspace of amc_model_integrated_gradients with `chunk` path points per pass: the training-mode workspace
+ * (amc_model_workspace) of max(2, chunk) * B frames, plus [src; baseline], both endpoints' embedding rows and the
+ * gradient sum in fp32. */
+int amc_model_ig_workspace(const AmcDesc* desc, int chunk, AmcWorkspaceInfo* out);
 
 /* nn.CrossEntropyLoss(label_smoothing) + argmax statistics (R/training/train.py:260,274-277,504).
  *   stats[0] += sum of per-frame losses * loss_scale, stats[1] += #correct (fp32 accumulators)

@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libamc_b200.so")
 
-ABI_VERSION = 11
+ABI_VERSION = 12
 KIND_RAWIQ, KIND_VIT = 0, 1
 F32, BF16 = 0, 1
 INPUT_MODEL, INPUT_RAW = 0, 1
@@ -63,6 +63,8 @@ def _load():
         "amc_model_bwd_ex": [C.POINTER(AmcDesc), vp, vp, vp, vp, vp, vp, vp, i32, i32, vp],
         "amc_model_attention": [C.POINTER(AmcDesc), vp, vp, vp, vp, C.c_uint32, vp, vp, vp],
         "amc_model_relevance": [C.POINTER(AmcDesc), vp, vp, vp, vp, vp, vp, vp, vp],
+        "amc_model_integrated_gradients": [C.POINTER(AmcDesc), vp, vp, vp, vp, vp, vp, i32, vp, vp, i32, vp, vp, vp],
+        "amc_model_ig_workspace": [C.POINTER(AmcDesc), i32, C.POINTER(AmcWorkspaceInfo)],
         "amc_ce_loss": [i32, i32, vp, vp, f32, f32, f32, vp, vp, vp],
         "amc_argmax": [i32, i32, vp, vp, vp],
         "amc_zero": [vp, C.c_size_t, vp],
@@ -123,6 +125,12 @@ def param_layout(desc: AmcDesc) -> AmcParamLayout:
 def workspace_bytes(desc: AmcDesc) -> int:
     out = AmcWorkspaceInfo()
     check(lib.amc_model_workspace(C.byref(desc), C.byref(out)), "amc_model_workspace")
+    return int(out.bytes)
+
+
+def ig_workspace_bytes(desc: AmcDesc, chunk: int) -> int:
+    out = AmcWorkspaceInfo()
+    check(lib.amc_model_ig_workspace(C.byref(desc), chunk, C.byref(out)), "amc_model_ig_workspace")
     return int(out.bytes)
 
 

@@ -505,6 +505,10 @@ struct Model {
     if (m.B == 0) return 0;
     AMC_TRY(pack_weights(D.training));
     AMC_TRY(frontend(src, pos));
+    return forward_layers(logits, enc_out);
+  }
+  // the encoder layers and the head, from the x0 rows in w.x16[0] / w.x32[0] (the weights packed)
+  int forward_layers(float* logits, float* enc_out) {
     // Only the CLS rows of the top layer reach the head (transformer_rawIQ.py:88-90, amc_transformer.py:29): when
     // just the logits are wanted, the top layer's out-proj / FFN / LayerNorms run on those B rows alone.
     const bool cls_top = m.has_cls && logits && !enc_out && m.L >= 1;
@@ -572,7 +576,7 @@ struct Model {
     AMC_CHECK_ARG(vn + (size_t)m.B * m.C <= m.M * (size_t)m.d, "amc_model_relevance: scratch too small");
     AMC_TRY(forward(src, pos, logits, nullptr));
     float* dlogits = w.u32 + vn;
-    AMC_PROF("relevance", 0.0, 0.0, relevance_seed(m.B, m.C, logits, target, dlogits, st));
+    AMC_PROF("relevance", 0.0, 0.0, relevance_seed(m.B, m.B, m.C, logits, target, nullptr, dlogits, st));
     AMC_TRY(backward(dlogits, nullptr, nullptr, nullptr, 0, 1));   // head
     const bool cls_top = m.has_cls;                                 // forward() ran with logits: mirrors its choice
     float* v[2] = {relevance, w.u32};
@@ -754,16 +758,18 @@ struct Model {
 
   // Input gradient (stage n_layers+1), autograd of the patch embedding and of the dataset z-score + framing:
   // dX = demb W_emb, then the transpose of the patch map into dsrc (caller's layout, * 1/std_c for dataset input).
-  int input_grad(float* dsrc) {
+  // With src and base (Integrated Gradients) every element is also multiplied by src - base.
+  int input_grad(const E* demb, float* dsrc, const float* src = nullptr, const float* base = nullptr) {
     const int Mt = m.B * m.Ttok;
+    const double mul_bytes = src ? 8.0 * Mt * m.K : 0.0;
     if (sizeof(E) == 2 && m.K % 8 != 0) {
-      AMC_PROF("frontend_bwd_dsrc", 2.0 * Mt * m.d * m.K, (double)Mt * (m.d * 2 + m.K * 4),
-               embed_smallk_dgrad(D, m.Ttok, m.d, m.K, (const bf16*)w.demb, (const bf16*)Wemb(), dsrc, st));
+      AMC_PROF("frontend_bwd_dsrc", 2.0 * Mt * m.d * m.K, (double)Mt * (m.d * 2 + m.K * 4) + mul_bytes,
+               embed_smallk_dgrad(D, m.Ttok, m.d, m.K, (const bf16*)demb, (const bf16*)Wemb(), dsrc, st, src, base));
       return 0;
     }
     GemmArgs g;
     g.M = Mt; g.N = m.K; g.K = m.d;
-    g.A = w.demb; g.lda = m.d;
+    g.A = demb; g.lda = m.d;
     if (sizeof(E) == 2) {   // tcgen05 needs both operands K-major: W_emb [d, K] -> [K, d]
       TransposeBatch tb;
       tb.n = 1;
@@ -776,7 +782,8 @@ struct Model {
     g.name = "frontend_bwd_dsrc";
     g.epi.D32 = w.dx; g.epi.ldd32 = m.K;
     AMC_TRY(gemm<E>(g, st));
-    AMC_PROF("frontend_bwd_dsrc", 0.0, (double)Mt * m.K * 8, patch_scatter(D, m.Ttok, m.K, w.dx, dsrc, st));
+    AMC_PROF("frontend_bwd_dsrc", 0.0, (double)Mt * m.K * 8 + mul_bytes,
+             patch_scatter(D, m.Ttok, m.K, w.dx, dsrc, st, src, base));
     return 0;
   }
 
@@ -826,12 +833,121 @@ struct Model {
           g.epi.D32 = GP(L.emb_w); g.epi.ldd32 = m.K; g.epi.accumulate = 1;
           AMC_TRY(gemm<E>(g, st));
         }
-        if (dsrc) AMC_TRY(input_grad(dsrc));
+        if (dsrc) AMC_TRY(input_grad((const E*)w.demb, dsrc));
       }
     }
     return 0;
   }
 };
+
+template <typename E>
+size_t model_ws_bytes(const AmcDesc& D, const Dims& m, const AmcParamLayout& L) {
+  Work w;
+  carve<E>(D, m, L, nullptr, w);
+  return std::max<size_t>(w.bytes, 256);
+}
+size_t model_ws_bytes(const AmcDesc& D, const Dims& m, const AmcParamLayout& L) {
+  return D.dtype == AMC_BF16 ? model_ws_bytes<bf16>(D, m, L) : model_ws_bytes<float>(D, m, L);
+}
+
+// ---- Integrated Gradients -----------------------------------------------------------------
+// Workspace of amc_model_integrated_gradients for chunks of `chunk` path points, in order: [src; baseline] as one
+// 2B-frame batch, the endpoint embeddings x0e = [x0(x); x0(x')] fp32, the fp32 sum of the token-row gradients over the
+// points, its E copy (the dsrc GEMM's operand), the chunk's seed and logits, then the training-mode workspace of the
+// larger of the 2B-frame endpoint forward and the chunk's chunk * B frames, which each pass carves afresh.
+struct IgPlan {
+  size_t src2, x0e, acc, demb, dlogits, clogits, model, bytes;
+};
+int ig_plan(const AmcDesc& D, int chunk, IgPlan& p) {
+  Dims m;
+  AmcParamLayout L;
+  AMC_TRY(validate(D, m));
+  AMC_TRY(make_layout(D, m, L));
+  AMC_CHECK_ARG(chunk >= 1, "integrated_gradients: chunk must be >= 1");
+  AMC_CHECK_ARG(std::max<int64_t>((int64_t)chunk * D.B, 2 * (int64_t)D.B) <= INT32_MAX,
+                "integrated_gradients: too many frames per pass");
+  AmcDesc D2 = D, Dc = D;
+  D2.B = 2 * D.B;
+  Dc.B = chunk * D.B;
+  Dims m2, mc;
+  AMC_TRY(validate(D2, m2));
+  AMC_TRY(validate(Dc, mc));
+  const size_t e = D.dtype == AMC_BF16 ? 2 : 4, B = D.B, tok = B * m.Ttok * m.d;
+  size_t off = 0;
+  auto take = [&](size_t bytes) { size_t r = off; off += align_up(bytes, 256); return r; };
+  p.src2 = take(2 * B * frame_floats(D) * 4);
+  p.x0e = take(2 * B * m.T * m.d * 4);
+  p.acc = take(tok * 4);
+  p.demb = e == 4 ? p.acc : take(tok * e);
+  p.dlogits = take((size_t)chunk * B * m.C * 4);
+  p.clogits = take((size_t)chunk * B * m.C * 4);
+  p.model = take(std::max(model_ws_bytes(D2, m2, L), model_ws_bytes(Dc, mc, L)));
+  p.bytes = off;
+  return 0;
+}
+
+// IG_t(x) = (x - x') * sum_k w_k dy_t/dx (x' + a_k (x - x')) over `steps` path points (a_k, w_k device fp32).
+//  1. one forward of [x; x'] (2B frames) gives both endpoints' logits and x0 rows;
+//  2. per chunk of n points: x0 rows blended in frame order k*B + b, the layers and head forward, the seed w_k e_t,
+//     the frozen backward (grads = NULL) down to dx0, and the token rows of dx0 summed over the chunk's points into acc
+//     (fixed order, no atomics);
+//  3. once: the dsrc GEMM on that sum and the scatter multiplied by src - base.
+// Each model pass carves the same region afresh; what lives across passes is in the plan's first buffers.
+template <typename E>
+int integrated_gradients(const AmcDesc& D, const float* src, const float* base, const float* params, const float* pos,
+                         char* ws, const int64_t* target, int steps, const float* alpha, const float* weight, int chunk,
+                         float* logits, float* attr, cudaStream_t st) {
+  AMC_CHECK_ARG(D.training == 1 && D.p_drop == 0.f,
+                "amc_model_integrated_gradients needs desc.training=1 and desc.p_drop=0");
+  AMC_CHECK_ARG(steps >= 1, "amc_model_integrated_gradients: steps must be >= 1");
+  IgPlan p;
+  AMC_TRY(ig_plan(D, chunk, p));
+  if (D.B == 0) return 0;
+  AMC_CHECK_ARG(ws != nullptr && (reinterpret_cast<uintptr_t>(ws) & 255) == 0,
+                "workspace is NULL or not 256-byte aligned");
+  const int B = D.B;
+  float* src2 = (float*)(ws + p.src2);
+  float* x0e = (float*)(ws + p.x0e);
+  float* acc = (float*)(ws + p.acc);
+  E* demb = (E*)(ws + p.demb);
+  float* dlogits = (float*)(ws + p.dlogits);
+  float* clogits = (float*)(ws + p.clogits);
+  const size_t nsrc = (size_t)B * frame_floats(D);
+  AMC_CUDA(cudaMemcpyAsync(src2, src, nsrc * 4, cudaMemcpyDeviceToDevice, st));
+  AMC_CUDA(cudaMemcpyAsync(src2 + nsrc, base, nsrc * 4, cudaMemcpyDeviceToDevice, st));
+  AmcDesc D2 = D;
+  D2.B = 2 * B;
+  Dims m;
+  {
+    Model<E> me(D2, params, st);
+    AMC_TRY(me.init(ws + p.model));
+    AMC_TRY(me.forward(src2, pos, logits, nullptr));
+    AMC_CUDA(cudaMemcpyAsync(x0e, me.w.x32[0], (size_t)me.m.M * me.m.d * 4, cudaMemcpyDeviceToDevice, st));
+    m = me.m;
+  }
+  const int64_t n_frame = (int64_t)B * m.T * m.d;
+  for (int k0 = 0; k0 < steps; k0 += chunk) {
+    const int n = std::min(chunk, steps - k0);
+    AmcDesc Dc = D;
+    Dc.B = n * B;
+    Model<E> mc(Dc, params, st);
+    AMC_TRY(mc.init(ws + p.model));
+    AMC_TRY(mc.pack_weights(true));
+    AMC_PROF("ig_blend", 0.0, (double)n * n_frame * (4 + sizeof(E)) + 2.0 * n_frame * 4,
+             ig_blend<E>(n, n_frame, alpha + k0, x0e, (E*)mc.w.x16[0], mc.w.x32[0], st));
+    AMC_TRY(mc.forward_layers(clogits, nullptr));
+    AMC_PROF("ig_seed", 0.0, 0.0, relevance_seed(n * B, B, m.C, logits, target, weight + k0, dlogits, st));
+    AMC_TRY(mc.backward(dlogits, nullptr, nullptr, nullptr, 0, m.L + 1));
+    const bool last = k0 + n >= steps;
+    const double tok = (double)B * m.Ttok * m.d;
+    AMC_PROF("ig_reduce", 0.0, tok * (4.0 * n + (k0 ? 8 : 4) + (last ? sizeof(E) : 0)),
+             ig_reduce<E>(B, m.T, m.Ttok, m.d, m.has_cls, n, mc.w.dy32, acc, k0 == 0, last ? demb : nullptr, st));
+  }
+  Model<E> mb(D, params, st);
+  AMC_TRY(mb.init(ws + p.model));
+  AMC_TRY(mb.pack_weights(false));
+  return mb.input_grad(demb, attr, src, base);
+}
 
 }  // namespace
 }  // namespace amc
@@ -857,12 +973,33 @@ int amc_model_workspace(const AmcDesc* desc, AmcWorkspaceInfo* out) {
   AmcParamLayout L;
   AMC_TRY(validate(*desc, m));
   AMC_TRY(make_layout(*desc, m, L));
-  Work w;
-  if (desc->dtype == AMC_BF16) carve<bf16>(*desc, m, L, nullptr, w);
-  else carve<float>(*desc, m, L, nullptr, w);
-  out->bytes = std::max<size_t>(w.bytes, 256);
+  out->bytes = model_ws_bytes(*desc, m, L);
   out->saved_bytes = out->bytes;
   return 0;
+}
+
+int amc_model_ig_workspace(const AmcDesc* desc, int chunk, AmcWorkspaceInfo* out) {
+  AMC_CHECK_ARG(desc && out, "NULL argument");
+  IgPlan p;
+  AMC_TRY(ig_plan(*desc, chunk, p));
+  out->bytes = p.bytes;
+  out->saved_bytes = p.bytes;
+  return 0;
+}
+
+int amc_model_integrated_gradients(const AmcDesc* desc, const float* src, const float* baseline, const float* params,
+                                   const float* pos, void* workspace, const int64_t* target, int steps,
+                                   const float* alpha, const float* weight, int chunk, float* logits, float* attr,
+                                   amc_stream_t stream) {
+  DeviceGuard dev_guard(params);
+  AMC_CHECK_ARG(desc && params && pos, "NULL argument");
+  AMC_CHECK_ARG(desc->B == 0 || (src && baseline && alpha && weight && logits && attr), "NULL argument");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (desc->dtype == AMC_BF16)
+    return integrated_gradients<bf16>(*desc, src, baseline, params, pos, (char*)workspace, target, steps, alpha, weight,
+                                      chunk, logits, attr, st);
+  return integrated_gradients<float>(*desc, src, baseline, params, pos, (char*)workspace, target, steps, alpha, weight,
+                                     chunk, logits, attr, st);
 }
 
 int amc_model_fwd(const AmcDesc* desc, const float* src, const float* params, const float* pos, void* workspace,

@@ -57,5 +57,7 @@ int attention_relevance_step(int B, int T, int h, int dh, const E* qkv, const E*
 int rollout_init(int B, int T, int has_cls, float* v, cudaStream_t st);
 // dlogits fp32 [B, C] = one_hot(target[b]), or of the first maximum of logits[b] with target NULL; NaN rows for targets
 // outside [0, C)
-int relevance_seed(int B, int C, const float* logits, const int64_t* target, float* dlogits, cudaStream_t st);
+// dlogits[r] = w_k one_hot(t_b) for the n rows r = k * B + b (see relevance_seed_kernel); weight NULL: w_k = 1
+int relevance_seed(int n, int B, int C, const float* logits, const int64_t* target, const float* weight, float* dlogits,
+                   cudaStream_t st);
 }  // namespace amc

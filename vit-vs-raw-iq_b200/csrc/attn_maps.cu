@@ -395,15 +395,19 @@ __global__ void rollout_init_kernel(int B, int T, int has_cls, float* __restrict
   v[i] = has_cls ? (t == 0 ? 1.f : 0.f) : 1.f / (float)T;
 }
 
-// dlogits[b] = one_hot(t_b): t_b = target[b], or with target NULL the first maximum of logits[b] (amc_argmax's rule);
-// a target outside [0, C) gives a NaN row.  One thread per frame.
-__global__ void relevance_seed_kernel(int B, int C, const float* __restrict__ logits, const int64_t* __restrict__ target,
+// dlogits[r] = w_k one_hot(t_b) for the n rows r = k * B + b: t_b = target[b], or with target NULL the first maximum of
+// logits[b] (amc_argmax's rule); w_k = weight[k], or 1 with weight NULL (relevance: n = B).  A target outside [0, C)
+// gives a NaN row.  One thread per row.
+__global__ void relevance_seed_kernel(int n, int B, int C, const float* __restrict__ logits,
+                                      const int64_t* __restrict__ target, const float* __restrict__ weight,
                                       float* __restrict__ dlogits) {
-  const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  if (b >= B) return;
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  const int k = r / B, b = r - k * B;
   const int64_t t = target ? target[b] : row_argmax(logits + (size_t)b * C, C);
   const bool ok = t >= 0 && t < C;
-  for (int c = 0; c < C; ++c) dlogits[(size_t)b * C + c] = ok ? (c == t ? 1.f : 0.f) : __int_as_float(0x7fffffff);
+  const float w = weight ? weight[k] : 1.f;
+  for (int c = 0; c < C; ++c) dlogits[(size_t)r * C + c] = ok ? (c == t ? w : 0.f) : __int_as_float(0x7fffffff);
 }
 
 // warps per CTA (at most `cap`) whose shared memory fits the plan, or 0
@@ -516,9 +520,10 @@ int rollout_init(int B, int T, int has_cls, float* v, cudaStream_t st) {
   return 0;
 }
 
-int relevance_seed(int B, int C, const float* logits, const int64_t* target, float* dlogits, cudaStream_t st) {
-  if (B == 0) return 0;
-  relevance_seed_kernel<<<(B + 127) / 128, 128, 0, st>>>(B, C, logits, target, dlogits);
+int relevance_seed(int n, int B, int C, const float* logits, const int64_t* target, const float* weight, float* dlogits,
+                   cudaStream_t st) {
+  if (n == 0) return 0;
+  relevance_seed_kernel<<<(n + 127) / 128, 128, 0, st>>>(n, B, C, logits, target, weight, dlogits);
   AMC_LAUNCH_CHECK();
   return 0;
 }

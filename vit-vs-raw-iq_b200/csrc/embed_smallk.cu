@@ -63,10 +63,13 @@ __global__ void __launch_bounds__(256) embed_smallk_bwd_kernel(int M, int N, int
 }
 
 // a warp per token row: the row of dY is read once, K <= 16 partial sums per lane are reduced across the warp in a
-// fixed order (no atomics: deterministic), lane k writes element k of the patch through the front end's map
+// fixed order (no atomics: deterministic), lane k writes element k of the patch through the front end's map;
+// MUL (Integrated Gradients) also multiplies it by src - base at that offset
+template <bool MUL>
 __global__ void __launch_bounds__(256) embed_smallk_dgrad_kernel(int M, int N, int K, const bf16* __restrict__ dY,
                                                                  const bf16* __restrict__ W, PatchP p,
-                                                                 float* __restrict__ dsrc) {
+                                                                 float* __restrict__ dsrc, const float* __restrict__ src,
+                                                                 const float* __restrict__ base) {
   extern __shared__ float sw[];   // W [N, K] in fp32
   for (int i = threadIdx.x; i < N * K; i += blockDim.x) sw[i] = to_f(W[i]);
   __syncthreads();
@@ -93,7 +96,8 @@ __global__ void __launch_bounds__(256) embed_smallk_dgrad_kernel(int M, int N, i
       const int b = m / p.Ttok, t = m - b * p.Ttok;
       int ch;
       const size_t o = patch_src_offset(p, b, t, lane, &ch);
-      dsrc[o] = ch < 0 ? v : v * p.inv_std[ch];
+      const float g = ch < 0 ? v : v * p.inv_std[ch];
+      dsrc[o] = MUL ? g * (__ldg(src + o) - __ldg(base + o)) : g;
     }
   }
 }
@@ -125,15 +129,19 @@ int embed_smallk_bwd(int M, int N, int K, const bf16* dY, int ldy, const bf16* A
 }
 
 int embed_smallk_dgrad(const AmcDesc& D, int Ttok, int N, int K, const bf16* dY, const bf16* W, float* dsrc,
-                       cudaStream_t st) {
+                       cudaStream_t st, const float* src, const float* base) {
   AMC_CHECK_ARG(embed_smallk_supported(K), "small-K embedding: K=%d unsupported (1..%d)", K, SK_MAX);
   const int M = D.B * Ttok;
   if (M == 0) return 0;
   if ((int64_t)Ttok * K != frame_floats(D))
     AMC_CUDA(cudaMemsetAsync(dsrc, 0, (size_t)D.B * frame_floats(D) * sizeof(float), st));
   const int blocks = std::min(ceil_div(M, 8), 148 * 8);
-  embed_smallk_dgrad_kernel<<<blocks, 256, (size_t)N * K * sizeof(float), st>>>(M, N, K, dY, W, make_patchp(D, Ttok, K),
-                                                                                 dsrc);
+  const size_t smem = (size_t)N * K * sizeof(float);
+  if (src)
+    embed_smallk_dgrad_kernel<true><<<blocks, 256, smem, st>>>(M, N, K, dY, W, make_patchp(D, Ttok, K), dsrc, src, base);
+  else
+    embed_smallk_dgrad_kernel<false><<<blocks, 256, smem, st>>>(M, N, K, dY, W, make_patchp(D, Ttok, K), dsrc, nullptr,
+                                                                nullptr);
   AMC_LAUNCH_CHECK();
   return 0;
 }

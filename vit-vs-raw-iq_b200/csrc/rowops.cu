@@ -279,8 +279,11 @@ __global__ void __launch_bounds__(256) patchify_kernel(PatchP p, const float* __
 }
 
 // Input gradient, last step: the transpose of patchify.  d(x - mean) * inv_std / dx = inv_std in dataset layout.
+// MUL (Integrated Gradients): the value is also multiplied by src - base at the same offset.
+template <bool MUL>
 __global__ void __launch_bounds__(256) patch_scatter_kernel(PatchP p, const float* __restrict__ dX,
-                                                            float* __restrict__ dsrc) {
+                                                            float* __restrict__ dsrc, const float* __restrict__ src,
+                                                            const float* __restrict__ base) {
   const size_t total = (size_t)p.B * p.Ttok * p.K;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
     const int k = (int)(i % p.K);
@@ -289,7 +292,8 @@ __global__ void __launch_bounds__(256) patch_scatter_kernel(PatchP p, const floa
     int ch;
     const size_t o = patch_src_offset(p, b, t, k, &ch);
     const float g = dX[i];
-    dsrc[o] = ch < 0 ? g : g * p.inv_std[ch];
+    const float v = ch < 0 ? g : g * p.inv_std[ch];
+    dsrc[o] = MUL ? v * (__ldg(src + o) - __ldg(base + o)) : v;
   }
 }
 
@@ -873,13 +877,17 @@ int patchify(const AmcDesc& D, int Ttok, int K, const float* src, E* A, cudaStre
 template int patchify<float>(const AmcDesc&, int, int, const float*, float*, cudaStream_t);
 template int patchify<bf16>(const AmcDesc&, int, int, const float*, bf16*, cudaStream_t);
 
-int patch_scatter(const AmcDesc& D, int Ttok, int K, const float* dX, float* dsrc, cudaStream_t st) {
+int patch_scatter(const AmcDesc& D, int Ttok, int K, const float* dX, float* dsrc, cudaStream_t st, const float* src,
+                  const float* base) {
   if (D.B == 0) return 0;
   if ((int64_t)Ttok * K != frame_floats(D))
     AMC_CUDA(cudaMemsetAsync(dsrc, 0, (size_t)D.B * frame_floats(D) * sizeof(float), st));
   const size_t total = (size_t)D.B * Ttok * K;
   const int blocks = (int)std::min<size_t>((total + 255) / 256, 148 * 16);
-  patch_scatter_kernel<<<blocks, 256, 0, st>>>(make_patchp(D, Ttok, K), dX, dsrc);
+  if (src)
+    patch_scatter_kernel<true><<<blocks, 256, 0, st>>>(make_patchp(D, Ttok, K), dX, dsrc, src, base);
+  else
+    patch_scatter_kernel<false><<<blocks, 256, 0, st>>>(make_patchp(D, Ttok, K), dX, dsrc, nullptr, nullptr);
   AMC_LAUNCH_CHECK();
   return 0;
 }

@@ -72,8 +72,10 @@ int colsum(int M, int N, const E* X, int ld, float* out, cudaStream_t st);
 template <typename E>
 int patchify(const AmcDesc& D, int Ttok, int K, const float* src, E* A, cudaStream_t st);
 // inverse of patchify for gradients: dsrc[map(row, k)] = dX[row, k] (* 1/std_c in dataset layout); every element of
-// dsrc is written (uncovered samples are zeroed)
-int patch_scatter(const AmcDesc& D, int Ttok, int K, const float* dX, float* dsrc, cudaStream_t st);
+// dsrc is written (uncovered samples are zeroed).  With src and base (Integrated Gradients) each value is also
+// multiplied by src - base at the same offset.
+int patch_scatter(const AmcDesc& D, int Ttok, int K, const float* dX, float* dsrc, cudaStream_t st,
+                  const float* src = nullptr, const float* base = nullptr);
 template <typename E>
 int cls_rows(int B, int T, int d, const float* cls, const float* pos, E* y16, float* y32, const DropoutCfg& drop,
              cudaStream_t st);
@@ -88,6 +90,13 @@ int head_fwd(int B, int T, int d, int C, int has_cls, int head_ln, float eps, co
 int head_bwd(int B, int T, int d, int C, int has_cls, int head_ln, const float* dlogits, const float* W,
              const float* lnw, const float* s_hl, const float* s_xhat, const float* s_rstd, float* dhl_scratch,
              float* dxL, float* dW, float* dbias, float* dlnw, float* dlnb, cudaStream_t st);
+// Integrated Gradients (attribution.cu): the path points' x0 rows blended from the two endpoint embeddings
+// x0e = [x0(x); x0(x')] (n_frame floats each), and the sum of their token-row gradients over the points
+template <typename E>
+int ig_blend(int n_points, int64_t n_frame, const float* alpha, const float* x0e, E* x16, float* x32, cudaStream_t st);
+template <typename E>
+int ig_reduce(int B, int T, int Ttok, int d, int has_cls, int n, const float* dx0, float* acc, bool first, E* out,
+              cudaStream_t st);
 int argmax_rows(int B, int C, const float* logits, int64_t* out, cudaStream_t st);
 int ce_loss(int B, int C, const float* logits, const int64_t* labels, float ls, float grad_scale, float loss_scale,
             float* dlogits, float* stats, cudaStream_t st);

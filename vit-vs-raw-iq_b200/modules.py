@@ -456,20 +456,7 @@ class _AMCBase(nn.Module):
         ``self.training`` is, in the model's compute dtype; parameters, their ``.grad`` and ``training`` are left as they
         are.  Memory: the training-mode workspace of the batch plus ``[B, T]`` and ``[B, num_classes]`` fp32."""
         core = self._core
-        B = int(src.shape[0]) if src.dim() >= 1 else -1
-        if target is not None:
-            if not isinstance(target, torch.Tensor):
-                raise ValueError(f"target must be None or an int64 CUDA tensor [B], got {type(target).__name__}")
-            if target.dtype != torch.int64 or target.dim() != 1 or target.shape[0] != B or not target.is_contiguous():
-                raise ValueError(f"target must be a contiguous int64 tensor of shape [{B}], got {target.dtype} "
-                                 f"{tuple(target.shape)}")
-            if target.device != core.params[0].device:
-                raise ValueError(f"target is on {target.device}, the model on {core.params[0].device}")
-            if B > 0:
-                lo, hi = torch.aminmax(target)
-                lo, hi = int(lo), int(hi)
-                if lo < 0 or hi >= core.C:
-                    raise ValueError(f"target values must lie in [0, {core.C}), got [{lo}, {hi}]")
+        self._check_target(src, target)
         # training=1 keeps every layer's activations for the backward; module_training=False turns dropout off
         desc = core.make_desc(src, training=True, module_training=False)
         dev = src.device
@@ -482,6 +469,119 @@ class _AMCBase(nn.Module):
                                                 torch.cuda.current_stream(dev).cuda_stream),
                    "amc_model_relevance")
         return rel
+
+    def _check_target(self, src, target) -> None:
+        """ValueError unless ``target`` is None or a contiguous int64 tensor [B] on the model's device with values in
+        [0, num_classes)."""
+        if target is None:
+            return
+        core = self._core
+        B = int(src.shape[0]) if src.dim() >= 1 else -1
+        if not isinstance(target, torch.Tensor):
+            raise ValueError(f"target must be None or an int64 CUDA tensor [B], got {type(target).__name__}")
+        if target.dtype != torch.int64 or target.dim() != 1 or target.shape[0] != B or not target.is_contiguous():
+            raise ValueError(f"target must be a contiguous int64 tensor of shape [{B}], got {target.dtype} "
+                             f"{tuple(target.shape)}")
+        if target.device != core.params[0].device:
+            raise ValueError(f"target is on {target.device}, the model on {core.params[0].device}")
+        if B > 0:
+            lo, hi = torch.aminmax(target)
+            lo, hi = int(lo), int(hi)
+            if lo < 0 or hi >= core.C:
+                raise ValueError(f"target values must lie in [0, {core.C}), got [{lo}, {hi}]")
+
+    # token rows (frames x tokens per frame) per device pass of integrated_gradients when internal_batch_size is None:
+    # measured at 256 frames of raw-IQ seg16 (T = 65), doubling a pass from 2^18 to 2^19 rows gains 3 % for twice the
+    # workspace (DESIGN §8.1)
+    IG_TOKEN_BUDGET = 1 << 18
+
+    @torch.no_grad()
+    def integrated_gradients(self, src, target=None, baseline=None, steps=32, internal_batch_size=None,
+                             return_delta=False):
+        """Integrated Gradients (Sundararajan, Taly & Yan, "Axiomatic Attribution for Deep Networks", ICML 2017) of
+        the target-class logit w.r.t. every input sample:
+
+            IG_t(x) = (x - x') * integral_0^1 dy_t/dx (x' + a (x - x')) da
+
+        with ``y_t`` the logit of class t (not the loss and not the softmax) and ``x'`` the baseline.  The integral is
+        the ``steps``-point Gauss-Legendre rule on [0, 1].  Completeness: ``attr[b].sum()`` approaches
+        ``y_t(x_b) - y_t(x'_b)`` as ``steps`` grows.
+
+        ``src`` is what ``forward`` takes, in either input layout; after ``set_raw_input`` the attribution is w.r.t. the
+        un-normalised dataset frames, as ``src.grad`` is.  ``baseline`` is ``None`` (zeros in that layout) or an fp32
+        tensor of the shape of ``src`` on its device.  ``target`` is ``None`` (each frame's predicted class at ``x``,
+        the first maximum of its logits, from the same forward) or a contiguous int64 CUDA tensor ``[B]`` with values
+        in ``[0, num_classes)``.  Returns fp32 with the shape and layout of ``src``; with ``return_delta=True`` also
+        ``delta`` fp32 ``[B]``, ``attr[b].sum() - (y_t(x_b) - y_t(x'_b))``, the convergence check.
+
+        All on the device: one forward of ``[x; x']``, then chunks of path points, each a blend of the two endpoint
+        embeddings (the front end is affine in ``src``), the layers, the seed ``w_k e_t`` and the frozen backward down
+        to the embedding; their gradients are summed in fp32 in a fixed order (repeated calls are bit-identical) and
+        the embedding dgrad and the scatter times ``x - x'`` run once.
+
+        ``internal_batch_size`` caps the frames per device pass: a pass takes at most
+        ``max(1, internal_batch_size // B)`` path points, ``n_c * B`` frames (never fewer than one point's B frames),
+        and the points are spread evenly over the fewest passes.  ``None`` caps a pass at ``IG_TOKEN_BUDGET`` = 2^18
+        token rows (frames x tokens per frame), so large batches run one point per pass.  Memory: the training-mode
+        workspace of ``max(2, n_c) * B`` frames plus fp32 copies of ``[x; x']``, of both endpoints' embeddings
+        ``[2B, T, d]`` and of the gradient sum: 7.1 GB for raw-IQ seg16 d128 L6 at B = 256 in bf16 (11 points a
+        pass), 17 GB for SPS-1 seg8 d256 L6 at B = 1024 (DESIGN §8.1).  Results for different
+        ``internal_batch_size`` agree to fp32 summation order.
+
+        Runs under ``torch.no_grad()`` with dropout off whatever ``self.training`` is, in the model's compute dtype;
+        parameters, their ``.grad`` and ``training`` are left as they are.  Raises ``ValueError`` for a bad
+        ``target``, ``baseline``, ``steps < 1`` or ``internal_batch_size < 1``."""
+        core = self._core
+        self._check_target(src, target)
+        if baseline is None:
+            baseline = torch.zeros_like(src)
+        else:
+            if not isinstance(baseline, torch.Tensor):
+                raise ValueError(f"baseline must be None or a tensor, got {type(baseline).__name__}")
+            if baseline.shape != src.shape or baseline.dtype != torch.float32 or baseline.device != src.device:
+                raise ValueError(f"baseline must be float32 {tuple(src.shape)} on {src.device}, got {baseline.dtype} "
+                                 f"{tuple(baseline.shape)} on {baseline.device}")
+            baseline = baseline.contiguous()
+        steps = self._positive_int("steps", steps)
+        ibs = None if internal_batch_size is None else self._positive_int("internal_batch_size", internal_batch_size)
+        desc = core.make_desc(src, training=True, module_training=False)
+        B, dev = desc.B, src.device
+        per_pass = max(1, ibs // max(B, 1) if internal_batch_size is not None else
+                       self.IG_TOKEN_BUDGET // max(B * core.layout.T, 1))
+        passes = -(-steps // per_pass)
+        chunk = -(-steps // passes)
+        x, w = np.polynomial.legendre.leggauss(steps)
+        alpha = torch.tensor((x + 1.0) / 2.0, dtype=torch.float32, device=dev)
+        weight = torch.tensor(w / 2.0, dtype=torch.float32, device=dev)
+        ws = torch.empty(_lib.ig_workspace_bytes(desc, chunk), dtype=torch.uint8, device=dev)
+        logits = torch.empty((2, B, core.C), dtype=torch.float32, device=dev)
+        attr = torch.empty_like(src)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(_lib.lib.amc_model_integrated_gradients(C.byref(desc), src.data_ptr(), baseline.data_ptr(),
+                                                           core.flat.data_ptr(), core.pos_buffer().data_ptr(),
+                                                           ws.data_ptr(), _lib.ptr(target), steps, alpha.data_ptr(),
+                                                           weight.data_ptr(), chunk, logits.data_ptr(),
+                                                           attr.data_ptr(), stream),
+                   "amc_model_integrated_gradients")
+        if not return_delta:
+            return attr
+        t = target
+        if t is None:
+            t = torch.empty(B, dtype=torch.int64, device=dev)
+            _lib.check(_lib.lib.amc_argmax(B, core.C, logits.data_ptr(), t.data_ptr(), stream), "amc_argmax")
+        y = logits.gather(2, t.view(1, B, 1).expand(2, B, 1)).squeeze(2).double()
+        delta = attr.reshape(B, -1).double().sum(1) - (y[0] - y[1])
+        return attr, delta.float()
+
+    @staticmethod
+    def _positive_int(name, v) -> int:
+        try:
+            i = operator.index(v)
+        except TypeError:
+            i = None
+        if isinstance(v, (bool, np.bool_)) or i is None or i < 1:
+            raise ValueError(f"{name} must be an integer >= 1, got {v!r}")
+        return i
 
     def _run(self, src, want_logits):
         # grad mode is switched off inside Function.forward, so decide here whether to keep activations
